@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- inspected frames/s over pre + post + measure (the metric BASELINE.json names).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config cfg2] [--impl b200|reference] [--dump-outputs DIR]
 
 A step = one pass of the hot path (K1 undistort+letterbox, K2 decode/filter, K3 NMS, K4 masks+statistics, K5 measure)
 over one batch of synthetic frames + planted head tensors already resident in HBM.  N=1 workload = BASELINE.json
@@ -10,10 +10,11 @@ its own batch (weak scaling, no data-path collective) and pushes its compact per
 through NVLink peer memory (shard.PeerGather; --gather nccl = an all-gather of the same buffers).  At N>1 the line also
 carries `cfg5_sharded`: BASELINE.json configs[4], 256 synthetic 4K frames SPLIT over the ranks (shard.shard_range,
 strong scaling), resident and end to end, records gathered -- beside the weak-scaled cfg2 headline.
-The CPU arm (cpu_baseline / --impl reference) runs the reference's OWN measurement.py (staged by
-baseline/stage_reference.py into baseline/_ref/) behind the Ultralytics restatement on real cv2/torch/torchvision
-operators; without the staged copy it falls back to the measure-stage port and says kind "port".
-Prints ONE JSON line on rank 0.
+The CPU arm (cpu_baseline / --impl reference) runs the reference's OWN measurement.py (from a checkout at
+oracle/_ref/ or VTI_REFERENCE_DIR) behind the Ultralytics restatement on real cv2/torch/torchvision operators;
+without one the arm runs the measure-stage port and says kind "port".
+Prints ONE JSON line on rank 0.  --dump-outputs DIR also writes what the last timed step computed (dump_arrays()),
+so that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -27,6 +28,10 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# A benchmark run leaves the tree as it found it (it may be read-only): no bytecode caches, here or in the spawned
+# CPU-arm workers.
+sys.dont_write_bytecode = True
+os.environ["PYTHONDONTWRITEBYTECODE"] = "1"
 
 import numpy as np  # noqa: E402
 
@@ -68,6 +73,51 @@ def stage_bytes(cfg, n_det_mean: float, n_cand_mean: float | None = None):
         "K4": 128 * ph * pw,
         "K5": 64 * n_det_mean,
     }
+
+
+DUMP_BYTES = 64 << 20            # --dump-outputs writes at most this much
+DUMP_NET_IN_SAMPLE = 1 << 22     # elements of K1's output it keeps (16 MB of float32; cfg2's whole tensor is 400 MB)
+
+
+def dump_sample_index(numel: int) -> np.ndarray:
+    """Flat indices of K1's output that --dump-outputs keeps: all of them up to DUMP_NET_IN_SAMPLE elements, else the
+    sorted, de-duplicated indices default_rng(0) draws -- the same on every run and every build."""
+    if numel <= DUMP_NET_IN_SAMPLE:
+        return np.arange(numel)
+    return np.unique(np.random.default_rng(0).integers(0, numel, DUMP_NET_IN_SAMPLE))
+
+
+def dump_arrays(net_in_sample, dets, counts, results) -> dict:
+    """--dump-outputs: what the last timed step handed its caller, as name -> array (host numpy in: the K1 sample at
+    dump_sample_index, the vti_det records (B, max_det), the counts, the vti_frame_result rows).  net_in_sample =
+    the K1 sample; counts = records per frame; dets_<field> = every field of the records (rows past a frame's count
+    zeroed: a caller never reads them); results_<field> = every field of the per-frame results.  float32 fields stay
+    float32, the others become float64 (which holds every integer field exactly).  Every value is finite: K5 marks
+    "no value" with NaN (a record without a distance, a frame without an average), so each floating-point array has
+    its non-finite entries set to 0 and <name>_nonfinite beside it says where they were (0 finite, 1 NaN, 2 +inf,
+    3 -inf).  The set of names does not depend on the data.  Raises SystemExit beyond DUMP_BYTES."""
+    arrays = {"net_in_sample": net_in_sample, "counts": counts}
+    valid = np.arange(dets.shape[1])[None, :] < counts[:, None]
+    for f in dets.dtype.names:
+        arrays["dets_" + f] = np.where(valid.reshape(valid.shape + (1,) * (dets[f].ndim - 2)), dets[f], 0)
+    for f in results.dtype.names:
+        arrays["results_" + f] = results[f]
+    for k in [k for k, a in arrays.items() if np.issubdtype(a.dtype, np.floating)]:
+        a = arrays[k]
+        arrays[k + "_nonfinite"] = np.select([np.isnan(a), a == np.inf, a == -np.inf], [1, 2, 3], 0).astype(np.float32)
+        arrays[k] = np.where(np.isfinite(a), a, a.dtype.type(0))
+    arrays = {k: a.astype(np.float32 if a.dtype == np.float32 else np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise SystemExit(f"--dump-outputs: {total / 2**20:.0f} MB of outputs at this batch, more than "
+                         f"{DUMP_BYTES >> 20} MB; use a smaller --batch")
+    return arrays
+
+
+def write_dump(out_dir, arrays: dict) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 class ClockSampler:
@@ -161,7 +211,7 @@ def cpu_reference(cfg, batch, calib, n_frames: int, warm: int = 3, single_thread
         one(i % nb)
         per.append(time.perf_counter() - t1)
     dt = time.perf_counter() - t0
-    cores = {"measure_stage": "verbatim reference (baseline/_ref)" if app is not None else "port (oracle/measure_port.py)",
+    cores = {"measure_stage": "verbatim reference (oracle/ref_verbatim.py)" if app is not None else "port (oracle/measure_port.py)",
              "os_cpu_count": os.cpu_count(), "torch_threads": torch.get_num_threads(), "cv2_threads": cv2.getNumThreads(),
              "ms_per_frame_median": 1e3 * float(np.median(per)), "ms_per_frame_p10": 1e3 * float(np.percentile(per, 10)),
              "ms_per_frame_p90": 1e3 * float(np.percentile(per, 90))}
@@ -219,7 +269,8 @@ def cpu_kind() -> tuple[str, str]:
         return "reference", ("pre/post = the Ultralytics calls restated on the real cv2 / torch / torchvision operators "
                              "(ultralytics itself is not installable offline), measure = the reference's own "
                              "process_frame run verbatim from " + os.path.relpath(ref_verbatim.REF, ROOT))
-    return "port", "cv2+torch+torchvision operators + measure-stage port (no staged reference copy found)"
+    return "port", ("cv2+torch+torchvision operators + measure-stage port "
+                    "(no reference checkout at oracle/_ref/ or VTI_REFERENCE_DIR)")
 
 
 def run_reference(args, cfg, rank, world):
@@ -605,6 +656,15 @@ def run_b200(args, cfg, rank, world, local_rank):
             dist.barrier()
         torch.cuda.synchronize()
 
+    # --dump-outputs: the K1 sample and the size of the dump are settled before anything is timed (a dry run on
+    # zeros of the real shapes refuses more than DUMP_BYTES here rather than after the run)
+    dump_idx = None
+    if args.dump_outputs and rank == 0:
+        from vision_textile_inspection_b200._lib import DET_DTYPE, RESULT_DTYPE
+        idx = dump_sample_index(net_in.numel())
+        dump_arrays(np.zeros(idx.size, np.float32), np.zeros((B, cfg.max_det), DET_DTYPE), np.zeros(B, np.int32),
+                    np.zeros(B, RESULT_DTYPE))
+        dump_idx = torch.from_numpy(idx).to(dev)
     fork()
     for _ in range(args.warmup):
         step()
@@ -624,6 +684,9 @@ def run_b200(args, cfg, rank, world, local_rank):
         step()
     join()
     e1.record()
+    # what the last timed step produced, for --dump-outputs (the steps below overwrite these buffers)
+    last_out = ([net_in.view(-1)[dump_idx]] + [t.clone() for t in bufs[(state["i"] - 1) & 1][1][:3]]
+                if dump_idx is not None else None)
     launches = sum(e.launch_count for e in set(engs)) + nodes_per_graph * replays["n"] - l0   # graph kernel nodes count
     # two more regions of K steps, timed the same way: the spread of the number (the reported value is the FIRST region)
     extra_ev = []
@@ -913,6 +976,9 @@ def run_b200(args, cfg, rank, world, local_rank):
     if cpu is not None:
         line["cpu_baseline"] = cpu
     print(json.dumps(line), file=REAL_STDOUT, flush=True)
+    if last_out is not None:
+        write_dump(args.dump_outputs, dump_arrays(last_out[0].cpu().numpy(), eng.dets_to_numpy(last_out[1]),
+                                                  last_out[2].cpu().numpy(), eng.results_to_numpy(last_out[3])))
     if world > 1:
         dist.destroy_process_group()
 
@@ -942,7 +1008,13 @@ def main():
                          "gain on cfg2 (K1-bound, 221 vs 226 k frames/s), +50 %% on the post-bound stress config cfg4")
     ap.add_argument("--gather", default="peer", choices=["peer", "nccl"],
                     help="N > 1: records to rank 0 through NVLink peer memory (default) or an NCCL all-gather")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed (rank 0's batch) as DIR/<name>.npy, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     _protect_stdout()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank = int(os.environ.get("RANK", "0"))

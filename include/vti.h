@@ -4,9 +4,9 @@
  * Drop-in boundary (SURVEY.md 8b).  The reference is pure Python and has no FFI of its own; the calls this
  * library replaces are
  *
- *   outer:  StitchMeasurementApp.process_frame(frame)            /root/reference/measurement.py:188  (main.py:211)
- *   inner:  self.model.predict(rgb, conf, iou, max_det, imgsz)   /root/reference/measurement.py:208-210
- *           (config 3: /root/reference/Utils/check_stitch_distance.py:281, :286)
+ *   outer:  StitchMeasurementApp.process_frame(frame)            measurement.py:188  (main.py:211)
+ *   inner:  self.model.predict(rgb, conf, iou, max_det, imgsz)   measurement.py:208-210
+ *           (config 3: Utils/check_stitch_distance.py:281, :286)
  *
  * and the binding a maintainer adds is a ctypes stub (INTEGRATION.md; ours is vision_textile_inspection_b200/_lib.py).
  * Plain pointers and sizes only: no torch / Python types.  Device pointers are raw CUDA device addresses, `stream`

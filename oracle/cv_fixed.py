@@ -4,7 +4,7 @@ This file is part of the CPU oracle.  Only tests/, __graft_entry__.smoke() and b
 --impl reference legs may import it.  The product (vision_textile_inspection_b200) never does.
 
 What is restated (SURVEY.md section 8a rows U0/U1/M2; the arithmetic lives in OpenCV, which the reference
-pins as opencv-contrib-python==4.11.0.86 in /root/reference/requirements.txt:2 and reaches through
+pins as opencv-contrib-python==4.11.0.86 in requirements.txt:2 and reaches through
 ultralytics LetterBox (measurement.py:208-210) and cv2.resize(INTER_NEAREST) (measurement.py:78-79)):
 
   * cv2.resize(..., INTER_LINEAR) on uint8: 11-bit coefficients, H pass then V pass
@@ -176,7 +176,7 @@ def scale_K(K, w: int, h: int, calib_w: int = 1280, calib_h: int = 960) -> np.nd
 
 # ---- camera-native ingest: packed YUV 4:2:2 -> BGR (OpenCV modules/imgproc/src/color_yuv.simd.hpp, YUV422toRGB8Invoker /
 # uvToRGBuv / yRGBuvToRGBA with the ITU-R BT.601 constants below; what cv2.VideoCapture.read() applies to a YUYV camera
-# stream before /root/reference/main.py:188 hands the frame to process_frame).  Pinned in tests/test_oracle_cv.py against
+# stream before main.py:188 hands the frame to process_frame).  Pinned in tests/test_oracle_cv.py against
 # cv2.cvtColor(.., COLOR_YUV2BGR_YUY2) over every (Y, U, V) triple.
 ITUR_BT_601_CY, ITUR_BT_601_CUB, ITUR_BT_601_CUG = 1220542, 2116026, -409993
 ITUR_BT_601_CVG, ITUR_BT_601_CVR, ITUR_BT_601_SHIFT = -852492, 1673527, 20

@@ -1,6 +1,7 @@
 """TEST INFRASTRUCTURE ONLY -- writes tests/golden/*.json by running the VERBATIM reference modules.
 
-Run in the build container (needs /root/reference):   python -m oracle.gen_golden
+Needs a checkout of the reference application at oracle/_ref/ (or VTI_REFERENCE_DIR=<checkout>):
+    python -m oracle.gen_golden
 
 Outputs
   vision_textile_inspection_b200/data/reference_calibration.json   K / dist / rvec / tvec values of the three
@@ -74,7 +75,7 @@ def run_scene(name, seed, calib, app_cache):
 
 
 def main():
-    assert ref_verbatim.available(), "needs /root/reference"
+    assert ref_verbatim.available(), "needs a checkout of the reference at oracle/_ref/ or VTI_REFERENCE_DIR"
     calib = load_calibration()
     os.makedirs(os.path.join(ROOT, "vision_textile_inspection_b200", "data"), exist_ok=True)
     with open(os.path.join(ROOT, "vision_textile_inspection_b200", "data", "reference_calibration.json"), "w") as f:

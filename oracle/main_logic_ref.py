@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE ONLY -- line-by-line restatement of the per-frame record logic that lives inline in
-/root/reference/main.py:main() (:167-168, :183-184, :213-293).  It cannot be imported from the reference (it is the
+main.py:main() (:167-168, :183-184, :213-293).  It cannot be imported from the reference (it is the
 body of a `while True` loop around a camera, a serial port and MySQL), so it is restated here with the same variable
 names and the same statement order; tests/test_postlogic.py drives it and the product's SeamRecordLogic with the same
 measurement sequence and the same jitter stream.  Parity unpinned by the reference (no tests, no recorded rows)."""

@@ -1,10 +1,10 @@
 """TEST INFRASTRUCTURE ONLY -- runs the record logic of the reference's main.py VERBATIM.
 
-/root/reference/main.py:main() is one long camera loop and cannot be imported and called piecewise, but the lines that
+main.py:main() is one long camera loop and cannot be imported and called piecewise, but the lines that
 turn process_frame's dict into a database row (from `current_stitch_count = serial_reader.get_stitch_count()` down to
 the `db.insert_measurement(...)` call, main.py:214-293) are plain Python on local names.  This module cuts exactly
-those lines out of the reference's own file (where it lies: /root/reference, or the copy staged by
-baseline/stage_reference.py), de-indents them and executes them, once per frame, in a namespace that supplies the names
+those lines out of the reference's own file (where it lies: oracle/_ref/ or VTI_REFERENCE_DIR, see
+oracle/ref_verbatim.py), de-indents them and executes them, once per frame, in a namespace that supplies the names
 the block reads: the constants from the reference's config module, stub `serial_reader` / `db` objects, the deques and
 counters the loop keeps, and `random` (seeded by the caller).  No line of the block is restated here.
 """
@@ -24,7 +24,7 @@ END = "# Update total distance"
 
 
 def available() -> bool:
-    return os.path.isfile(os.path.join(ref_verbatim.REF, "main.py"))
+    return ref_verbatim.available() and os.path.isfile(os.path.join(ref_verbatim.REF, "main.py"))
 
 
 def _block() -> str:

@@ -4,14 +4,14 @@ the reference's own files).
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this.
 
 Follows, step by step (SURVEY.md 8a rows M1-M8):
-  variant 0: /root/reference/measurement.py:44-65 (plane, pixel->world), :70-86 (instance bitmap), :88-113 (k-means),
+  variant 0: measurement.py:44-65 (plane, pixel->world), :70-86 (instance bitmap), :88-113 (k-means),
              :160-185 (union, lower envelope), :188-511 (process_frame, numbers only -- no drawing)
-  variant 1: /root/reference/Utils/check_stitch_distance.py:57-80, :85-111, :143-171, :226-251, :281-553
+  variant 1: Utils/check_stitch_distance.py:57-80, :85-111, :143-171, :226-251, :281-553
 
 It makes the same library calls in the same order as the reference (cv2.resize INTER_NEAREST on the full
 letterboxed mask, cv2.moments, np.any/np.where, cv2.undistortPoints, np.median/np.mean), so timing it is timing the
 reference's algorithm, and it is pinned against the reference itself: oracle/gen_golden.py imports the verbatim
-/root/reference modules in the build container and tests/test_oracle_measure.py checks this port against the
+reference modules (oracle/ref_verbatim.py) and tests/test_oracle_measure.py checks this port against the
 vectors it wrote to tests/golden/ (plus the known-answer vectors of SURVEY.md 8c).
 
 Unlike the reference it returns every intermediate (per-stitch centroids, widths, selections) so the CUDA

@@ -2,9 +2,9 @@
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this.
 
-The arithmetic restated here lives in `ultralytics` (unpinned, /root/reference/requirements.txt:13), reached from
-/root/reference/measurement.py:208-210 (`self.model.predict(rgb, conf=..., iou=..., max_det=..., imgsz=960)`) and
-/root/reference/Utils/check_stitch_distance.py:286.  `ultralytics` is not vendored under /root/reference and is not
+The arithmetic restated here lives in `ultralytics` (unpinned, requirements.txt:13), reached from
+measurement.py:208-210 (`self.model.predict(rgb, conf=..., iou=..., max_det=..., imgsz=960)`) and
+Utils/check_stitch_distance.py:286.  `ultralytics` is not vendored in the reference and is not
 installed, so this restates its published algorithm (SURVEY.md 8a rows U3-U7):
 
   U3  Detect/Segment head tail: DFL softmax-expectation over 16 bins, dist2bbox(xywh), x stride, class sigmoid

@@ -1,10 +1,12 @@
 """TEST INFRASTRUCTURE ONLY -- loads the reference's own measure-stage modules VERBATIM.
 
-Source: /root/reference in the build container; on the GPU box (which has no /root/reference) the copy that
-baseline/stage_reference.py staged into baseline/_ref/ (git-ignored, shipped by gpurun).  Used by oracle/gen_golden.py
-to produce tests/golden/*.json, by tests/test_oracle_measure.py to pin oracle/measure_port.py against the reference
-itself, by tests/test_app.py to run the reference's own process_frame with the B200 predictor plugged in
-(INTEGRATION.md 2), and by bench.py's CPU arm (kind "reference").  The modules are imported where they lie.
+Source: a checkout of the reference application (github.com/RishWijewardhena/vision-textile-inspection), placed or
+linked at oracle/_ref/ (git-ignored) or named by the environment variable VTI_REFERENCE_DIR, which takes precedence.
+It is not part of this repository: without it the tests that run the reference live skip, and the committed goldens
+stand for it.  Used by
+oracle/gen_golden.py to produce tests/golden/*.json, by tests/test_oracle_measure.py to pin oracle/measure_port.py
+against the reference itself, by tests/test_app.py to run the reference's own process_frame with the B200 predictor
+plugged in (INTEGRATION.md 2), and by bench.py's CPU arm (kind "reference").  The modules are imported where they lie.
 
 Recipe (SURVEY.md 8c): stub `ultralytics` (measurement.py:9) and `serial` (config.py:7 -> hardware_utils.py:1), set
 dummy DB_* variables (config.py:132-133 raises without them), then build StitchMeasurementApp with __new__ so that
@@ -22,8 +24,7 @@ from collections import deque
 
 import numpy as np
 
-_STAGED = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "baseline", "_ref")
-REF = "/root/reference" if os.path.isfile("/root/reference/measurement.py") else _STAGED
+REF = os.path.abspath(os.environ.get("VTI_REFERENCE_DIR") or os.path.join(os.path.dirname(__file__), "_ref"))
 
 
 def available() -> bool:
@@ -49,7 +50,7 @@ def _stubs():
 
 
 def load(variant: int):
-    """variant 0 -> /root/reference/measurement.py, 1 -> /root/reference/Utils/check_stitch_distance.py."""
+    """variant 0 -> <REF>/measurement.py, 1 -> <REF>/Utils/check_stitch_distance.py."""
     _stubs()
     path = REF if variant == 0 else os.path.join(REF, "Utils")
     if path not in sys.path:

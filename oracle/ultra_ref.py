@@ -2,8 +2,8 @@
 
 Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / --impl reference legs may import this.
 
-/root/reference/measurement.py:208-210 calls `ultralytics` `YOLO.predict`; ultralytics is a pip dependency
-(/root/reference/requirements.txt:13, unpinned), absent from /root/reference and not installed here.  This module
+measurement.py:208-210 calls `ultralytics` `YOLO.predict`; ultralytics is a pip dependency
+(requirements.txt:13, unpinned), absent from the reference and not installed here.  This module
 restates what that call does around the backbone (SURVEY.md 8a U0-U7), using the same operators ultralytics itself
 calls -- cv2.resize / cv2.copyMakeBorder / cv2.undistort, torch softmax / sigmoid / matmul / F.interpolate,
 torchvision.ops.nms -- so the third-party CPU kernels stay in the loop.  It is both the parity oracle for the CUDA

@@ -1,6 +1,6 @@
 """The drop-in host boundary (vision_textile_inspection_b200/app.py) against the reference's contract (SURVEY 8b):
 constructor errors, the process_frame dict, error paths, and -- on the GPU -- the VERBATIM reference's frame sequence
-(tests/golden/scenes.json, written by oracle/gen_golden.py through /root/reference/measurement.py)."""
+(tests/golden/scenes.json, written by oracle/gen_golden.py through measurement.py)."""
 import json
 import os
 
@@ -178,12 +178,12 @@ def test_predict_inner_boundary_matches_oracle():
 @pytest.mark.gpu
 def test_verbatim_reference_process_frame_with_b200_predictor_plugged_in():
     """INTEGRATION.md 2, the zero-edit drop-in: the reference's OWN process_frame (measurement.py:188-511, run where it
-    lies: /root/reference, or the copy baseline/stage_reference.py staged for the GPU box) with `app.model` replaced by
+    lies: oracle/_ref/ or VTI_REFERENCE_DIR) with `app.model` replaced by
     B200Predictor -- letterbox, decode, NMS and masks on the GPU, the reference's measure stage on those results --
     must return what it returned with the CPU Ultralytics restatement when the goldens were written."""
     from oracle import cv_fixed, measure_port, ref_verbatim
     if not ref_verbatim.available():
-        pytest.skip("no reference copy (run baseline/stage_reference.py in the build container)")
+        pytest.skip("needs a checkout of the reference at oracle/_ref/ or VTI_REFERENCE_DIR")
     g = json.load(open(os.path.join(G, "scenes.json")))
     calib = helpers.load_calib()
     cfg = synth.CONFIGS["native"]

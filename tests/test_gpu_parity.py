@@ -257,7 +257,7 @@ def test_mask_variant_b(name, seeds, calib):
 
 
 def test_against_verbatim_reference_goldens(calib):
-    """tests/golden/scenes.json was written by the VERBATIM /root/reference process_frame (oracle/gen_golden.py)."""
+    """tests/golden/scenes.json was written by the VERBATIM reference process_frame (oracle/gen_golden.py)."""
     g = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "scenes.json")))
     for s in g["scenes"]:
         cfg = synth.CONFIGS[s["config"]]

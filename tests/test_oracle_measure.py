@@ -1,5 +1,6 @@
 """Pins oracle/measure_port.py against the reference's own code: golden vectors written by oracle/gen_golden.py
-from the VERBATIM /root/reference modules (and, when /root/reference is present, against those modules live)."""
+from the VERBATIM reference modules (and, when a checkout of the reference is at oracle/_ref/ or
+VTI_REFERENCE_DIR, against those modules live)."""
 import json
 import os
 
@@ -66,7 +67,8 @@ def test_temporal_sequence_matches_verbatim(calib):
         assert d["stitch_count"] == fr["stitch_count"]
 
 
-@pytest.mark.skipif(not ref_verbatim.available(), reason="/root/reference only exists in the build container")
+@pytest.mark.skipif(not ref_verbatim.available(),
+                    reason="needs a checkout of the reference at oracle/_ref/ or VTI_REFERENCE_DIR")
 def test_port_matches_reference_live_with_error_paths(calib):
     """Live run of the verbatim reference, including the 'Fabric not detected' / 'No stitches detected' returns."""
     from oracle import gen_golden

@@ -1,4 +1,4 @@
-"""SURVEY 8f rank 4: the per-frame record logic of /root/reference/main.py:213-293 (offsets, validity window, 5-deep
+"""SURVEY 8f rank 4: the per-frame record logic of main.py:213-293 (offsets, validity window, 5-deep
 fallback buffers, travelled distance, DB row) -- product state machine vs the line-by-line restatement, same jitter."""
 import random
 
@@ -54,7 +54,7 @@ def test_record_logic_matches_the_verbatim_main_py_block():
     from oracle import main_verbatim
     from vision_textile_inspection_b200 import postlogic
     if not main_verbatim.available():
-        pytest.skip("no reference copy (baseline/stage_reference.py)")
+        pytest.skip("needs a checkout of the reference at oracle/_ref/ or VTI_REFERENCE_DIR")
     for seed in range(5):
         ms, counts = _sequence(seed)
         ref, ns = main_verbatim.run(ms, counts, seed, total_distance_mm=12.5)

@@ -4,11 +4,11 @@ Two boundaries are mirrored, same names / argument meaning / error behaviour as 
 
   outer   StitchMeasurementApp(calib_path, extr_path, model_path, camera_index=0, calib_w=640, calib_h=640,
                                frame_buffer=8, min_stitches=3, stitch_id=0, fabric_id=1)
-          .process_frame(frame) -> (annotated, measurements)          /root/reference/measurement.py:123-126, 188-511
-          (constructed at /root/reference/main.py:80-91, called at main.py:211); force_camera_resolution(cap, w, h)
+          .process_frame(frame) -> (annotated, measurements)          measurement.py:123-126, 188-511
+          (constructed at main.py:80-91, called at main.py:211); force_camera_resolution(cap, w, h)
           is importable from here as well (main.py:16, 198).
   inner   B200Predictor.predict(rgb, verbose=False, conf=, iou=, max_det=, imgsz=) -> [Results]
-          with r.boxes.cls / r.boxes.xyxy / r.masks.data                /root/reference/measurement.py:208-210, 244-245, 74-75
+          with r.boxes.cls / r.boxes.xyxy / r.masks.data                measurement.py:208-210, 244-245, 74-75
           Assigning a B200Predictor to the reference app's `.model` accelerates pre + post with zero edits there.
 
 The YOLOv8-seg backbone stays in PyTorch and only produces the raw head tensors: a `backbone` is any callable
@@ -31,7 +31,7 @@ import torch
 from . import _lib
 from .engine import EngineConfig, InspectionEngine
 
-# /root/reference/config.py:59-95 defaults (the reference star-imports them; here they are constructor keywords)
+# config.py:59-95 defaults (the reference star-imports them; here they are constructor keywords)
 CALIB_W, CALIB_H = 1280, 960
 CONF_THRESH, IOU_THRESH, MAX_DETECTIONS = 0.20, 0.25, 200
 FRAME_BUFFER, MIN_STITCHES = 8, 3
@@ -50,7 +50,7 @@ def load_json(path):
 
 
 def force_camera_resolution(cap, w, h):
-    """Same contract as /root/reference/measurement.py:23-42: set the capture size, report what the camera gave."""
+    """Same contract as measurement.py:23-42: set the capture size, report what the camera gave."""
     import cv2
     cap.set(cv2.CAP_PROP_FRAME_WIDTH, w)
     cap.set(cv2.CAP_PROP_FRAME_HEIGHT, h)
@@ -67,7 +67,7 @@ def backbone_from_ultralytics(model_path: str, device="cuda"):
     """Wrap an Ultralytics YOLOv8-seg checkpoint so that it returns RAW head tensors (no decode, no NMS).
 
     Needs the `ultralytics` package and the weight file, neither of which exists in the build container
-    (/root/reference/.MISSING_LARGE_BLOBS): this adapter is provided for integration and is NOT covered by tests.
+    (the reference's .MISSING_LARGE_BLOBS): this adapter is provided for integration and is NOT covered by tests.
     """
     try:
         from ultralytics import YOLO
@@ -186,7 +186,7 @@ class B200Predictor:
 
 
 class StitchMeasurementApp:
-    """Outer boundary: what /root/reference/main.py:80-91 constructs and main.py:211 calls.
+    """Outer boundary: what main.py:80-91 constructs and main.py:211 calls.
 
     Extra keywords (all optional) carry what the reference reads from config.py / the camera: `backbone` (callable, see
     module docstring; default = backbone_from_ultralytics(model_path)), `roi`, `conf`, `iou`, `max_det`, `imgsz`,
@@ -382,7 +382,7 @@ class StitchMeasurementApp:
 
 
 class CheckStitchDistanceApp(StitchMeasurementApp):
-    """Outer drop-in for BASELINE config 3: the class /root/reference/Utils/check_stitch_distance.py:176 also calls
+    """Outer drop-in for BASELINE config 3: the class Utils/check_stitch_distance.py:176 also calls
     StitchMeasurementApp, whose process_frame (:281-553) returns `(annotated, info_text)` -- a string, not a dict.
 
     Same constructor signature (:177-187); semantics of that file: no ROI, predict() without imgsz (Ultralytics'

@@ -1,7 +1,7 @@
 """Stand-in YOLOv8-seg network in plain PyTorch (SURVEY.md 8f rank 1): the step BETWEEN pre and post.
 
-The reference loads `best_Model.pt` through Ultralytics (/root/reference/measurement.py:145, :208); neither the weights
-nor the package exist offline (/root/reference/.MISSING_LARGE_BLOBS), so this module rebuilds the published YOLOv8-seg
+The reference loads `best_Model.pt` through Ultralytics (measurement.py:145, :208); neither the weights
+nor the package exist offline (the reference's .MISSING_LARGE_BLOBS), so this module rebuilds the published YOLOv8-seg
 TOPOLOGY (Conv-BN-SiLU stem, C2f stages, SPPF, PAN-FPN neck, Segment head with DFL box branch, class branch, mask
 coefficient branch and the Proto module) with random weights and the head-bias initialisation Ultralytics uses, and
 returns the RAW head tensors in the layouts include/vti.h names:

@@ -1,9 +1,9 @@
 // K0 -- camera-native frame ingest: packed YUV 4:2:2 (YUYV / "YUY2", 2 bytes per pixel) -> BGR u8, bit-exact against
 // cv2.cvtColor(.., COLOR_YUV2BGR_YUY2).
 //
-// Replaces (SURVEY.md 8f rank 2): the colour conversion inside cv2.VideoCapture.read() -- /root/reference/main.py:188
+// Replaces (SURVEY.md 8f rank 2): the colour conversion inside cv2.VideoCapture.read() -- main.py:188
 // `ret, frame = measurement_app.cap.read()`; the reference opens the camera without a FOURCC
-// (/root/reference/measurement.py:22-38), so OpenCV's V4L2 backend negotiates YUYV before MJPEG and converts every frame
+// (measurement.py:22-38), so OpenCV's V4L2 backend negotiates YUYV before MJPEG and converts every frame
 // to BGR on the CPU before process_frame sees it.  Here the frame crosses PCIe as the camera delivered it (2/3 of the
 // BGR bytes) and is converted on the device, in front of K1.
 // Spec: oracle/cv_fixed.py yuyv_to_bgr (OpenCV's ITU-R BT.601 fixed-point form, 20 fractional bits):

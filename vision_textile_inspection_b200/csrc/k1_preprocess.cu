@@ -1,7 +1,7 @@
 // K1 -- fused [cv2.undistort] + Ultralytics LetterBox (cv2.resize INTER_LINEAR + 114 border) + HWC->CHW + /255.
 //
 // Replaces (SURVEY.md 8a U0-U2): cv2.undistort (north-star addition), ultralytics LetterBox.__call__ and
-// BasePredictor.preprocess, reached from /root/reference/measurement.py:205-210.
+// BasePredictor.preprocess, reached from measurement.py:205-210.
 // Spec: oracle/cv_fixed.py (bit-exact integer formulas, pinned against cv2 in tests/test_oracle_cv.py).
 //
 // One CTA produces a TY x TX tile of the letterboxed output for all three planes.  Pixels travel through shared

@@ -2,7 +2,7 @@
 // surviving anchors only, DFL softmax-expectation + dist2bbox + xywh->xyxy.
 //
 // Replaces (SURVEY.md 8a U3 + the prelude of U4): ultralytics Detect._inference / DFL.forward / dist2bbox and the
-// `xc = amax(cls) > conf` selection of ops.non_max_suppression, reached from /root/reference/measurement.py:208-210.
+// `xc = amax(cls) > conf` selection of ops.non_max_suppression, reached from measurement.py:208-210.
 // Spec: oracle/post_spec.py decode_spec / candidates_spec -- every float op below is the same single-rounded
 // IEEE op in the same order (no FMA contraction), so boxes and scores are bit-identical to the spec.
 //

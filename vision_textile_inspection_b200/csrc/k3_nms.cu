@@ -2,7 +2,7 @@
 // scale_boxes / clip / int() / ROI epilogue and the coefficient gather for the kept detections.
 //
 // Replaces (SURVEY.md 8a U4, U5, U7 and the box half of M1): ops.non_max_suppression + torchvision.ops.nms +
-// ops.scale_boxes (reached from /root/reference/measurement.py:208-210) and measurement.py:251-260.
+// ops.scale_boxes (reached from measurement.py:208-210) and measurement.py:251-260.
 // Spec: oracle/post_spec.py nms_spec / scale_boxes_spec (bit-identical: same fp32 op order, no FMA, IoU compared
 // against the threshold in double exactly like the C++ kernel's `ovr > iou_threshold`).
 //

@@ -2,7 +2,7 @@
 // AND the nearest-resize mask statistics of the measure stage, so full-resolution masks are never materialised.
 //
 // Replaces (SURVEY.md 8a U6, M2, M3, M4): ultralytics ops.process_mask / crop_mask / F.interpolate / gt_(0.5)
-// (variant A), reached from /root/reference/measurement.py:208-210 and consumed at :74-75, and then
+// (variant A), reached from measurement.py:208-210 and consumed at :74-75, and then
 //   measurement.py:78-81   cv2.resize(mask, (w,h), INTER_NEAREST) > 0        -> per-axis multiplicity LUTs
 //   measurement.py:160-185 union of fabric masks + lower envelope            -> atomicMax per letterbox column
 //   (Utils/check_stitch_distance.py:238-251 upper envelope                   -> atomicMin)

@@ -2,11 +2,11 @@
 // column extent, 1-D k-means row selection, envelope-proximity filter and the fp64 pixel -> millimetre projection.
 //
 // Replaces (SURVEY.md 8a M1, M3-M8; all fp64, exactly the reference's decisions):
-//   /root/reference/measurement.py:44-65    compute_camera_plane / pixel_to_world_using_camera_plane
+//   measurement.py:44-65    compute_camera_plane / pixel_to_world_using_camera_plane
 //                                           (cv2.undistortPoints == exactly 5 fixed-point iterations, (u-cx)*(1/fx))
-//   /root/reference/measurement.py:88-113   kmeans_1d_two_clusters (labels NOT updated on break)
-//   /root/reference/measurement.py:280-289, 302-330, 343-356, 390-430, 440-472
-//   variant 1: /root/reference/Utils/check_stitch_distance.py:143-171 (labels updated on break), :331-334 (bbox-filled
+//   measurement.py:88-113   kmeans_1d_two_clusters (labels NOT updated on break)
+//   measurement.py:280-289, 302-330, 343-356, 390-430, 440-472
+//   variant 1: Utils/check_stitch_distance.py:143-171 (labels updated on break), :331-334 (bbox-filled
 //              fabric fallback), :349 (upper envelope), :442-443 (0 < d < 150), :489-507 (widths of final stitches only)
 // Spec / oracle: oracle/measure_port.py (pinned against the verbatim reference through tests/golden/).
 //

@@ -1,6 +1,6 @@
 // K6 -- annotated overlay rasterised on the GPU + JPEG encode with nvJPEG (SURVEY.md 8f rank 3).
 //
-// Replaces the drawing calls of /root/reference/measurement.py (they have no effect on the numbers; main.py:302-314 saves
+// Replaces the drawing calls of measurement.py (they have no effect on the numbers; main.py:302-314 saves
 // the annotated frame as a JPEG for every inspected frame):
 //   :230-236  ROI rectangle                       cv2.rectangle(.., ROI_BORDER_COLOR, 2)
 //   :268-272  per-detection boxes                 stitch (255,255,0) thickness 1, fabric (255,0,255) thickness 2
@@ -296,7 +296,7 @@ extern "C" long long vti_encode_jpeg(vti_handle* h, const uint8_t* image, int qu
 }
 
 // Frame ingest from a compressed camera stream (SURVEY.md 8f rank 2): the camera of the reference delivers MJPEG
-// (cv2.VideoCapture, /root/reference/main.py:188 decodes it on the CPU before process_frame sees the array).  Decodes ONE
+// (cv2.VideoCapture, main.py:188 decodes it on the CPU before process_frame sees the array).  Decodes ONE
 // baseline JPEG (host bytes) with nvJPEG straight into the device frame buffer K1 reads (frame_h x frame_w x 3 BGR), so
 // that the frame crosses PCIe compressed.  The image must have the handle's frame size.
 extern "C" int vti_decode_jpeg(vti_handle* h, const uint8_t* jpeg, long long nbytes, uint8_t* frame, void* stream) {

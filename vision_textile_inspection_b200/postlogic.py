@@ -1,4 +1,4 @@
-"""Post-boundary record logic (SURVEY.md 8f rank 4) -- what /root/reference/main.py does with the dict that
+"""Post-boundary record logic (SURVEY.md 8f rank 4) -- what main.py does with the dict that
 process_frame returns, frame after frame, before the database row is written (main.py:213-293):
 
   offsets (config.py:156-157) -> validity window (config.py:147-150) -> 5-deep buffers of the last valid values,

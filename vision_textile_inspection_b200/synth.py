@@ -6,8 +6,8 @@ constructed so that decoding them yields 5-30 overlapping candidates per instanc
 Frames are woven-fabric textures with the same scene geometry.  Everything is numpy + default_rng => identical
 bytes on every machine for a given (config, seed).
 
-Shapes follow /root/repo/BASELINE.md section 3 (configs 1-5) plus the reference deployment ("native", 1280x960,
-/root/reference/config.py:59-60).
+Shapes follow BASELINE.md section 3 (configs 1-5) plus the reference deployment ("native", 1280x960,
+config.py:59-60).
 """
 from __future__ import annotations
 
@@ -75,7 +75,7 @@ class WorkloadConfig:
         return sum((self.LH // s) * (self.LW // s) for s in STRIDES)
 
     def roi(self):
-        """ROI of /root/reference/config.py:91-95 scaled from the 1280x960 calibration size to this frame."""
+        """ROI of config.py:91-95 scaled from the 1280x960 calibration size to this frame."""
         if self.variant == 1:
             return (0, 0, 0, 0, 0)
         sx, sy = self.frame_w / 1280.0, self.frame_h / 960.0
