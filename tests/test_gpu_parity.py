@@ -517,23 +517,6 @@ def test_decode_nms_other_class_counts(nc):
     assert np.array_equal(d["box_lb"].view(np.uint32), sp["box_lb"].view(np.uint32))
 
 
-def test_k4_tma_form_matches_ldg_form(monkeypatch):
-    """The opt-in TMA form of K4 (cp.async.bulk.tensor boxes + mbarrier double buffering; slower on B200, kept as a
-    measured experiment) must produce byte-identical records to the default LDG form."""
-    cfg = synth.CONFIGS["cfg2"]
-    seeds = [2000, 2001, 2002]
-    monkeypatch.delenv("VTI_K4_TMA", raising=False)
-    _, _, d1, c1, r1, m1 = run_gpu(cfg, seeds, export_masks=True)
-    monkeypatch.setenv("VTI_K4_TMA", "1")
-    _, _, d2, c2, r2, m2 = run_gpu(cfg, seeds, export_masks=True)
-    assert np.array_equal(c1, c2)
-    for b in range(len(seeds)):
-        n = int(c1[b])
-        assert torch.equal(m1[b, :n], m2[b, :n])                   # (slots past the count are never written)
-        assert d1[b, :n].tobytes() == d2[b, :n].tobytes()
-    assert r1.tobytes() == r2.tobytes()
-
-
 def test_misaligned_frames_are_refused_not_faulted():
     cfg = synth.CONFIGS["cfg2"]
     eng = make_engine(cfg, 1)
@@ -691,24 +674,6 @@ def test_k4_tcgen05_tile_form_matches_unit_form(name, seeds):
                 assert abs(r0[b][key] - r2[b][key]) <= MM_RTOL * abs(r0[b][key])
     print(f"\ntcgen05 tile form vs unit form ({name}): {flipped} differing mask pixels of {total}")
     assert flipped <= max(2, total // 100000)
-
-
-def test_k1_tma_output_store_is_bit_identical(monkeypatch):
-    """VTI_K1_TMA=1: the output tile leaves through one cp.async.bulk.tensor store instead of per-thread stores."""
-    cfg = synth.CONFIGS["cfg2"]
-    frames = dev(np.stack([synth.fabric_frame(cfg, 2300 + i) for i in range(3)]))
-    eng = make_engine(cfg, 3)
-    ref = eng.preprocess(frames).clone()
-    monkeypatch.setenv("VTI_K1_TMA", "1")
-    got = eng.preprocess(frames)
-    torch.cuda.synchronize()
-    assert torch.equal(ref, got)
-    cfg1 = synth.CONFIGS["cfg1"]                      # upscale, no undistort: the plain staging path
-    f1 = dev(np.stack([synth.fabric_frame(cfg1, 1300 + i) for i in range(2)]))
-    e1 = make_engine(cfg1, 2)
-    got1 = e1.preprocess(f1)
-    monkeypatch.delenv("VTI_K1_TMA")
-    assert torch.equal(e1.preprocess(f1), got1)
 
 
 def test_two_geometries_alive_at_once():

@@ -1,6 +1,8 @@
 """K1-only microbench for kernel tuning (not the headline bench): times vti_preprocess alone on one config with CUDA
-events and checks the output bit-exactly against real cv2 (cv2.undistort + resize + copyMakeBorder, as Ultralytics' LetterBox).  Several library variants (tools/k1_sweep.sh) are
-loaded into ONE process and timed in interleaved rounds, so clock ramp-up and order effects hit all of them alike:
+events and checks the output bit-exactly against real cv2 (cv2.undistort + resize + copyMakeBorder, as Ultralytics' LetterBox).  Several library variants are
+loaded into ONE process and timed in interleaved rounds, so clock ramp-up and order effects hit all of them alike.  Build
+each variant side by side, then pass them all:
+    VTI_LIB=tools/_variants/libvti_A.so VTI_NVCC_FLAGS="-D..." python vision_textile_inspection_b200/build.py --force
     python tools/k1_bench.py [--libs tools/_variants/libvti_*.so]"""
 import argparse
 import glob

@@ -19,16 +19,9 @@
 // HBM traffic: frame read once (tile halos hit L2) + 12*LH*LW written once; the 4 B/px remap table is L2-resident
 // across the batch.
 #include <algorithm>
-#include <cstdlib>
 #include <vector>
 
-#include <cuda.h>
-
 #include "vti_internal.h"
-
-// k4_masks.cu: cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda)
-bool vti_encode_tmap_f32_3d(CUtensorMap* m, const void* base, unsigned long long d0, unsigned long long d1,
-                            unsigned long long d2, unsigned b0, unsigned b1, unsigned b2);
 
 namespace {
 
@@ -294,82 +287,14 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a
 //     columns at once, one IDP.2A (dp2a) does the column blend + rounding constant: 2 PRMT + 2 IMAD + 1 IDP + 1 SHF.
 //   * resize math: PRMT pairs the two horizontal taps of two channels, IDP.2A applies the 11-bit (a0, a1) taps;
 //     the V pass multiplies by (b0, b1), PRMT extracts both >>16 at once and IDP.2A adds them with the +2.
+// What was tried and rejected: DESIGN.md 5.
 // ====================================================================================================================
-#ifndef VTI_FTY
-#define VTI_FTY 32
-#endif
-#ifndef VTI_FT_THREADS
-#define VTI_FT_THREADS 256
-#endif
-#ifndef VTI_FT_MINB
-#define VTI_FT_MINB 5
-#endif
-#ifndef VTI_FTX
-#define VTI_FTX 64
-#endif
-#ifndef VTI_K1_HSHARE
-#define VTI_K1_HSHARE 1
-#endif
-// round-2 changes (each can be switched off for A/B runs: tools/k1_sweep.sh; what was tried and rejected: DESIGN.md 5)
-#ifndef VTI_K1_LWT       // output row pitch as a template constant: plane stores take immediate offsets
-#define VTI_K1_LWT 1
-#endif
-#ifndef VTI_K1_DIVFMA    // x / 255 as FMUL + FFMA on split constants (exact for 0..255) instead of a shared-memory table
-#define VTI_K1_DIVFMA 1
-#endif
-#ifndef VTI_K1_TMAOUT    // compile the variant whose output tile leaves through ONE TMA tensor store (run-time opt-in: VTI_K1_TMA=1)
-#define VTI_K1_TMAOUT 1
-#endif
-#ifndef VTI_K1_PADROWS   // strips that contain letterbox padding rows stay on the register-sharing resize path
-#define VTI_K1_PADROWS 1
-#endif
-constexpr int FTX = VTI_FTX, FTY = VTI_FTY;  // fast-path output tile
-constexpr int FT_THREADS = VTI_FT_THREADS;
+constexpr int FTX = 64, FTY = 32;            // fast-path output tile
+constexpr int FT_THREADS = 256;
+constexpr int FT_MINB = 5;                   // __launch_bounds__ minimum resident CTAs per SM (caps registers at 48)
 constexpr int FT_CHUNK = 2 * FT_THREADS;     // the remap loop handles 2 entries per thread and iteration (prefetched)
 constexpr int FT_MAXROWS = 2 * FTY + 2, FT_MAXCOLS = 2 * FTX + 2;
-#ifndef VTI_K1_RAWP
-#define VTI_K1_RAWP 112
-#endif
-constexpr int K1_RAWP = VTI_K1_RAWP;    // raw-box row pitch (words) baked into the remap kernel when no tile needs more
-
-#if !VTI_K1_DIVFMA
-// float32(i) / 255.0f (a true division, IEEE round-to-nearest), as bit patterns: i/255 for the 256 uint8 values.
-// Generated with numpy float32; tests/test_gpu_parity.py::test_k1_bit_exact compares every value against cv2 + torch.
-__device__ const unsigned g_div255_bits[256] = {
-    0x00000000u, 0x3b808081u, 0x3c008081u, 0x3c40c0c1u, 0x3c808081u, 0x3ca0a0a1u, 0x3cc0c0c1u, 0x3ce0e0e1u,
-    0x3d008081u, 0x3d109091u, 0x3d20a0a1u, 0x3d30b0b1u, 0x3d40c0c1u, 0x3d50d0d1u, 0x3d60e0e1u, 0x3d70f0f1u,
-    0x3d808081u, 0x3d888889u, 0x3d909091u, 0x3d989899u, 0x3da0a0a1u, 0x3da8a8a9u, 0x3db0b0b1u, 0x3db8b8b9u,
-    0x3dc0c0c1u, 0x3dc8c8c9u, 0x3dd0d0d1u, 0x3dd8d8d9u, 0x3de0e0e1u, 0x3de8e8e9u, 0x3df0f0f1u, 0x3df8f8f9u,
-    0x3e008081u, 0x3e048485u, 0x3e088889u, 0x3e0c8c8du, 0x3e109091u, 0x3e149495u, 0x3e189899u, 0x3e1c9c9du,
-    0x3e20a0a1u, 0x3e24a4a5u, 0x3e28a8a9u, 0x3e2cacadu, 0x3e30b0b1u, 0x3e34b4b5u, 0x3e38b8b9u, 0x3e3cbcbdu,
-    0x3e40c0c1u, 0x3e44c4c5u, 0x3e48c8c9u, 0x3e4ccccdu, 0x3e50d0d1u, 0x3e54d4d5u, 0x3e58d8d9u, 0x3e5cdcddu,
-    0x3e60e0e1u, 0x3e64e4e5u, 0x3e68e8e9u, 0x3e6cecedu, 0x3e70f0f1u, 0x3e74f4f5u, 0x3e78f8f9u, 0x3e7cfcfdu,
-    0x3e808081u, 0x3e828283u, 0x3e848485u, 0x3e868687u, 0x3e888889u, 0x3e8a8a8bu, 0x3e8c8c8du, 0x3e8e8e8fu,
-    0x3e909091u, 0x3e929293u, 0x3e949495u, 0x3e969697u, 0x3e989899u, 0x3e9a9a9bu, 0x3e9c9c9du, 0x3e9e9e9fu,
-    0x3ea0a0a1u, 0x3ea2a2a3u, 0x3ea4a4a5u, 0x3ea6a6a7u, 0x3ea8a8a9u, 0x3eaaaaabu, 0x3eacacadu, 0x3eaeaeafu,
-    0x3eb0b0b1u, 0x3eb2b2b3u, 0x3eb4b4b5u, 0x3eb6b6b7u, 0x3eb8b8b9u, 0x3ebababbu, 0x3ebcbcbdu, 0x3ebebebfu,
-    0x3ec0c0c1u, 0x3ec2c2c3u, 0x3ec4c4c5u, 0x3ec6c6c7u, 0x3ec8c8c9u, 0x3ecacacbu, 0x3ecccccdu, 0x3ecececfu,
-    0x3ed0d0d1u, 0x3ed2d2d3u, 0x3ed4d4d5u, 0x3ed6d6d7u, 0x3ed8d8d9u, 0x3edadadbu, 0x3edcdcddu, 0x3edededfu,
-    0x3ee0e0e1u, 0x3ee2e2e3u, 0x3ee4e4e5u, 0x3ee6e6e7u, 0x3ee8e8e9u, 0x3eeaeaebu, 0x3eececedu, 0x3eeeeeefu,
-    0x3ef0f0f1u, 0x3ef2f2f3u, 0x3ef4f4f5u, 0x3ef6f6f7u, 0x3ef8f8f9u, 0x3efafafbu, 0x3efcfcfdu, 0x3efefeffu,
-    0x3f008081u, 0x3f018182u, 0x3f028283u, 0x3f038384u, 0x3f048485u, 0x3f058586u, 0x3f068687u, 0x3f078788u,
-    0x3f088889u, 0x3f09898au, 0x3f0a8a8bu, 0x3f0b8b8cu, 0x3f0c8c8du, 0x3f0d8d8eu, 0x3f0e8e8fu, 0x3f0f8f90u,
-    0x3f109091u, 0x3f119192u, 0x3f129293u, 0x3f139394u, 0x3f149495u, 0x3f159596u, 0x3f169697u, 0x3f179798u,
-    0x3f189899u, 0x3f19999au, 0x3f1a9a9bu, 0x3f1b9b9cu, 0x3f1c9c9du, 0x3f1d9d9eu, 0x3f1e9e9fu, 0x3f1f9fa0u,
-    0x3f20a0a1u, 0x3f21a1a2u, 0x3f22a2a3u, 0x3f23a3a4u, 0x3f24a4a5u, 0x3f25a5a6u, 0x3f26a6a7u, 0x3f27a7a8u,
-    0x3f28a8a9u, 0x3f29a9aau, 0x3f2aaaabu, 0x3f2babacu, 0x3f2cacadu, 0x3f2dadaeu, 0x3f2eaeafu, 0x3f2fafb0u,
-    0x3f30b0b1u, 0x3f31b1b2u, 0x3f32b2b3u, 0x3f33b3b4u, 0x3f34b4b5u, 0x3f35b5b6u, 0x3f36b6b7u, 0x3f37b7b8u,
-    0x3f38b8b9u, 0x3f39b9bau, 0x3f3ababbu, 0x3f3bbbbcu, 0x3f3cbcbdu, 0x3f3dbdbeu, 0x3f3ebebfu, 0x3f3fbfc0u,
-    0x3f40c0c1u, 0x3f41c1c2u, 0x3f42c2c3u, 0x3f43c3c4u, 0x3f44c4c5u, 0x3f45c5c6u, 0x3f46c6c7u, 0x3f47c7c8u,
-    0x3f48c8c9u, 0x3f49c9cau, 0x3f4acacbu, 0x3f4bcbccu, 0x3f4ccccdu, 0x3f4dcdceu, 0x3f4ececfu, 0x3f4fcfd0u,
-    0x3f50d0d1u, 0x3f51d1d2u, 0x3f52d2d3u, 0x3f53d3d4u, 0x3f54d4d5u, 0x3f55d5d6u, 0x3f56d6d7u, 0x3f57d7d8u,
-    0x3f58d8d9u, 0x3f59d9dau, 0x3f5adadbu, 0x3f5bdbdcu, 0x3f5cdcddu, 0x3f5ddddeu, 0x3f5ededfu, 0x3f5fdfe0u,
-    0x3f60e0e1u, 0x3f61e1e2u, 0x3f62e2e3u, 0x3f63e3e4u, 0x3f64e4e5u, 0x3f65e5e6u, 0x3f66e6e7u, 0x3f67e7e8u,
-    0x3f68e8e9u, 0x3f69e9eau, 0x3f6aeaebu, 0x3f6bebecu, 0x3f6cecedu, 0x3f6dedeeu, 0x3f6eeeefu, 0x3f6feff0u,
-    0x3f70f0f1u, 0x3f71f1f2u, 0x3f72f2f3u, 0x3f73f3f4u, 0x3f74f4f5u, 0x3f75f5f6u, 0x3f76f6f7u, 0x3f77f7f8u,
-    0x3f78f8f9u, 0x3f79f9fau, 0x3f7afafbu, 0x3f7bfbfcu, 0x3f7cfcfdu, 0x3f7dfdfeu, 0x3f7efeffu, 0x3f800000u,
-};
-#endif
+constexpr int K1_RAWP = 112;                 // raw-box row pitch (words) baked into the remap kernel when no tile needs more
 
 struct K1FastArgs {
     const uint8_t* frames;
@@ -476,47 +401,31 @@ __device__ __forceinline__ void store_at(float* base, int idx, float v) {
                  :: "l"(base), "r"(idx), "f"(v) : "memory");
 }
 
-__device__ __forceinline__ float div255_q(unsigned q, const unsigned char* divb);
-
-// One output pixel (3 channels) of cv2.resize's fixed-point bilinear (or the exact-2x area average) + /255.
-template <bool AREA>
-__device__ __forceinline__ void resize_px(const unsigned char* p0, const unsigned char* p1, unsigned a01, unsigned b0,
-                                          unsigned b1, const unsigned char* divb, float& v0, float& v1, float& v2) {
-    const unsigned t00 = *reinterpret_cast<const unsigned*>(p0), t01 = *reinterpret_cast<const unsigned*>(p0 + 4);
-    const unsigned t10 = *reinterpret_cast<const unsigned*>(p1), t11 = *reinterpret_cast<const unsigned*>(p1 + 4);
-    const unsigned bg0 = __byte_perm(t00, t01, 0x5140), rr0 = __byte_perm(t00, t01, 0x3362);
-    const unsigned bg1 = __byte_perm(t10, t11, 0x5140), rr1 = __byte_perm(t10, t11, 0x3362);
-    const unsigned S0b = __dp2a_lo(a01, bg0, 0u), S0g = __dp2a_hi(a01, bg0, 0u), S0r = __dp2a_lo(a01, rr0, 0u);
-    unsigned qb, qg, qr;                     // 4 * quantised value + (0..3): the byte offset into s_div after & ~3
-    if (AREA) {
-        qb = __dp2a_lo(a01, bg1, S0b + 2u); qg = __dp2a_hi(a01, bg1, S0g + 2u); qr = __dp2a_lo(a01, rr1, S0r + 2u);
-    } else {
-        const unsigned S1b = __dp2a_lo(a01, bg1, 0u), S1g = __dp2a_hi(a01, bg1, 0u), S1r = __dp2a_lo(a01, rr1, 0u);
-        // ((b0 (S0 >> 4)) >> 16) + ((b1 (S1 >> 4)) >> 16) + 2: PRMT takes both >> 16 at once, dp2a adds them.
-        // The plan guarantees a0 + a1 <= 2049 and b0 + b1 <= 2049, so the sum is <= 1022: no saturation needed.
-        qb = __dp2a_lo(__byte_perm(b0 * (S0b >> 4), b1 * (S1b >> 4), 0x7632), 0x0101u, 2u);
-        qg = __dp2a_lo(__byte_perm(b0 * (S0g >> 4), b1 * (S1g >> 4), 0x7632), 0x0101u, 2u);
-        qr = __dp2a_lo(__byte_perm(b0 * (S0r >> 4), b1 * (S1r >> 4), 0x7632), 0x0101u, 2u);
-    }
-    v0 = div255_q(qb, divb);
-    v1 = div255_q(qg, divb);
-    v2 = div255_q(qr, divb);
-}
-
-// float32(v) / 255.0f for q = 4 v + (0..3), v in 0..255, WITHOUT the table: x = float(4 v) is exact, 1/1020 is split
+// float32(v) / 255.0f for q = 4 v + (0..3), v in 0..255, without a table: x = float(4 v) is exact, 1/1020 is split
 // into c1 + c2 (c1 = RN(1/1020), c2 = RN(1/1020 - c1)), t = RN(x c2), y = RN(x c1 + t) (one FMA).  x c1 + x c2 differs
 // from the quotient by < 2^-48 relative, far below the distance of any v / 255 to a rounding boundary: all 256 values
 // were checked against numpy's float32 division with exact rational arithmetic (tools/check_div255.py), and
 // tests/test_gpu_parity.py::test_k1_bit_exact compares the kernel's output with cv2 + torch bit for bit.
 // K1 is bound by the L1 data pipe (shared-memory wavefronts), not by issue slots: 2 more instructions per value on the
 // otherwise idle FP32 pipe replace one table LDS (1.34 wavefronts measured, values in a warp collide on banks).
-__device__ __forceinline__ float div255_q(unsigned q, const unsigned char* divb) {
-#if VTI_K1_DIVFMA
+__device__ __forceinline__ float div255_q(unsigned q) {
     const float x = __uint2float_rn(q & 0x3FCu);
     return __fmaf_rn(x, __uint_as_float(0x3a808081u), __fmul_rn(x, __uint_as_float(0xae7efeffu)));
-#else
-    return *reinterpret_cast<const float*>(divb + (q & 0x3FCu));
-#endif
+}
+
+// One output pixel (3 channels) of the exact-2x area average + /255.
+__device__ __forceinline__ void area_px(const unsigned char* p0, const unsigned char* p1, unsigned a01, float& v0,
+                                        float& v1, float& v2) {
+    const unsigned t00 = *reinterpret_cast<const unsigned*>(p0), t01 = *reinterpret_cast<const unsigned*>(p0 + 4);
+    const unsigned t10 = *reinterpret_cast<const unsigned*>(p1), t11 = *reinterpret_cast<const unsigned*>(p1 + 4);
+    const unsigned bg0 = __byte_perm(t00, t01, 0x5140), rr0 = __byte_perm(t00, t01, 0x3362);
+    const unsigned bg1 = __byte_perm(t10, t11, 0x5140), rr1 = __byte_perm(t10, t11, 0x3362);
+    const unsigned S0b = __dp2a_lo(a01, bg0, 0u), S0g = __dp2a_hi(a01, bg0, 0u), S0r = __dp2a_lo(a01, rr0, 0u);
+    // 4 * quantised value + (0..3)
+    const unsigned qb = __dp2a_lo(a01, bg1, S0b + 2u), qg = __dp2a_hi(a01, bg1, S0g + 2u), qr = __dp2a_lo(a01, rr1, S0r + 2u);
+    v0 = div255_q(qb);
+    v1 = div255_q(qg);
+    v2 = div255_q(qr);
 }
 
 // One plane store.  LW_T > 0: the row pitch is a compile-time constant, the address is base + immediate.
@@ -531,9 +440,8 @@ __device__ __forceinline__ void store_px(float* base, int i, int oi, float v) {
 // row i + 1's upper one: 2 of 3 rows at 4/3), so its H pass is not reloaded and recomputed; the test is warp-uniform
 // (the row taps are per tile row).  CHECK: the strip may hold letterbox padding rows (offset -2) or end early.
 template <int LW_T, bool CHECK>
-__device__ __forceinline__ void resize_strip(const int4* rowtap, unsigned col, unsigned a01,
-                                             const unsigned char* divb, float* o0, float* o1, float* o2, int LW,
-                                             int n_out, float pad) {
+__device__ __forceinline__ void resize_strip(const int4* rowtap, unsigned col, unsigned a01, float* o0, float* o1,
+                                             float* o2, int LW, int n_out, float pad) {
     constexpr int RPT = FTY / (FT_THREADS / FTX);
     unsigned pb = 0u, pg = 0u, pr = 0u;                    // (H pass >> 4) of the source row at byte offset `have`
     int have = -1, oi = 0;
@@ -557,24 +465,23 @@ __device__ __forceinline__ void resize_strip(const int4* rowtap, unsigned col, u
         const unsigned nb = __dp2a_lo(a01, bg, 0u) >> 4, ng = __dp2a_hi(a01, bg, 0u) >> 4, nr = __dp2a_lo(a01, rr, 0u) >> 4;
         const unsigned b0 = (unsigned)rt.z, b1 = (unsigned)rt.w;
         unsigned qb, qg, qr;
-        // PRMT takes both >> 16 at once, dp2a adds them.  The plan guarantees b0 + b1 <= 2049: no saturation needed.
+        // ((b0 (S0 >> 4)) >> 16) + ((b1 (S1 >> 4)) >> 16) + 2: PRMT takes both >> 16 at once, dp2a adds them.
+        // The plan guarantees a0 + a1 <= 2049 and b0 + b1 <= 2049, so the sum is <= 1022: no saturation needed.
         qb = __dp2a_lo(__byte_perm(b0 * pb, b1 * nb, 0x7632), 0x0101u, 2u);
         qg = __dp2a_lo(__byte_perm(b0 * pg, b1 * ng, 0x7632), 0x0101u, 2u);
         qr = __dp2a_lo(__byte_perm(b0 * pr, b1 * nr, 0x7632), 0x0101u, 2u);
-        store_px<LW_T>(o0, i, oi, div255_q(qb, divb));
-        store_px<LW_T>(o1, i, oi, div255_q(qg, divb));
-        store_px<LW_T>(o2, i, oi, div255_q(qr, divb));
+        store_px<LW_T>(o0, i, oi, div255_q(qb));
+        store_px<LW_T>(o1, i, oi, div255_q(qg));
+        store_px<LW_T>(o2, i, oi, div255_q(qr));
         pb = nb; pg = ng; pr = nr; have = rt.y;
     }
 }
 
 // The resize phase of one thread: RPT output rows of one column, three planes, written to o0 / o0 + plane / o0 + 2 plane
-// with row pitch LW_T (compile time) or LW.  `o0` is either the thread's first pixel in the global output or in the
-// shared-memory output tile that a TMA store ships (row pitch FTX).
+// with row pitch LW_T (compile time) or LW; `o0` is the thread's first output pixel.
 template <bool AREA, int LW_T>
 __device__ __forceinline__ void resize_phase(const K1FastArgs& a, float* __restrict__ o0, size_t plane, int LW, int X, int Y0,
-                                             int j0, int nrows, int c_lo, const unsigned* s_und, const int4* s_rowtap,
-                                             const unsigned char* divb) {
+                                             int j0, int nrows, int c_lo, const unsigned* s_und, const int4* s_rowtap) {
     const float pad = __uint_as_float(0x3ee4e4e5u);            // float32(114) / 255.0f, the LetterBox border
     constexpr int RPT = FTY / (FT_THREADS / FTX);          // rows per thread
     float* __restrict__ o1 = o0 + plane;
@@ -595,28 +502,23 @@ __device__ __forceinline__ void resize_phase(const K1FastArgs& a, float* __restr
     const unsigned a01 = (unsigned)(unsigned short)a.tap_x_a[2 * rx] | ((unsigned)(unsigned short)a.tap_x_a[2 * rx + 1] << 16);
     const unsigned char* col = reinterpret_cast<const unsigned char*>(s_und) + (sx - c_lo) * 4;   // taps at col, col + 4
     const bool full = (ry0 >= 0) && (ry0 + RPT <= a.new_h) && (n_out == RPT);      // warp-uniform
-    if (!AREA && VTI_K1_HSHARE && full) {
-        resize_strip<LW_T, false>(s_rowtap + j0, smem_addr(col), a01, divb, o0, o1, o2, LW, RPT, pad);
-    } else if (!AREA && VTI_K1_HSHARE && VTI_K1_PADROWS) {
-        resize_strip<LW_T, true>(s_rowtap + j0, smem_addr(col), a01, divb, o0, o1, o2, LW, n_out, pad);
-    } else {
+    if (AREA) {
         for (int i = 0; i < n_out; ++i, oi += LW) {
             const int4 rt = s_rowtap[j0 + i];
             float v0 = pad, v1 = pad, v2 = pad;
-            if (rt.x >= 0) {
-                resize_px<AREA>(col + rt.x, col + rt.y, a01, (unsigned)rt.z, (unsigned)rt.w, divb, v0, v1, v2);
-            }
+            if (rt.x >= 0) area_px(col + rt.x, col + rt.y, a01, v0, v1, v2);
             store_px<LW_T>(o0, i, oi, v0); store_px<LW_T>(o1, i, oi, v1); store_px<LW_T>(o2, i, oi, v2);
         }
+    } else if (full) {
+        resize_strip<LW_T, false>(s_rowtap + j0, smem_addr(col), a01, o0, o1, o2, LW, RPT, pad);
+    } else {                                                // padding rows in the strip, or it ends at row LH
+        resize_strip<LW_T, true>(s_rowtap + j0, smem_addr(col), a01, o0, o1, o2, LW, n_out, pad);
     }
 }
 
-template <bool REMAP, bool AREA, int LW_T, int RAWP_T, bool TMAOUT>
-__global__ void __launch_bounds__(FT_THREADS, VTI_FT_MINB) k1_fast_kernel(const K1FastArgs a, const __grid_constant__ CUtensorMap omap) {
-    extern __shared__ __align__(128) unsigned s_dyn[];     // s_und [und_words], then the raw box (REMAP) / the output tile (TMAOUT)
-#if !VTI_K1_DIVFMA
-    __shared__ float s_div[256];
-#endif
+template <bool REMAP, bool AREA, int LW_T, int RAWP_T>
+__global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const K1FastArgs a) {
+    extern __shared__ __align__(128) unsigned s_dyn[];     // s_und [und_words], then the raw box (REMAP)
     __shared__ int4 s_rowtap[FTY];                          // (byte offset row0, byte offset row1, b0, b1)
 
     const int tid = threadIdx.x;
@@ -630,9 +532,6 @@ __global__ void __launch_bounds__(FT_THREADS, VTI_FT_MINB) k1_fast_kernel(const 
 
     const int4 h0 = __ldg(a.tile_hdr + 2 * tile), h1 = __ldg(a.tile_hdr + 2 * tile + 1);
     const int r_lo = h1.x, c_lo = h1.y, nrows = h1.z;
-#if !VTI_K1_DIVFMA
-    for (int i = tid; i < 256; i += FT_THREADS) s_div[i] = __uint_as_float(g_div255_bits[i]);
-#endif
     if (tid < FTY) {
         const int ry = Y0 + tid - a.top;
         int4 t = make_int4(-2, -2, 0, 0);                   // padding row (never equal to a real row offset)
@@ -680,33 +579,8 @@ __global__ void __launch_bounds__(FT_THREADS, VTI_FT_MINB) k1_fast_kernel(const 
     const int X = X0 + (tid & (FTX - 1));
     constexpr int RPT = FTY / (FT_THREADS / FTX);          // rows per thread
     const int j0 = (tid / FTX) * RPT;
-#if VTI_K1_DIVFMA
-    const unsigned char* divb = nullptr;
-#else
-    const unsigned char* divb = reinterpret_cast<const unsigned char*>(s_div);
-#endif
-    if (TMAOUT) {
-        // The tile's three planes are assembled in shared memory -- in the raw-box region, dead since the barrier above --
-        // and leave through ONE cp.async.bulk.tensor store ({FTX, FTY, 3} box of the [3 B][LH][LW] output; the TMA unit
-        // clips what lies outside the tensor): 24 shared stores per thread at immediate offsets instead of 24 global
-        // stores, and the 24.6 KB of a tile stay off the LSU data pipe (global stores drain at 64 B per cycle there).
-        float* s_out = reinterpret_cast<float*>(s_dyn + a.und_words);
-        if (X < LW)
-            resize_phase<AREA, FTX>(a, s_out + j0 * FTX + (tid & (FTX - 1)), (size_t)FTY * FTX, FTX, X, Y0, j0, nrows, c_lo,
-                                    s_und, s_rowtap, divb);
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%1, %2, %3}], [%4];"
-                         :: "l"(reinterpret_cast<unsigned long long>(&omap)), "r"(X0), "r"(Y0), "r"(3 * b), "r"(smem_addr(s_out))
-                         : "memory");
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");     // shared memory may go once it has been read
-        }
-        return;
-    }
     if (X >= LW) return;
-    resize_phase<AREA, LW_T>(a, out + (size_t)(Y0 + j0) * LW + X, (size_t)a.LH * LW, LW, X, Y0, j0, nrows, c_lo, s_und, s_rowtap, divb);
+    resize_phase<AREA, LW_T>(a, out + (size_t)(Y0 + j0) * LW + X, (size_t)a.LH * LW, LW, X, Y0, j0, nrows, c_lo, s_und, s_rowtap);
 }
 
 }  // namespace
@@ -725,7 +599,7 @@ static bool k1_fast_plan(vti_handle* h, const std::vector<int32_t>& xi, const st
     const int fw = h->p.frame_w, fh = h->p.frame_h;
     if (fw & 7) return false;
     if (h->resize_mode == 1) {
-        // no-saturation guarantee of resize_px, and the unconditional read of column sx + 1
+        // no-saturation guarantee of resize_strip, and the unconditional read of column sx + 1
         for (int d = 0; d < g.new_w; ++d) {
             if (xa[2 * d] < 0 || xa[2 * d + 1] < 0 || xa[2 * d] + xa[2 * d + 1] > 2049) return false;
             if (xi[d] + 1 > fw - 1 && xa[2 * d + 1] != 0) return false;
@@ -822,38 +696,35 @@ static bool k1_fast_plan(vti_handle* h, const std::vector<int32_t>& xi, const st
 
 // The one place that names every instantiation of the fast kernel: launch == 0 raises each one's dynamic
 // shared-memory limit (plan time), launch == 1 launches the one that matches the handle.
-template <bool REMAP, bool AREA, int LW_T, int RAWP_T, bool TMAOUT>
-static int k1_fast_one(const K1FastArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s, const CUtensorMap* om) {
-    if (!launch) return vti_raise_dyn_smem((const void*)k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, TMAOUT>, smem);
-    k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, TMAOUT><<<*grid, FT_THREADS, smem, s>>>(*f, *om);
+template <bool REMAP, bool AREA, int LW_T, int RAWP_T>
+static int k1_fast_one(const K1FastArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
+    if (!launch) return vti_raise_dyn_smem((const void*)k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T>, smem);
+    k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T><<<*grid, FT_THREADS, smem, s>>>(*f);
     return VTI_OK;
 }
-template <int LW_T, bool TMAOUT>
+template <int LW_T>
 static int k1_fast_lw(bool remap, bool area, int rawp, const K1FastArgs* f, int launch, const dim3* grid, size_t smem,
-                      cudaStream_t s, const CUtensorMap* om) {
+                      cudaStream_t s) {
     int rc = VTI_OK;
     const bool fixed = rawp == K1_RAWP;
-    if (!launch || (remap && area && fixed)) if ((rc = k1_fast_one<true, true, LW_T, K1_RAWP, TMAOUT>(f, launch, grid, smem, s, om))) return rc;
-    if (!launch || (remap && !area && fixed)) if ((rc = k1_fast_one<true, false, LW_T, K1_RAWP, TMAOUT>(f, launch, grid, smem, s, om))) return rc;
-    if (!launch || (remap && area && !fixed)) if ((rc = k1_fast_one<true, true, LW_T, 0, TMAOUT>(f, launch, grid, smem, s, om))) return rc;
-    if (!launch || (remap && !area && !fixed)) if ((rc = k1_fast_one<true, false, LW_T, 0, TMAOUT>(f, launch, grid, smem, s, om))) return rc;
-    if (!launch || (!remap && area)) if ((rc = k1_fast_one<false, true, LW_T, 0, TMAOUT>(f, launch, grid, smem, s, om))) return rc;
-    if (!launch || (!remap && !area)) if ((rc = k1_fast_one<false, false, LW_T, 0, TMAOUT>(f, launch, grid, smem, s, om))) return rc;
+    if (!launch || (remap && area && fixed)) if ((rc = k1_fast_one<true, true, LW_T, K1_RAWP>(f, launch, grid, smem, s))) return rc;
+    if (!launch || (remap && !area && fixed)) if ((rc = k1_fast_one<true, false, LW_T, K1_RAWP>(f, launch, grid, smem, s))) return rc;
+    if (!launch || (remap && area && !fixed)) if ((rc = k1_fast_one<true, true, LW_T, 0>(f, launch, grid, smem, s))) return rc;
+    if (!launch || (remap && !area && !fixed)) if ((rc = k1_fast_one<true, false, LW_T, 0>(f, launch, grid, smem, s))) return rc;
+    if (!launch || (!remap && area)) if ((rc = k1_fast_one<false, true, LW_T, 0>(f, launch, grid, smem, s))) return rc;
+    if (!launch || (!remap && !area)) if ((rc = k1_fast_one<false, false, LW_T, 0>(f, launch, grid, smem, s))) return rc;
     return rc;
 }
-// tma: the output tile leaves through a TMA tensor store (`om` = tensor map of this call's output buffer)
 static int k1_fast_dispatch(vti_handle* h, const K1FastArgs* f, int launch, const dim3* grid, size_t smem,
-                            cudaStream_t s = nullptr, bool tma = false, const CUtensorMap* om = nullptr) {
+                            cudaStream_t s = nullptr) {
     const bool remap = h->k1_mode == MODE_FAST_REMAP, area = h->resize_mode == 2;
     const int LW = h->g.LW, rawp = h->k1_raw_pitch;
     int rc = VTI_OK;
-    if (VTI_K1_TMAOUT && (!launch || tma)) if ((rc = k1_fast_lw<0, true>(remap, area, rawp, f, launch, grid, smem, s, om)) || tma) return rc;
-    static const CUtensorMap none = {};
-    if (!om) om = &none;
-    // imgsz 960 and 640 letterboxes (every BASELINE config) get the row pitch as a compile-time constant
-    if (VTI_K1_LWT && (!launch || LW == 960)) if ((rc = k1_fast_lw<960, false>(remap, area, rawp, f, launch, grid, smem, s, om))) return rc;
-    if (VTI_K1_LWT && (!launch || LW == 640)) if ((rc = k1_fast_lw<640, false>(remap, area, rawp, f, launch, grid, smem, s, om))) return rc;
-    if (!launch || !VTI_K1_LWT || (LW != 960 && LW != 640)) rc = k1_fast_lw<0, false>(remap, area, rawp, f, launch, grid, smem, s, om);
+    // imgsz 960 and 640 letterboxes (every BASELINE config) get the output row pitch as a compile-time constant: the
+    // plane stores take immediate offsets
+    if (!launch || LW == 960) if ((rc = k1_fast_lw<960>(remap, area, rawp, f, launch, grid, smem, s))) return rc;
+    if (!launch || LW == 640) if ((rc = k1_fast_lw<640>(remap, area, rawp, f, launch, grid, smem, s))) return rc;
+    if (!launch || (LW != 960 && LW != 640)) rc = k1_fast_lw<0>(remap, area, rawp, f, launch, grid, smem, s);
     return rc;
 }
 
@@ -870,12 +741,14 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
         size_t raw_words = 0;
         if (k1_fast_plan(h, xi, yi, xa, yb, und_ix, und_iy, hdr, lut, pitch_u, rows_u, raw_words, lut_stride, raw_pitch)) {
             const int und_words = (rows_u * pitch_u + 4 + FT_CHUNK - 1) / FT_CHUNK * FT_CHUNK;
-            if (VTI_K1_TMAOUT) raw_words = std::max(raw_words, (size_t)3 * FTY * FTX);      // the output tile reuses the raw-box region
+            // The measured configuration: the region past the footprint buffer is at least one output tile (3 x FTY x
+            // FTX floats, 24 KB), so the plain path (no raw box) asks for these 24 KB too.  This sets how many K1 CTAs
+            // share an SM with the post kernels (DESIGN.md 5a); dropping it is a change to measure on its own.
+            raw_words = std::max(raw_words, (size_t)3 * FTY * FTX);
             size_t smem = ((size_t)und_words + raw_words) * 4;
             // Leave room on every SM for the post kernels that run beside K1 (two streams): at most 4 resident K1 CTAs.
             // Measured: 5 CTAs/SM make K1 alone 5 % faster and the whole pre || post step 8 % slower.
-            if (getenv("VTI_K1_SMEM_FLOOR")) smem = std::max(smem, (size_t)atoi(getenv("VTI_K1_SMEM_FLOOR")));
-            else if (und_ix) smem = std::max(smem, (size_t)(46 * 1024 + 512));     // (measured with the remap path)
+            if (und_ix) smem = std::max(smem, (size_t)(46 * 1024 + 512));     // (measured with the remap path)
             if (smem <= 110 * 1024) {
                 h->k1_mode = und_ix ? MODE_FAST_REMAP : MODE_FAST_PLAIN;
                 h->k1_pitch_u = pitch_u; h->k1_rows_u = rows_u; h->k1_smem = smem;
@@ -975,16 +848,7 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cu
         f.und_words = h->k1_und_words; f.lut_stride = h->k1_lut_stride;
         f.raw_pitch = h->k1_raw_pitch;
         dim3 grid((f.LW + FTX - 1) / FTX, (f.LH + FTY - 1) / FTY, B);
-        // TMA output: a tensor map of THIS call's output buffer ([3 B][LH][LW] float32, box {FTX, FTY, 3}); any buffer that is
-        // not 16-byte aligned (or a toolkit without the encoder) takes the plain-store kernel instead
-        CUtensorMap om;
-        // OPT-IN (VTI_K1_TMA=1): measured on B200 the TMA form is bit-exact and 5 % SLOWER alone (203.6 vs 193.3 us per 64
-        // frames; the same 0.278 ms inside the whole step): the CTA has to stay resident until the TMA unit has read its
-        // 24.6 KB tile out of shared memory, which costs more SM-slot time than the 24 fire-and-forget STG per thread.
-        const bool tma = VTI_K1_TMAOUT && getenv("VTI_K1_TMA") && (reinterpret_cast<uintptr_t>(net_in) & 15) == 0 &&
-                         vti_encode_tmap_f32_3d(&om, net_in, (unsigned long long)f.LW, (unsigned long long)f.LH,
-                                                (unsigned long long)3 * B, FTX, FTY, 3);
-        int rc = k1_fast_dispatch(h, &f, 1, &grid, h->k1_smem, s, tma, tma ? &om : nullptr);
+        int rc = k1_fast_dispatch(h, &f, 1, &grid, h->k1_smem, s);
         if (rc) return rc;
         h->launches++;
         VTI_CUDA(cudaGetLastError());

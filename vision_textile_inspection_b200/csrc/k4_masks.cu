@@ -31,22 +31,17 @@
 #include <climits>
 #include <cstdlib>
 
-#include <cuda.h>
-
 #include "vti_internal.h"
 
 namespace {
 
-#ifndef VTI_K4_THREADS
-#define VTI_K4_THREADS 256
-#endif
-constexpr int K4_THREADS = VTI_K4_THREADS;
+constexpr int K4_THREADS = 256;
 constexpr int NWARP = K4_THREADS / 32;
 constexpr int UR = VTI_K4_UR, UC = VTI_K4_UC;
 constexpr int SCW = UC + 1;                 // corner columns per unit
 constexpr float MARGIN = 1e-5f;             // >> fp32 rounding of the lerp; cells within the margin are evaluated per pixel
-constexpr float MARGIN_B = 1e-3f;
-constexpr int MAX_DENSE_DETS = 1024;         // = the max_det ceiling of vti_create           // variant B: logits (|values| up to ~30) instead of probabilities
+constexpr float MARGIN_B = 1e-3f;           // variant B: logits (|values| up to ~30) instead of probabilities
+constexpr int MAX_DENSE_DETS = 1024;        // = the max_det ceiling of vti_create
 
 struct K4Args {
     const float* proto;         // [B][32][ph][pw]
@@ -257,131 +252,6 @@ __global__ void __launch_bounds__(K4_THREADS, 1024 / K4_THREADS) k4_units_kernel
 
 
 // ====================================================================================================================
-// TMA form of the unit kernel (opt-in, kept as a measured experiment: see vti_launch_k4).  A unit's prototype corner block is a 3-D box {TB_W columns, UR+1 rows, 32 channels} of
-// the [B*32][ph][pw] prototype tensor: ONE cp.async.bulk.tensor (TMA) brings it into shared memory, where the LDG
-// form needs 32 loads + 64 address instructions per lane and iteration.  Each warp double-buffers: the box of its next
-// unit is in flight (mbarrier with the byte count) while it contracts, classifies and reduces the current one, so the
-// L2/HBM latency that bounded the LDG form (issue slots 47-60 % used) is off the critical path.  Out-of-plane parts of
-// a box are zero-filled by the TMA unit and never read: the replicate clamp of the upsample is applied to the
-// shared-memory index.
-// ====================================================================================================================
-constexpr int TB_W = 24;                           // box columns: the box starts at the 16-byte-aligned column at or below
-                                                   // C0 - 1 (TMA needs 16-byte-aligned row starts), so 3 + UC + 1 = 20 <= 24
-constexpr int TB_H = UR + 1;
-constexpr int TB_FLOATS = VTI_NM * TB_H * TB_W;
-constexpr int TB_BYTES = TB_FLOATS * 4;            // 15 360 with UR = 4
-constexpr int T_WARPS = 3;                         // warps per CTA: 3 x 2 buffers x 15 KB = 90 KB, two CTAs per SM
-static_assert(TB_BYTES % 128 == 0, "TMA destination alignment");
-
-__device__ __forceinline__ unsigned k4_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-
-struct UnitGeo {
-    int b, k, R0, C0, nr, ncw;
-    bool fabric;
-    VtiWindow w;
-};
-__device__ __forceinline__ UnitGeo unit_geo(const uint4 un) {
-    UnitGeo g;
-    g.b = (int)(un.x & 0x7FFFu); g.k = (int)(un.x >> 16);
-    g.fabric = (un.x & 0x8000u) != 0u;
-    const int br = (int)(un.y & 0xFFFFu), bc = (int)(un.y >> 16);
-    g.w.cx_lo = (int)(un.z & 0xFFFFu); g.w.cy_lo = (int)(un.z >> 16);
-    g.w.cx_hi = (int)(un.w & 0xFFFFu); g.w.cy_hi = (int)(un.w >> 16);
-    g.w.empty = false;
-    g.R0 = g.w.cy_lo + br * UR; g.C0 = g.w.cx_lo + bc * UC;
-    const int R1 = min(g.R0 + UR - 1, g.w.cy_hi + 1), C1 = min(g.C0 + UC - 1, g.w.cx_hi + 1);
-    g.nr = R1 - g.R0 + 2; g.ncw = C1 - g.C0 + 2;
-    return g;
-}
-
-template <bool EXPORT>
-__global__ void __launch_bounds__(T_WARPS * 32, 2) k4_tma_kernel(const __grid_constant__ CUtensorMap tmap, const K4Args a) {
-    extern __shared__ __align__(128) float s_box[];                     // [T_WARPS][2][TB_FLOATS]
-    __shared__ __align__(8) unsigned long long s_bar[T_WARPS][2];
-    __shared__ float s_c[T_WARPS][(UR + 1) * SCW];
-    __shared__ __align__(16) float s_coef[T_WARPS][VTI_NM];
-    __shared__ int s_envw[T_WARPS][4 * UC];
-
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int total = *a.unit_count;
-    const int nwarps = gridDim.x * T_WARPS;
-    int u = blockIdx.x * T_WARPS + warp;
-    if (u >= total) return;                                             // (no block-wide barrier anywhere below)
-    float* buf0 = s_box + (size_t)warp * 2 * TB_FLOATS;
-    float* sc = s_c[warp];
-    const unsigned long long tmap_addr = reinterpret_cast<unsigned long long>(&tmap);
-    if (lane == 0) {
-        asm volatile("mbarrier.init.shared.b64 [%0], 1;" :: "r"(k4_smem_u32(&s_bar[warp][0])) : "memory");
-        asm volatile("mbarrier.init.shared.b64 [%0], 1;" :: "r"(k4_smem_u32(&s_bar[warp][1])) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-    auto issue = [&](const UnitGeo& g, int slot) {                      // lane 0: arm the barrier, start the box copy
-        const unsigned bar = k4_smem_u32(&s_bar[warp][slot]);
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"((unsigned)TB_BYTES) : "memory");
-        asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                     :: "r"(k4_smem_u32(buf0 + (size_t)slot * TB_FLOATS)), "l"(tmap_addr), "r"((g.C0 - 1) & ~3), "r"(g.R0 - 1),
-                        "r"(g.b * VTI_NM), "r"(bar) : "memory");
-    };
-    UnitGeo g = unit_geo(__ldg(a.units + u));
-    if (lane == 0) issue(g, 0);
-    unsigned parity0 = 0u, parity1 = 0u;
-    for (int it = 0;; ++it) {
-        const int cur = it & 1;
-        const int un = u + nwarps;
-        const bool more = un < total;
-        UnitGeo gn = g;
-        if (more) {
-            gn = unit_geo(__ldg(a.units + un));
-            if (lane == 0) issue(gn, cur ^ 1);                          // that buffer was consumed one iteration ago
-        }
-        // this unit's coefficients and envelope scratch while its box lands
-        vti_det* __restrict__ det = a.dets + (size_t)g.b * a.max_det + g.k;
-        s_coef[warp][lane] = __ldg(a.det_coef + ((size_t)g.b * a.max_det + g.k) * VTI_NM + lane);
-        if (g.fabric) { s_envw[warp][lane] = a.upper ? INT_MAX : -1; s_envw[warp][lane + 32] = a.upper ? INT_MAX : -1; }
-        {
-            const unsigned bar = k4_smem_u32(&s_bar[warp][cur]), par = cur ? parity1 : parity0;
-            asm volatile(
-                "{\n\t.reg .pred p;\n\t"
-                "W_%=:\n\t"
-                "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                "@p bra D_%=;\n\t"
-                "bra W_%=;\n\t"
-                "D_%=:\n\t}"
-                :: "r"(bar), "r"(par) : "memory");
-            if (cur) parity1 ^= 1u; else parity0 ^= 1u;
-        }
-        __syncwarp();
-        // (1) logits -> sigmoid -> crop over the corner rectangle, prototype values from the box in shared memory
-        const float* box = buf0 + (size_t)cur * TB_FLOATS;
-        const float inv_ncw = 1.0f / (float)g.ncw;
-        for (int i = lane; i < g.nr * g.ncw; i += 32) {
-            const int r = (int)(((float)i + 0.5f) * inv_ncw), c = i - r * g.ncw;
-            const int py = min(max(g.R0 - 1 + r, 0), a.ph - 1), px = min(max(g.C0 - 1 + c, 0), a.pw - 1);
-            float v = 0.0f;
-            if (py >= g.w.cy_lo && py <= g.w.cy_hi && px >= g.w.cx_lo && px <= g.w.cx_hi) {
-                const float* src = box + (py - (g.R0 - 1)) * TB_W + (px - ((g.C0 - 1) & ~3));   // replicate clamp on the index
-                float acc = 0.0f;
-#pragma unroll
-                for (int q = 0; q < VTI_NM; q += 4) {
-                    const float4 cf = *reinterpret_cast<const float4*>(&s_coef[warp][q]);
-                    acc = fmaf(cf.x, src[(q + 0) * TB_H * TB_W], acc); acc = fmaf(cf.y, src[(q + 1) * TB_H * TB_W], acc);
-                    acc = fmaf(cf.z, src[(q + 2) * TB_H * TB_W], acc); acc = fmaf(cf.w, src[(q + 3) * TB_H * TB_W], acc);
-                }
-                v = 1.0f / (1.0f + expf(-acc));
-            }
-            sc[r * SCW + c] = v;
-        }
-        __syncwarp();
-        unit_cells<EXPORT, false>(a, g.b, g.k, det, g.fabric, g.R0, g.C0, g.nr, g.ncw, sc, s_envw[warp], lane);
-        __syncwarp();                                                   // everyone is done with box[cur], s_c, s_coef
-        if (!more) break;
-        g = gn; u = un;
-    }
-}
-
-
-// ====================================================================================================================
 // Dense tile form on the 5th-generation tensor cores (tcgen05.mma kind::tf32, accumulators in TMEM).
 //
 // The north star names the N x 32 @ 32 x (ph*pw) contraction as the one tensor-core candidate.  On the configured
@@ -408,6 +278,7 @@ constexpr int DB_BYTES = DN * VTI_NM * 4;           // 8 KB per B part
 constexpr size_t K4_DENSE_SMEM = 2 * DA_BYTES + 2 * DB_BYTES + (size_t)DN * DT_M * 4 + 1024;   // + s_c, + alignment slack
 static_assert(DT_CR * DT_CC <= DT_M, "tile corners must fit the MMA M");
 
+__device__ __forceinline__ unsigned k4_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ unsigned tf32_rna(float x) {
     unsigned r;
     asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
@@ -628,51 +499,12 @@ __global__ void __launch_bounds__(256) k4_fetch_proto_kernel(const float* __rest
 
 }  // namespace
 
-typedef CUresult (*vti_encode_tiled_t)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                       const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                       CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static vti_encode_tiled_t g_encode_tiled = nullptr;
-constexpr size_t K4_TMA_SMEM = (size_t)T_WARPS * 2 * TB_BYTES;
-
-// 3-D float32 tensor map (innermost dimension first) with box {b0, b1, b2}; false if the driver entry point is missing
-bool vti_encode_tmap_f32_3d(CUtensorMap* m, const void* base, unsigned long long d0, unsigned long long d1,
-                            unsigned long long d2, unsigned b0, unsigned b1, unsigned b2) {
-    if (!g_encode_tiled) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            g_encode_tiled = reinterpret_cast<vti_encode_tiled_t>(fn);
-        else
-            cudaGetLastError();
-        if (!g_encode_tiled) return false;
-    }
-    const cuuint64_t gdim[3] = {d0, d1, d2};
-    const cuuint64_t gstr[2] = {d0 * 4, d0 * d1 * 4};
-    const cuuint32_t box[3] = {b0, b1, b2}, estr[3] = {1, 1, 1};
-    return g_encode_tiled(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<void*>(base), gdim, gstr, box, estr,
-                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                          CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-
 int vti_k4_prepare() {
-    // cuTensorMapEncodeTiled through the runtime's driver entry point: no link-time dependency on libcuda
-    if (!g_encode_tiled) {
-        void* fn = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q) == cudaSuccess &&
-            q == cudaDriverEntryPointSuccess)
-            g_encode_tiled = reinterpret_cast<vti_encode_tiled_t>(fn);
-        else
-            cudaGetLastError();
-    }
     int rc;
     if ((rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<true, true>, K4_DENSE_SMEM)) ||
         (rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<true, false>, K4_DENSE_SMEM)) ||
         (rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<false, true>, K4_DENSE_SMEM)) ||
         (rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<false, false>, K4_DENSE_SMEM))) return rc;
-    VTI_CUDA(cudaFuncSetAttribute(k4_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K4_TMA_SMEM));
-    VTI_CUDA(cudaFuncSetAttribute(k4_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)K4_TMA_SMEM));
     return VTI_OK;
 }
 
@@ -694,38 +526,18 @@ int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const
         k4_zero_masks_kernel<<<dim3(a.max_det, B), 256, 0, s>>>(masks, counts, a.max_det, wpm);
         h->launches++;
     }
-    // TMA form: the prototype tensor as [B*32][ph][pw] float32, boxes of {TB_W, UR+1, 32}
-    CUtensorMap tmap;
-    // OPT-IN (VTI_K4_TMA=1): measured on B200 the TMA form is 2x SLOWER than the LDG form (137 vs 70 us per 64 frames):
-    // a unit's box is 128 rows of 96 bytes, and the TMA unit's per-row request rate, not bandwidth or latency, bounds it.
+    // Alone, K4 is fastest with four 8-warp CTAs per SM (66 vs 88 us on cfg2), but those fill every register file and
+    // K1 -- which runs beside it on the pre stream -- then waits for K4 to finish.  Two CTAs per SM leave half of each SM
+    // to K1: the K1 || K2-K5 step is 2.3 % faster on cfg2 / cfg3.  When K1 has little to do (no remap, no resize: cfg4)
+    // K4 is on the critical path and keeps the four.
     const bool vb = h->p.mask_variant == 1;
-    bool tma = g_encode_tiled && getenv("VTI_K4_TMA") && !vb && (reinterpret_cast<uintptr_t>(proto) & 15) == 0 &&
-               (a.pw % 4) == 0;
-    if (tma) {
-        const cuuint64_t gdim[3] = {(cuuint64_t)a.pw, (cuuint64_t)a.ph, (cuuint64_t)VTI_NM * B};
-        const cuuint64_t gstr[2] = {(cuuint64_t)a.pw * 4, (cuuint64_t)a.pw * a.ph * 4};
-        const cuuint32_t box[3] = {TB_W, TB_H, VTI_NM}, estr[3] = {1, 1, 1};
-        tma = g_encode_tiled(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(proto), gdim, gstr, box, estr,
-                             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-    }
-    if (tma) {
-        const int grid = 2 * h->num_sms;                   // two 4-warp CTAs per SM, grid-stride over the unit list
-        if (masks) k4_tma_kernel<true><<<grid, T_WARPS * 32, K4_TMA_SMEM, s>>>(tmap, a);
-        else k4_tma_kernel<false><<<grid, T_WARPS * 32, K4_TMA_SMEM, s>>>(tmap, a);
-    } else {
-        // LDG form.  Alone, K4 is fastest with four 8-warp CTAs per SM (66 vs 88 us on cfg2), but those fill every
-        // register file and K1 -- which runs beside it on the pre stream -- then waits for K4 to finish.  Two CTAs per
-        // SM leave half of each SM to K1: the K1 || K2-K5 step is 2.3 % faster on cfg2 / cfg3.  When K1 has little to do
-        // (no remap, no resize: cfg4) K4 is on the critical path and keeps the four.  VTI_K4_GRID overrides.
-        const bool k1_heavy = h->p.undistort || h->p.frame_w != h->g.new_w || h->p.frame_h != h->g.new_h;
-        const int grid = (getenv("VTI_K4_GRID") ? atoi(getenv("VTI_K4_GRID")) : (k1_heavy ? 2 : 4)) * h->num_sms;
-        if (h->p.k4_dense == 2) { /* every frame goes through the tile form below: K3 emitted no units */ }
-        else if (masks && vb) k4_units_kernel<true, true><<<grid, K4_THREADS, 0, s>>>(a);
-        else if (masks) k4_units_kernel<true, false><<<grid, K4_THREADS, 0, s>>>(a);
-        else if (vb) k4_units_kernel<false, true><<<grid, K4_THREADS, 0, s>>>(a);
-        else k4_units_kernel<false, false><<<grid, K4_THREADS, 0, s>>>(a);
-    }
+    const bool k1_heavy = h->p.undistort || h->p.frame_w != h->g.new_w || h->p.frame_h != h->g.new_h;
+    const int grid = (k1_heavy ? 2 : 4) * h->num_sms;
+    if (h->p.k4_dense == 2) { /* every frame goes through the tile form below: K3 emitted no units */ }
+    else if (masks && vb) k4_units_kernel<true, true><<<grid, K4_THREADS, 0, s>>>(a);
+    else if (masks) k4_units_kernel<true, false><<<grid, K4_THREADS, 0, s>>>(a);
+    else if (vb) k4_units_kernel<false, true><<<grid, K4_THREADS, 0, s>>>(a);
+    else k4_units_kernel<false, false><<<grid, K4_THREADS, 0, s>>>(a);
     if (h->p.k4_dense != 2) h->launches++;
     if (h->p.k4_dense) {
         // tcgen05 tile form for the frames K3 flagged: one CTA per (tile, frame); CTAs of other frames / empty tiles exit
