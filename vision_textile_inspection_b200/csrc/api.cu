@@ -8,18 +8,12 @@
 #include <climits>
 #include <cmath>
 #include <cstdlib>
-#include <cstring>
+#include <initializer_list>
 #include <map>
 #include <mutex>
 #include <utility>
 
 #include "vti_internal.h"
-
-size_t vti_k3_smem_bytes(int cap);
-int vti_k3_prepare(int cap);
-int vti_k3_cap_pad(int cap);
-int vti_k4_prepare();
-int vti_k5_prepare(int max_det);
 
 static thread_local std::string g_err;
 void vti_set_error(const std::string& s) { g_err = s; }
@@ -147,14 +141,7 @@ extern "C" int vti_plan_nearest_map(int dst_n, int src_n, int32_t* map) {
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-template <typename T>
-static int upload(T** dptr, const std::vector<T>& v) {
-    VTI_CUDA(cudaMalloc((void**)dptr, sizeof(T) * (v.empty() ? 1 : v.size())));
-    if (!v.empty()) VTI_CUDA(cudaMemcpy(*dptr, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
-    return VTI_OK;
-}
-
-static int build_axis_lut(int frame_n, int lb_n, AxisLut* lut, int32_t** d_map) {
+static int build_axis_lut(vti_handle* h, int frame_n, int lb_n, AxisLut* lut, int32_t** d_map) {
     std::vector<int32_t> map(frame_n), cnt(lb_n, 0), sum(lb_n, 0), first(lb_n, INT_MAX), last(lb_n, -1);
     vti_plan_nearest_map(frame_n, lb_n, map.data());
     for (int d = 0; d < frame_n; ++d) {
@@ -164,11 +151,6 @@ static int build_axis_lut(int frame_n, int lb_n, AxisLut* lut, int32_t** d_map) 
         if (d < first[s]) first[s] = d;
         if (d > last[s]) last[s] = d;
     }
-    int rc;
-    if ((rc = upload(&lut->cnt, cnt))) return rc;
-    if ((rc = upload(&lut->sum, sum))) return rc;
-    if ((rc = upload(&lut->first, first))) return rc;
-    if ((rc = upload(&lut->last, last))) return rc;
     std::vector<int32_t> pc(lb_n + 1, 0), ps(lb_n + 1, 0), prev_last(lb_n, -1), next_first(lb_n, INT_MAX);
     for (int i = 0; i < lb_n; ++i) {
         pc[i + 1] = pc[i] + cnt[i];
@@ -176,31 +158,136 @@ static int build_axis_lut(int frame_n, int lb_n, AxisLut* lut, int32_t** d_map) 
         prev_last[i] = std::max(i ? prev_last[i - 1] : -1, last[i]);
     }
     for (int i = lb_n - 1; i >= 0; --i) next_first[i] = std::min(i + 1 < lb_n ? next_first[i + 1] : INT_MAX, first[i]);
-    if ((rc = upload(&lut->pc, pc)) || (rc = upload(&lut->ps, ps)) || (rc = upload(&lut->prev_last, prev_last)) ||
-        (rc = upload(&lut->next_first, next_first))) return rc;
-    if (d_map) return upload(d_map, map);
+    int rc;
+    if ((rc = vti_upload(h, &lut->cnt, cnt)) || (rc = vti_upload(h, &lut->sum, sum)) || (rc = vti_upload(h, &lut->first, first)) ||
+        (rc = vti_upload(h, &lut->last, last)) || (rc = vti_upload(h, &lut->pc, pc)) || (rc = vti_upload(h, &lut->ps, ps)) ||
+        (rc = vti_upload(h, &lut->prev_last, prev_last)) || (rc = vti_upload(h, &lut->next_first, next_first))) return rc;
+    if (d_map) return vti_upload(h, d_map, map);
     return VTI_OK;
+}
+
+static int create_events(cudaEvent_t* ev, int n, unsigned flags) {
+    for (int i = 0; i < n; ++i) VTI_CUDA(cudaEventCreateWithFlags(&ev[i], flags));
+    return VTI_OK;
+}
+
+static void destroy_events(cudaEvent_t* ev, int n) {
+    for (int i = 0; i < n; ++i)
+        if (ev[i]) { cudaEventDestroy(ev[i]); ev[i] = nullptr; }
+}
+
+// frees the handle's allocations past the first `keep`, and the streams and events of the host-buffer path
+static void release_from(vti_handle* h, size_t keep) {
+    for (size_t i = keep; i < h->allocs.size(); ++i) cudaFree(h->allocs[i]);
+    h->allocs.resize(keep);
+    if (h->own_stream) cudaStreamDestroy(h->own_stream);
+    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
+    h->own_stream = h->copy_stream = nullptr;
+    destroy_events(h->chunk_ev, 4);
 }
 
 extern "C" void vti_destroy(vti_handle* h) {
     if (!h) return;
+    int caller = h->device;
+    cudaGetDevice(&caller);
     cudaSetDevice(h->device);
-    void* ptrs[] = {h->d_tap_x_idx, h->d_tap_x_a, h->d_tap_y_i, h->d_tap_y_b, h->d_und_lut, h->lutY.cnt, h->lutY.sum,
-                    h->lutY.first, h->lutY.last, h->lutX.cnt, h->lutX.sum, h->lutX.first, h->lutX.last, h->d_xmap,
-                    h->lutY.pc, h->lutY.ps, h->lutY.prev_last, h->lutY.next_first, h->lutX.pc, h->lutX.ps,
-                    h->lutX.prev_last, h->lutX.next_first,
-                    h->d_cand_count, h->d_cand_key, h->d_cand_box, h->d_det_coef, h->d_env, h->d_env_frame, h->d_flags,
-                    h->d_yuyv, h->d_frames, h->d_net_in, h->d_p[0], h->d_p[1], h->d_p[2], h->d_coef, h->d_proto, h->d_dets,
-                    h->d_counts, h->d_results, h->d_k1_tiles, h->d_k1_lut, h->d_units, h->d_proto_bbox, h->d_dense};
-    for (void* p : ptrs)
-        if (p) cudaFree(p);
-    if (h->own_stream) cudaStreamDestroy(h->own_stream);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    for (int i = 0; i < 4; ++i)
-        if (h->chunk_ev[i]) cudaEventDestroy(h->chunk_ev[i]);
-    for (int i = 0; i < 8; ++i)
-        if (h->ev[i]) cudaEventDestroy(h->ev[i]);
+    release_from(h, 0);
+    destroy_events(h->ev, 8);
+    if (caller != h->device) cudaSetDevice(caller);
     delete h;
+}
+
+// vti_create after the argument checks; on failure vti_create destroys the partial handle
+static int init_handle(vti_handle* h, const vti_params* p) {
+    VTI_CUDA(cudaGetDevice(&h->device));
+    VTI_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
+    h->p = *p;
+    int rc = vti_plan_geometry(p->frame_h, p->frame_w, p->imgsz, p->stride, p->max_det, p->max_candidates, &h->g);
+    if (rc) return rc;
+    {
+        // K4 accumulates a work unit's moments (<= 1024 letterbox pixels, each standing for up to my x mx frame pixels
+        // at coordinates < max(h, w)) in 32 bits before its 64-bit atomics
+        const unsigned long long my = (p->frame_h + h->g.LH - 1) / h->g.LH + 1, mx = (p->frame_w + h->g.LW - 1) / h->g.LW + 1;
+        if (1024ull * my * mx * (unsigned long long)std::max(p->frame_h, p->frame_w) >= (1ull << 31)) {
+            vti_set_error("vti_create: frame too large for the imgsz (mask moments would overflow a work unit's 32-bit sums)");
+            return VTI_EINVAL;
+        }
+    }
+    const vti_geometry& g = h->g;
+    const int fh = p->frame_h, fw = p->frame_w;
+    h->all_dets_env = getenv("VTI_ALL_DETS") != nullptr;
+    if (p->variant == 0 && p->roi_enabled) {                // measurement.py:220-238
+        const int x_min = std::clamp(p->roi_x_min, 0, fw - 1), x_max = std::clamp(p->roi_x_max, 0, fw - 1);
+        const int y_min = std::clamp(p->roi_y_min, 0, fh - 1), y_max = std::clamp(p->roi_y_max, 0, fh - 1);
+        if (x_min < x_max && y_min < y_max) h->roi = VtiRoi{1, x_min, y_min, x_max, y_max};
+    }
+
+    // ---- K1 tables
+    std::vector<int32_t> xi(g.new_w), yi(2 * (size_t)g.new_h);
+    std::vector<int16_t> xa(2 * (size_t)g.new_w), yb(2 * (size_t)g.new_h);
+    if (fw == 2 * g.new_w && fh == 2 * g.new_h) {
+        h->resize_mode = 2;                                  // OpenCV's silent INTER_AREA switch
+        for (int d = 0; d < g.new_w; ++d) { xi[d] = 2 * d; xa[2 * d] = 1; xa[2 * d + 1] = 1; }
+        for (int d = 0; d < g.new_h; ++d) { yi[2 * d] = 2 * d; yi[2 * d + 1] = 2 * d + 1; yb[2 * d] = 1; yb[2 * d + 1] = 1; }
+    } else {
+        h->resize_mode = 1;
+        std::vector<int32_t> i0(g.new_h), i1(g.new_h);
+        std::vector<int16_t> a0(g.new_w), a1(g.new_w), b0(g.new_h), b1(g.new_h);
+        if (fw == g.new_w && fh == g.new_h) {                // LetterBox skips cv2.resize: identity taps
+            for (int d = 0; d < g.new_w; ++d) { xi[d] = d; a0[d] = 2048; a1[d] = 0; }
+            for (int d = 0; d < g.new_h; ++d) { i0[d] = d; i1[d] = d; b0[d] = 2048; b1[d] = 0; }
+        } else {
+            vti_plan_resize_taps_x(fw, g.new_w, xi.data(), a0.data(), a1.data());
+            vti_plan_resize_taps_y(fh, g.new_h, i0.data(), i1.data(), b0.data(), b1.data());
+        }
+        for (int d = 0; d < g.new_w; ++d) { xa[2 * d] = a0[d]; xa[2 * d + 1] = a1[d]; }
+        for (int d = 0; d < g.new_h; ++d) { yi[2 * d] = i0[d]; yi[2 * d + 1] = i1[d]; yb[2 * d] = b0[d]; yb[2 * d + 1] = b1[d]; }
+    }
+    if ((rc = vti_upload(h, &h->d_tap_x_idx, xi)) || (rc = vti_upload(h, &h->d_tap_x_a, xa)) ||
+        (rc = vti_upload(h, &h->d_tap_y_i, yi)) || (rc = vti_upload(h, &h->d_tap_y_b, yb))) return rc;
+    {
+        std::vector<int32_t> ix, iy;
+        if (p->undistort) {
+            ix.resize((size_t)fh * fw); iy.resize((size_t)fh * fw);
+            std::vector<int32_t> packed((size_t)fh * fw);
+            vti_plan_undistort_map(p->K, p->dist, fh, fw, ix.data(), iy.data());
+            for (int v = 0; v < fh; ++v)
+                for (int u = 0; u < fw; ++u) {
+                    const size_t i = (size_t)v * fw + u;
+                    const int dx = ix[i] - 32 * u, dy = iy[i] - 32 * v;
+                    if (dx < -32768 || dx > 32767 || dy < -32768 || dy > 32767) {
+                        vti_set_error("vti_create: lens displacement exceeds +-1024 px, unsupported");
+                        return VTI_EINVAL;
+                    }
+                    packed[i] = (int32_t)(((uint32_t)(uint16_t)(int16_t)dy << 16) | (uint32_t)(uint16_t)(int16_t)dx);
+                }
+            if ((rc = vti_upload(h, &h->d_und_lut, packed))) return rc;
+        }
+        if ((rc = vti_k1_plan(h, xi, yi, xa, yb, p->undistort ? &ix : nullptr, p->undistort ? &iy : nullptr))) return rc;
+    }
+    // ---- measurement tables
+    if ((rc = build_axis_lut(h, fh, g.LH, &h->lutY, nullptr)) || (rc = build_axis_lut(h, fw, g.LW, &h->lutX, &h->d_xmap)))
+        return rc;
+    // ---- post scratch
+    const size_t B = p->max_batch;
+    auto alloc = [&](auto** ptr, size_t bytes) { if (!rc) rc = vti_alloc(h, ptr, bytes); };
+    alloc(&h->d_cand_count, sizeof(int32_t) * (B + 1));
+    alloc(&h->d_cand_key, sizeof(unsigned long long) * B * vti_k3_cap_pad(g.max_candidates));
+    alloc(&h->d_cand_box, sizeof(float4) * B * g.A);
+    alloc(&h->d_det_coef, sizeof(float) * B * p->max_det * VTI_NM);
+    alloc(&h->d_env, sizeof(int32_t) * B * g.LW);
+    alloc(&h->d_env_frame, sizeof(int32_t) * B * fw);
+    alloc(&h->d_flags, sizeof(int32_t) * B);
+    for (int l = 0; l < 3; ++l) h->head_floats[l] = (size_t)(64 + p->nc) * g.lvl_h[l] * g.lvl_w[l];
+    h->head_floats[3] = (size_t)VTI_NM * g.A;
+    h->head_floats[4] = (size_t)VTI_NM * g.ph * g.pw;
+    h->units_per_det = ((g.ph + 1 + VTI_K4_UR - 1) / VTI_K4_UR) * ((g.pw + 1 + VTI_K4_UC - 1) / VTI_K4_UC);
+    alloc(&h->d_units, sizeof(uint4) * B * p->max_det * h->units_per_det);
+    alloc(&h->d_proto_bbox, sizeof(int4) * B);
+    alloc(&h->d_dense, sizeof(int32_t) * B);
+    if (rc) return rc;
+    if ((rc = vti_k3_prepare(g.max_candidates)) || (rc = vti_k4_prepare()) || (rc = vti_k5_prepare(p->max_det))) return rc;
+    return VTI_OK;
 }
 
 extern "C" int vti_create(const vti_params* p, vti_handle** out) {
@@ -225,98 +312,8 @@ extern "C" int vti_create(const vti_params* p, vti_handle** out) {
         return VTI_ENODEV;
     }
     vti_handle* h = new vti_handle();
-    std::memset((void*)h, 0, sizeof(*h));
-    h->p = *p;
-    int rc = vti_plan_geometry(p->frame_h, p->frame_w, p->imgsz, p->stride, p->max_det, p->max_candidates, &h->g);
-    if (rc) { delete h; return rc; }
-    {
-        // K4 accumulates a work unit's moments (<= 1024 letterbox pixels, each standing for up to my x mx frame pixels
-        // at coordinates < max(h, w)) in 32 bits before its 64-bit atomics
-        const unsigned long long my = (p->frame_h + h->g.LH - 1) / h->g.LH + 1, mx = (p->frame_w + h->g.LW - 1) / h->g.LW + 1;
-        if (1024ull * my * mx * (unsigned long long)std::max(p->frame_h, p->frame_w) >= (1ull << 31)) {
-            vti_set_error("vti_create: frame too large for the imgsz (mask moments would overflow a work unit's 32-bit sums)");
-            delete h;
-            return VTI_EINVAL;
-        }
-    }
-    VTI_CUDA(cudaGetDevice(&h->device));
-    VTI_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
-    const vti_geometry& g = h->g;
-    const int fh = p->frame_h, fw = p->frame_w;
-
-    // ---- K1 tables
-    std::vector<int32_t> xi(g.new_w), yi(2 * (size_t)g.new_h);
-    std::vector<int16_t> xa(2 * (size_t)g.new_w), yb(2 * (size_t)g.new_h);
-    if (fw == 2 * g.new_w && fh == 2 * g.new_h) {
-        h->resize_mode = 2;                                  // OpenCV's silent INTER_AREA switch
-        for (int d = 0; d < g.new_w; ++d) { xi[d] = 2 * d; xa[2 * d] = 1; xa[2 * d + 1] = 1; }
-        for (int d = 0; d < g.new_h; ++d) { yi[2 * d] = 2 * d; yi[2 * d + 1] = 2 * d + 1; yb[2 * d] = 1; yb[2 * d + 1] = 1; }
-    } else {
-        h->resize_mode = 1;
-        std::vector<int32_t> i0(g.new_h), i1(g.new_h);
-        std::vector<int16_t> a0(g.new_w), a1(g.new_w), b0(g.new_h), b1(g.new_h);
-        if (fw == g.new_w && fh == g.new_h) {                // LetterBox skips cv2.resize: identity taps
-            for (int d = 0; d < g.new_w; ++d) { xi[d] = d; a0[d] = 2048; a1[d] = 0; }
-            for (int d = 0; d < g.new_h; ++d) { i0[d] = d; i1[d] = d; b0[d] = 2048; b1[d] = 0; }
-        } else {
-            vti_plan_resize_taps_x(fw, g.new_w, xi.data(), a0.data(), a1.data());
-            vti_plan_resize_taps_y(fh, g.new_h, i0.data(), i1.data(), b0.data(), b1.data());
-        }
-        for (int d = 0; d < g.new_w; ++d) { xa[2 * d] = a0[d]; xa[2 * d + 1] = a1[d]; }
-        for (int d = 0; d < g.new_h; ++d) { yi[2 * d] = i0[d]; yi[2 * d + 1] = i1[d]; yb[2 * d] = b0[d]; yb[2 * d + 1] = b1[d]; }
-    }
-    if ((rc = upload(&h->d_tap_x_idx, xi)) || (rc = upload(&h->d_tap_x_a, xa)) || (rc = upload(&h->d_tap_y_i, yi)) ||
-        (rc = upload(&h->d_tap_y_b, yb))) { vti_destroy(h); return rc; }
-    {
-        std::vector<int32_t> ix, iy;
-        if (p->undistort) {
-            ix.resize((size_t)fh * fw); iy.resize((size_t)fh * fw);
-            std::vector<int32_t> packed((size_t)fh * fw);
-            vti_plan_undistort_map(p->K, p->dist, fh, fw, ix.data(), iy.data());
-            for (int v = 0; v < fh; ++v)
-                for (int u = 0; u < fw; ++u) {
-                    const size_t i = (size_t)v * fw + u;
-                    const int dx = ix[i] - 32 * u, dy = iy[i] - 32 * v;
-                    if (dx < -32768 || dx > 32767 || dy < -32768 || dy > 32767) {
-                        vti_set_error("vti_create: lens displacement exceeds +-1024 px, unsupported");
-                        vti_destroy(h);
-                        return VTI_EINVAL;
-                    }
-                    packed[i] = (int32_t)(((uint32_t)(uint16_t)(int16_t)dy << 16) | (uint32_t)(uint16_t)(int16_t)dx);
-                }
-            if ((rc = upload(&h->d_und_lut, packed))) { vti_destroy(h); return rc; }
-        }
-        if ((rc = vti_k1_plan(h, xi, yi, xa, yb, p->undistort ? &ix : nullptr, p->undistort ? &iy : nullptr))) {
-            vti_destroy(h);
-            return rc;
-        }
-    }
-    // ---- measurement tables
-    if ((rc = build_axis_lut(fh, g.LH, &h->lutY, nullptr)) || (rc = build_axis_lut(fw, g.LW, &h->lutX, &h->d_xmap))) {
-        vti_destroy(h);
-        return rc;
-    }
-    // ---- post scratch
-    const size_t B = p->max_batch;
-    cudaError_t e = cudaSuccess;
-    auto alloc = [&](void** ptr, size_t bytes) { if (e == cudaSuccess) e = cudaMalloc(ptr, bytes); };
-    alloc((void**)&h->d_cand_count, sizeof(int32_t) * (B + 1));
-    alloc((void**)&h->d_cand_key, sizeof(unsigned long long) * B * vti_k3_cap_pad(g.max_candidates));
-    alloc((void**)&h->d_cand_box, sizeof(float4) * B * g.A);
-    alloc((void**)&h->d_det_coef, sizeof(float) * B * p->max_det * VTI_NM);
-    alloc((void**)&h->d_env, sizeof(int32_t) * B * g.LW);
-    alloc((void**)&h->d_env_frame, sizeof(int32_t) * B * fw);
-    alloc((void**)&h->d_flags, sizeof(int32_t) * B);
-    h->units_per_det = ((g.ph + 1 + VTI_K4_UR - 1) / VTI_K4_UR) * ((g.pw + 1 + VTI_K4_UC - 1) / VTI_K4_UC);
-    alloc((void**)&h->d_units, sizeof(uint4) * B * p->max_det * h->units_per_det);
-    alloc((void**)&h->d_proto_bbox, sizeof(int4) * B);
-    alloc((void**)&h->d_dense, sizeof(int32_t) * B);
-    if (e != cudaSuccess) {
-        vti_set_error(std::string("vti_create: cudaMalloc: ") + cudaGetErrorString(e));
-        vti_destroy(h);
-        return VTI_ENOMEM;
-    }
-    if ((rc = vti_k3_prepare(g.max_candidates)) || (rc = vti_k4_prepare()) || (rc = vti_k5_prepare(h->p.max_det))) { vti_destroy(h); return rc; }
+    const int rc = init_handle(h, p);
+    if (rc) { vti_destroy(h); return rc; }
     *out = h;
     return VTI_OK;
 }
@@ -336,8 +333,10 @@ static inline void mark(vti_handle* h, int i, cudaStream_t s) {
 
 extern "C" int vti_set_profiling(vti_handle* h, int on) {
     if (!h) return VTI_EINVAL;
-    if (on && !h->ev[0])
-        for (int i = 0; i < 8; ++i) VTI_CUDA(cudaEventCreate(&h->ev[i]));
+    if (on && !h->ev[0]) {
+        const int rc = create_events(h->ev, 8, cudaEventDefault);
+        if (rc) { destroy_events(h->ev, 8); return rc; }      // all or none: a retry starts clean
+    }
     h->profiling = on ? 1 : 0;
     for (int i = 0; i < 8; ++i) h->ev_set[i] = false;
     return VTI_OK;
@@ -364,6 +363,18 @@ static int check_batch(const vti_handle* h, int B) {
     return VTI_OK;
 }
 
+struct Aligned { const char* name; const void* ptr; unsigned bytes; };
+
+// VTI_EINVAL naming the first buffer not aligned to the width its kernels read it with (null passes)
+static int check_aligned(const char* fn, std::initializer_list<Aligned> bufs) {
+    for (const Aligned& b : bufs)
+        if (reinterpret_cast<uintptr_t>(b.ptr) % b.bytes) {
+            vti_set_error(std::string(fn) + ": " + b.name + " must be " + std::to_string(b.bytes) + "-byte aligned");
+            return VTI_EINVAL;
+        }
+    return VTI_OK;
+}
+
 extern "C" int vti_preprocess(vti_handle* h, const uint8_t* frames, int B, float* net_in, void* stream) {
     int rc = check_batch(h, B);
     if (rc) return rc;
@@ -374,36 +385,38 @@ extern "C" int vti_preprocess(vti_handle* h, const uint8_t* frames, int B, float
     return rc;
 }
 
+// K2 -> K3 -> K4 [-> K5], the one post chain of vti_postprocess (so of vti_post_measure) and of every chunk of
+// vti_process_host.  head: p3, p4, p5, coef, proto.  fetch_into: the prototypes are device-mapped host memory, fetched
+// after K3 (which sizes the rectangle K4 reads) into fetch_into.  results: K5 too.  timed: record the stage events.
+static int post_chain(vti_handle* h, const float* const head[5], float* fetch_into, int B, vti_det* dets, int32_t* counts,
+                      uint32_t* masks, vti_frame_result* results, bool timed, cudaStream_t s) {
+    auto stage = [&](int i) { if (timed) mark(h, i, s); };
+    // K3 and K4 evaluate the masks of every kept detection, not only of the routed stitch / fabric ones, when masks are
+    // exported, under VTI_ALL_DETS (the dense-overlap experiments of tools/k4_dense_bench.py) and for mask variant B: it
+    // removes every detection whose mask is empty (newer Ultralytics, construct_result), routed or not.
+    const int all_dets = masks != nullptr || h->p.mask_variant == 1 || h->all_dets_env;
+    int rc;
+    stage(2);
+    if ((rc = vti_launch_k2(h, head[0], head[1], head[2], B, s))) return rc;
+    stage(3);
+    if ((rc = vti_launch_k3(h, head[3], B, dets, counts, all_dets, s))) return rc;
+    stage(4);
+    if (fetch_into && (rc = vti_launch_fetch_proto(h, head[4], fetch_into, B, s))) return rc;
+    if ((rc = vti_launch_k4(h, fetch_into ? fetch_into : head[4], B, dets, counts, masks, all_dets, s))) return rc;
+    stage(5);
+    return results ? vti_launch_k5(h, B, dets, counts, results, s) : VTI_OK;
+}
+
 extern "C" int vti_postprocess(vti_handle* h, const float* p3, const float* p4, const float* p5, const float* coef,
                                const float* proto, int B, vti_det* dets, int32_t* counts, uint32_t* masks,
                                void* stream) {
     int rc = check_batch(h, B);
     if (rc) return rc;
-    if (!p3 || !p4 || !p5 || !coef || !proto || !dets || !counts) {
-        vti_set_error("vti_postprocess: null buffer");
-        return VTI_EINVAL;
-    }
-    if ((reinterpret_cast<uintptr_t>(dets) & 7) || (reinterpret_cast<uintptr_t>(counts) & 3) ||
-        ((reinterpret_cast<uintptr_t>(p3) | reinterpret_cast<uintptr_t>(p4) | reinterpret_cast<uintptr_t>(p5) |
-          reinterpret_cast<uintptr_t>(coef) | reinterpret_cast<uintptr_t>(proto)) & 3) ||
-        (masks && (reinterpret_cast<uintptr_t>(masks) & 15))) {
-        vti_set_error("vti_postprocess: misaligned buffer (dets 8, counts/head tensors 4, masks 16 bytes)");
-        return VTI_EINVAL;
-    }
-    cudaStream_t s = (cudaStream_t)stream;
-    mark(h, 2, s);
-    if ((rc = vti_launch_k2(h, p3, p4, p5, B, s))) return rc;
-    mark(h, 3, s);
-    // (VTI_ALL_DETS: mask statistics for EVERY kept detection, not only routed stitch / fabric ones -- the dense-overlap
-    //  experiments of tools/k4_dense_bench.py use many classes so that class-offset NMS keeps overlapping boxes)
-    // Mask variant B removes every detection whose mask is empty (newer Ultralytics, construct_result), routed or not: the
-    // masks of ALL kept detections are then evaluated so that the drop flags and n_det are the reference's.
-    if ((rc = vti_launch_k3(h, coef, B, dets, counts, masks != nullptr || h->p.mask_variant == 1 || getenv("VTI_ALL_DETS") != nullptr, s)))
-        return rc;
-    mark(h, 4, s);
-    rc = vti_launch_k4(h, proto, B, dets, counts, masks, s);
-    mark(h, 5, s);
-    return rc;
+    if (!p3 || !p4 || !p5 || !coef || !proto || !dets || !counts) { vti_set_error("vti_postprocess: null buffer"); return VTI_EINVAL; }
+    if ((rc = check_aligned("vti_postprocess", {{"dets", dets, 8}, {"counts", counts, 4}, {"p3", p3, 4}, {"p4", p4, 4}, {"p5", p5, 4},
+                                                {"coef", coef, 4}, {"proto", proto, 4}, {"masks", masks, 16}}))) return rc;
+    const float* head[5] = {p3, p4, p5, coef, proto};
+    return post_chain(h, head, nullptr, B, dets, counts, masks, nullptr, true, (cudaStream_t)stream);
 }
 
 extern "C" int vti_measure(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* results,
@@ -411,11 +424,7 @@ extern "C" int vti_measure(vti_handle* h, int B, vti_det* dets, const int32_t* c
     int rc = check_batch(h, B);
     if (rc) return rc;
     if (!dets || !counts || !results) { vti_set_error("vti_measure: null buffer"); return VTI_EINVAL; }
-    if ((reinterpret_cast<uintptr_t>(dets) & 7) || (reinterpret_cast<uintptr_t>(results) & 7) ||
-        (reinterpret_cast<uintptr_t>(counts) & 3)) {
-        vti_set_error("vti_measure: misaligned buffer (dets/results 8, counts 4 bytes)");
-        return VTI_EINVAL;
-    }
+    if ((rc = check_aligned("vti_measure", {{"dets", dets, 8}, {"results", results, 8}, {"counts", counts, 4}}))) return rc;
     mark(h, 6, (cudaStream_t)stream);
     rc = vti_launch_k5(h, B, dets, counts, results, (cudaStream_t)stream);
     mark(h, 7, (cudaStream_t)stream);
@@ -430,24 +439,21 @@ extern "C" int vti_post_measure(vti_handle* h, const float* p3, const float* p4,
     return vti_measure(h, B, dets, counts, results, stream);
 }
 
-static int ensure_staging(vti_handle* h) {
-    if (h->staged_batch) return VTI_OK;
-    const vti_geometry& g = h->g;
+// The host-buffer path's streams, events and buffers, made by its first call
+static int create_staging(vti_handle* h) {
     const size_t B = h->p.max_batch;
     VTI_CUDA(cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking));
     VTI_CUDA(cudaStreamCreateWithFlags(&h->copy_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 4; ++i) VTI_CUDA(cudaEventCreateWithFlags(&h->chunk_ev[i], cudaEventDisableTiming));
-    VTI_CUDA(cudaMalloc((void**)&h->d_frames, B * h->p.frame_h * h->p.frame_w * 3));
-    VTI_CUDA(cudaMalloc((void**)&h->d_net_in, sizeof(float) * B * 3 * g.LH * g.LW));
-    for (int l = 0; l < 3; ++l)
-        VTI_CUDA(cudaMalloc((void**)&h->d_p[l], sizeof(float) * B * (64 + h->p.nc) * g.lvl_h[l] * g.lvl_w[l]));
-    VTI_CUDA(cudaMalloc((void**)&h->d_coef, sizeof(float) * B * VTI_NM * g.A));
-    VTI_CUDA(cudaMalloc((void**)&h->d_proto, sizeof(float) * B * VTI_NM * g.ph * g.pw));
-    VTI_CUDA(cudaMalloc((void**)&h->d_dets, sizeof(vti_det) * B * h->p.max_det));
-    VTI_CUDA(cudaMalloc((void**)&h->d_counts, sizeof(int32_t) * B));
-    VTI_CUDA(cudaMalloc((void**)&h->d_results, sizeof(vti_frame_result) * B));
-    h->staged_batch = B;
-    return VTI_OK;
+    int rc = create_events(h->chunk_ev, 4, cudaEventDisableTiming);
+    auto alloc = [&](auto** ptr, size_t bytes) { if (!rc) rc = vti_alloc(h, ptr, bytes); };
+    alloc(&h->d_frames, B * h->p.frame_h * h->p.frame_w * 3);
+    alloc(&h->d_net_in, sizeof(float) * B * 3 * h->g.LH * h->g.LW);
+    for (int t = 0; t < 5; ++t) alloc(&h->d_head[t], sizeof(float) * B * h->head_floats[t]);
+    alloc(&h->d_dets, sizeof(vti_det) * B * h->p.max_det);
+    alloc(&h->d_counts, sizeof(int32_t) * B);
+    alloc(&h->d_results, sizeof(vti_frame_result) * B);
+    if (!rc) h->staged_batch = B;
+    return rc;
 }
 
 extern "C" int vti_ingest_yuyv(vti_handle* h, const uint8_t* yuyv, int B, uint8_t* frames, void* stream) {
@@ -455,8 +461,17 @@ extern "C" int vti_ingest_yuyv(vti_handle* h, const uint8_t* yuyv, int B, uint8_
     if (rc) return rc;
     if (!yuyv || !frames) { vti_set_error("vti_ingest_yuyv: null buffer"); return VTI_EINVAL; }
     if (h->p.frame_w & 1) { vti_set_error("vti_ingest_yuyv: packed 4:2:2 needs an even frame width"); return VTI_EINVAL; }
-    if ((reinterpret_cast<uintptr_t>(yuyv) & 3)) { vti_set_error("vti_ingest_yuyv: the YUYV buffer must be 4-byte aligned"); return VTI_EINVAL; }
+    if ((rc = check_aligned("vti_ingest_yuyv", {{"the YUYV buffer", yuyv, 4}}))) return rc;
     return vti_launch_k0_yuyv(h, yuyv, B, frames, (cudaStream_t)stream);
+}
+
+// The device alias of a pinned, device-mapped host buffer, or null: pageable memory, or VTI_NO_ZERO_COPY set (read on
+// every call, so that one handle can time both paths).
+static const float* mapped_alias(const float* host) {
+    cudaPointerAttributes at;
+    if (getenv("VTI_NO_ZERO_COPY")) return nullptr;
+    if (cudaPointerGetAttributes(&at, host) != cudaSuccess) { cudaGetLastError(); return nullptr; }   // old drivers: pageable
+    return at.type == cudaMemoryTypeHost ? static_cast<const float*>(at.devicePointer) : nullptr;
 }
 
 // fmt 0: BGR frames (3 bytes per pixel); 1: camera-native YUYV (2 bytes per pixel, converted by K0 on the device)
@@ -470,73 +485,46 @@ static int process_host_impl(vti_handle* h, const uint8_t* frames, int fmt, cons
         return VTI_EINVAL;
     }
     if (fmt == 1 && (h->p.frame_w & 1)) { vti_set_error("vti_process_host_yuyv: packed 4:2:2 needs an even frame width"); return VTI_EINVAL; }
-    if ((rc = ensure_staging(h))) return rc;
-    if (fmt == 1 && !h->d_yuyv) VTI_CUDA(cudaMalloc((void**)&h->d_yuyv, (size_t)h->p.max_batch * h->p.frame_h * h->p.frame_w * 2));
-    const vti_geometry& g = h->g;
+    const size_t keep = h->allocs.size();                  // all or nothing: a call after a failure starts clean
+    if (!h->staged_batch && (rc = create_staging(h))) { release_from(h, keep); return rc; }
+    if (fmt == 1 && !h->d_yuyv && (rc = vti_alloc(h, &h->d_yuyv, (size_t)h->p.max_batch * h->p.frame_h * h->p.frame_w * 2)))
+        return rc;
     cudaStream_t s = h->own_stream, cs = h->copy_stream;
-    const float* hp[3] = {p3, p4, p5};
     // The batch goes through in up to 4 chunks: chunk i+1's host->device copies (copy stream) run under chunk i's
     // kernels and device->host record copies (compute stream), so the call costs the PCIe time of its inputs plus
     // one chunk of compute.
     const int nchunk = B < 4 ? 1 : 4;
-    const size_t fsz = (size_t)h->p.frame_h * h->p.frame_w * 3, nsz = (size_t)3 * g.LH * g.LW;
+    const size_t fsz = (size_t)h->p.frame_h * h->p.frame_w * 3, nsz = (size_t)3 * h->g.LH * h->g.LW;
     const size_t ysz = (size_t)h->p.frame_h * h->p.frame_w * 2;
-    size_t lsz[3];
-    for (int l = 0; l < 3; ++l) lsz[l] = (size_t)(64 + h->p.nc) * g.lvl_h[l] * g.lvl_w[l];
-    const size_t csz = (size_t)VTI_NM * g.A, psz = (size_t)VTI_NM * g.ph * g.pw;
+    const size_t* hsz = h->head_floats;
     // Head tensors that sit in PINNED (device-mapped) host memory are not copied: K2 reads only the class planes and the
     // 64 box logits of each candidate, K3 only the coefficient rows of the kept detections -- a few hundred KB of the
     // 4.2 MB per frame -- so those kernels read them in place over PCIe (zero copy) and the DMA engine moves only the
-    // frames and the prototypes.  Pageable buffers are copied as before.
-    const float* dev_p[3];
-    bool zc_p[3];
-    for (int l = 0; l < 3; ++l) {
-        cudaPointerAttributes at;
-        zc_p[l] = !getenv("VTI_NO_ZERO_COPY") && cudaPointerGetAttributes(&at, hp[l]) == cudaSuccess &&
-                  at.type == cudaMemoryTypeHost && at.devicePointer != nullptr;
-        dev_p[l] = zc_p[l] ? static_cast<const float*>(at.devicePointer) : h->d_p[l];
-    }
-    const float* dev_coef = h->d_coef;
-    bool zc_coef = false;
-    {
-        cudaPointerAttributes at;
-        zc_coef = !getenv("VTI_NO_ZERO_COPY") && cudaPointerGetAttributes(&at, coef) == cudaSuccess &&
-                  at.type == cudaMemoryTypeHost && at.devicePointer != nullptr;
-        if (zc_coef) dev_coef = static_cast<const float*>(at.devicePointer);
-    }
-    // Pinned prototypes are not DMA-copied either: after K3 a fetch kernel reads, per frame, only the union rectangle of
-    // the crop windows (all that K4 ever touches) over PCIe into the device buffer.
-    const float* map_proto = nullptr;
-    {
-        cudaPointerAttributes at;
-        if (!getenv("VTI_NO_ZERO_COPY") && cudaPointerGetAttributes(&at, proto) == cudaSuccess &&
-            at.type == cudaMemoryTypeHost && at.devicePointer != nullptr)
-            map_proto = static_cast<const float*>(at.devicePointer);
-    }
-    cudaGetLastError();                                    // (a pageable pointer makes the query return an error on old drivers)
+    // frames and the prototypes.  Pinned prototypes are not DMA-copied either: the post chain fetches, per frame, only
+    // the union rectangle of the crop windows (all that K4 ever touches).  Pageable buffers are copied whole.
+    const float* host[5] = {p3, p4, p5, coef, proto};
+    const float* mapped[5];
+    for (int t = 0; t < 5; ++t) mapped[t] = mapped_alias(host[t]);
     for (int c = 0; c < nchunk; ++c) {
         const int b0 = (int)((long long)B * c / nchunk), b1 = (int)((long long)B * (c + 1) / nchunk), nb = b1 - b0;
         if (nb <= 0) continue;
         if (fmt == 1) VTI_CUDA(cudaMemcpyAsync(h->d_yuyv + b0 * ysz, frames + b0 * ysz, nb * ysz, cudaMemcpyHostToDevice, cs));
         else VTI_CUDA(cudaMemcpyAsync(h->d_frames + b0 * fsz, frames + b0 * fsz, nb * fsz, cudaMemcpyHostToDevice, cs));
-        for (int l = 0; l < 3; ++l)
-            if (!zc_p[l])
-                VTI_CUDA(cudaMemcpyAsync(h->d_p[l] + b0 * lsz[l], hp[l] + b0 * lsz[l], sizeof(float) * nb * lsz[l],
+        const float* head[5];
+        for (int t = 0; t < 5; ++t) {
+            head[t] = (mapped[t] ? mapped[t] : h->d_head[t]) + b0 * hsz[t];
+            if (!mapped[t])
+                VTI_CUDA(cudaMemcpyAsync(h->d_head[t] + b0 * hsz[t], host[t] + b0 * hsz[t], sizeof(float) * nb * hsz[t],
                                          cudaMemcpyHostToDevice, cs));
-        if (!zc_coef)
-            VTI_CUDA(cudaMemcpyAsync(h->d_coef + b0 * csz, coef + b0 * csz, sizeof(float) * nb * csz, cudaMemcpyHostToDevice, cs));
-        if (!map_proto)
-            VTI_CUDA(cudaMemcpyAsync(h->d_proto + b0 * psz, proto + b0 * psz, sizeof(float) * nb * psz, cudaMemcpyHostToDevice, cs));
+        }
         VTI_CUDA(cudaEventRecord(h->chunk_ev[c], cs));
         VTI_CUDA(cudaStreamWaitEvent(s, h->chunk_ev[c], 0));
         vti_det* cd = h->d_dets + (size_t)b0 * h->p.max_det;
         if (fmt == 1 && (rc = vti_launch_k0_yuyv(h, h->d_yuyv + b0 * ysz, nb, h->d_frames + b0 * fsz, s))) return rc;
         if ((rc = vti_launch_k1(h, h->d_frames + b0 * fsz, nb, h->d_net_in + b0 * nsz, s))) return rc;
-        if ((rc = vti_launch_k2(h, dev_p[0] + b0 * lsz[0], dev_p[1] + b0 * lsz[1], dev_p[2] + b0 * lsz[2], nb, s))) return rc;
-        if ((rc = vti_launch_k3(h, dev_coef + b0 * csz, nb, cd, h->d_counts + b0, h->p.mask_variant == 1, s))) return rc;
-        if (map_proto && (rc = vti_launch_fetch_proto(h, map_proto + b0 * psz, h->d_proto + b0 * psz, nb, s))) return rc;
-        if ((rc = vti_launch_k4(h, h->d_proto + b0 * psz, nb, cd, h->d_counts + b0, nullptr, s))) return rc;
-        if ((rc = vti_launch_k5(h, nb, cd, h->d_counts + b0, h->d_results + b0, s))) return rc;
+        if ((rc = post_chain(h, head, mapped[4] ? h->d_head[4] + b0 * hsz[4] : nullptr, nb, cd, h->d_counts + b0, nullptr,
+                             h->d_results + b0, false, s)))
+            return rc;
         if (net_in)
             VTI_CUDA(cudaMemcpyAsync(net_in + b0 * nsz, h->d_net_in + b0 * nsz, sizeof(float) * nb * nsz, cudaMemcpyDeviceToHost, s));
         VTI_CUDA(cudaMemcpyAsync(dets + (size_t)b0 * h->p.max_det, cd, sizeof(vti_det) * nb * h->p.max_det, cudaMemcpyDeviceToHost, s));

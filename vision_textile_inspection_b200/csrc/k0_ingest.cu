@@ -69,13 +69,10 @@ __global__ void __launch_bounds__(K0_THREADS) k0_yuyv2_kernel(const unsigned* __
 
 int vti_launch_k0_yuyv(vti_handle* h, const uint8_t* yuyv, int B, uint8_t* frames, cudaStream_t s) {
     const size_t npx = (size_t)B * h->p.frame_h * h->p.frame_w;
-    int sms = 148;
-    int dev = 0;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const bool quad = (npx % 4 == 0) && ((reinterpret_cast<uintptr_t>(yuyv) & 7) == 0) && ((reinterpret_cast<uintptr_t>(frames) & 3) == 0);
     const size_t items = quad ? npx / 4 : npx / 2;
     const size_t want = (items + K0_THREADS - 1) / K0_THREADS;
-    const int grid = (int)std::min<size_t>(want, (size_t)sms * 8 * 4);      // 8 resident CTAs per SM, 4 waves at most: grid-stride beyond
+    const int grid = (int)std::min<size_t>(want, (size_t)h->num_sms * 8 * 4);      // 8 resident CTAs per SM, 4 waves at most: grid-stride beyond
     if (grid <= 0) return VTI_OK;
     if (quad) k0_yuyv4_kernel<<<grid, K0_THREADS, 0, s>>>(reinterpret_cast<const uint2*>(yuyv), reinterpret_cast<unsigned*>(frames), items);
     else k0_yuyv2_kernel<<<grid, K0_THREADS, 0, s>>>(reinterpret_cast<const unsigned*>(yuyv), frames, items);

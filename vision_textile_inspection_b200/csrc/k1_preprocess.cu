@@ -753,12 +753,8 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
                 h->k1_mode = und_ix ? MODE_FAST_REMAP : MODE_FAST_PLAIN;
                 h->k1_pitch_u = pitch_u; h->k1_rows_u = rows_u; h->k1_smem = smem;
                 h->k1_und_words = und_words; h->k1_lut_stride = lut_stride; h->k1_raw_pitch = raw_pitch;
-                VTI_CUDA(cudaMalloc((void**)&h->d_k1_tiles, sizeof(int4) * hdr.size()));
-                VTI_CUDA(cudaMemcpy(h->d_k1_tiles, hdr.data(), sizeof(int4) * hdr.size(), cudaMemcpyHostToDevice));
-                if (und_ix) {
-                    VTI_CUDA(cudaMalloc((void**)&h->d_k1_lut, sizeof(unsigned) * lut.size()));
-                    VTI_CUDA(cudaMemcpy(h->d_k1_lut, lut.data(), sizeof(unsigned) * lut.size(), cudaMemcpyHostToDevice));
-                }
+                int rc;
+                if ((rc = vti_upload(h, &h->d_k1_tiles, hdr)) || (und_ix && (rc = vti_upload(h, &h->d_k1_lut, lut)))) return rc;
                 return k1_fast_dispatch(h, nullptr, 0, nullptr, smem);          // raises the shared-memory limits only
             }
         }
@@ -820,8 +816,7 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
         if (all_contig && (fw & 3) == 0 && tot <= 160 * 1024) {
             h->k1_mode = MODE_RAW;
             h->k1_smem = tot;
-            VTI_CUDA(cudaMalloc((void**)&h->d_k1_tiles, sizeof(int4) * boxes.size()));
-            VTI_CUDA(cudaMemcpy(h->d_k1_tiles, boxes.data(), sizeof(int4) * boxes.size(), cudaMemcpyHostToDevice));
+            if (const int rc = vti_upload(h, &h->d_k1_tiles, boxes)) return rc;
         } else {
             h->k1_mode = MODE_GATHER;
         }

@@ -17,8 +17,6 @@
 //                     kernel, the block that owned a row of stitches decoded ~400 candidates alone.)
 #include "vti_internal.h"
 
-int vti_k3_cap_pad(int cap);
-
 namespace {
 
 constexpr int K2_THREADS = 256;

@@ -494,15 +494,7 @@ int vti_launch_k3(vti_handle* h, const float* coef, int B, vti_det* dets, int32_
     a.padx = (float)nearbyint((LW - fw * gain) / 2 - 0.1);
     a.pady = (float)nearbyint((LH - fh * gain) / 2 - 0.1);
     a.fw = (float)fw; a.fh = (float)fh;
-    a.roi_active = 0; a.rx1 = a.ry1 = a.rx2 = a.ry2 = 0;
-    if (h->p.variant == 0 && h->p.roi_enabled) {        // measurement.py:220-238
-        auto clampi = [](int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); };
-        const int x_min = clampi(h->p.roi_x_min, 0, fw - 1), x_max = clampi(h->p.roi_x_max, 0, fw - 1);
-        const int y_min = clampi(h->p.roi_y_min, 0, fh - 1), y_max = clampi(h->p.roi_y_max, 0, fh - 1);
-        if (x_min < x_max && y_min < y_max) {
-            a.roi_active = 1; a.rx1 = x_min; a.ry1 = y_min; a.rx2 = x_max; a.ry2 = y_max;
-        }
-    }
+    a.roi_active = h->roi.active; a.rx1 = h->roi.x1; a.ry1 = h->roi.y1; a.rx2 = h->roi.x2; a.ry2 = h->roi.y2;
     a.stitch_id = h->p.stitch_id; a.fabric_id = h->p.fabric_id;
     {
         const float c = h->p.conf > 0.0f ? h->p.conf : 0.0f, one = 1.0f;

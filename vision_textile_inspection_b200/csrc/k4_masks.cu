@@ -509,7 +509,7 @@ int vti_k4_prepare() {
 }
 
 int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const int32_t* counts, uint32_t* masks,
-                  cudaStream_t s) {
+                  int all_dets, cudaStream_t s) {
     K4Args a;
     a.proto = proto;
     a.dets = dets;
@@ -542,7 +542,6 @@ int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const
     if (h->p.k4_dense) {
         // tcgen05 tile form for the frames K3 flagged: one CTA per (tile, frame); CTAs of other frames / empty tiles exit
         const dim3 dgrid(((a.pw + 1 + DT_C - 1) / DT_C) * ((a.ph + 1 + DT_R - 1) / DT_R), B);
-        const int all_dets = masks != nullptr || h->p.mask_variant == 1 || getenv("VTI_ALL_DETS") != nullptr;
         if (masks && vb) k4_dense_kernel<true, true><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);
         else if (masks) k4_dense_kernel<true, false><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);
         else if (vb) k4_dense_kernel<false, true><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);

@@ -215,13 +215,7 @@ extern "C" int vti_annotate(vti_handle* h, const uint8_t* frames, int B, const v
     K6Args a;
     a.img = annotated; a.dets = dets; a.counts = counts; a.env_frame = h->d_env_frame;
     a.h = fh; a.w = fw; a.max_det = h->p.max_det;
-    a.roi_active = 0; a.rx1 = a.ry1 = a.rx2 = a.ry2 = 0;
-    if (h->p.variant == 0 && h->p.roi_enabled) {                 // measurement.py:220-238
-        auto clampi = [](int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); };
-        const int x_min = clampi(h->p.roi_x_min, 0, fw - 1), x_max = clampi(h->p.roi_x_max, 0, fw - 1);
-        const int y_min = clampi(h->p.roi_y_min, 0, fh - 1), y_max = clampi(h->p.roi_y_max, 0, fh - 1);
-        if (x_min < x_max && y_min < y_max) { a.roi_active = 1; a.rx1 = x_min; a.ry1 = y_min; a.rx2 = x_max; a.ry2 = y_max; }
-    }
+    a.roi_active = h->roi.active; a.rx1 = h->roi.x1; a.ry1 = h->roi.y1; a.rx2 = h->roi.x2; a.ry2 = h->roi.y2;
     const dim3 gdet(a.max_det, B);
     k6_boxes_kernel<<<dim3(1, B), 128, 0, s>>>(a, 0);            // ROI
     k6_boxes_kernel<<<gdet, 128, 0, s>>>(a, 1);                  // fabric boxes

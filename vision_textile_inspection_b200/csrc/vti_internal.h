@@ -30,12 +30,19 @@ struct AxisLut {
     int32_t* next_first;  // min first[] over entries >= i (INT_MAX if none)
 };
 
+// The ROI rectangle of measurement.py:220-238 clamped to the frame; active only for variant 0 with a non-empty clamp.
+struct VtiRoi { int active, x1, y1, x2, y2; };
+
+// Value-initialised (`new vti_handle()`): every pointer and count starts at zero.
 struct vti_handle {
     vti_params p;
     vti_geometry g;
     int device;
     int num_sms;
     int64_t launches;
+    bool all_dets_env;                             // VTI_ALL_DETS, read at create
+    VtiRoi roi;
+    std::vector<void*> allocs;                     // every device allocation of the handle (vti_alloc)
 
     // ---- K1 tables (device)
     int32_t* d_tap_x_idx;  int16_t* d_tap_x_a;    // [new_w], [new_w*2]
@@ -68,7 +75,8 @@ struct vti_handle {
     cudaStream_t own_stream, copy_stream;
     cudaEvent_t chunk_ev[4];
     uint8_t* d_yuyv;                               // camera-native staging (vti_process_host_yuyv), allocated on first use
-    uint8_t* d_frames; float* d_net_in; float* d_p[3]; float* d_coef; float* d_proto;
+    uint8_t* d_frames; float* d_net_in; float* d_head[5];     // head: p3, p4, p5, coef, proto
+    size_t head_floats[5];                         // floats per frame of each head tensor
     vti_det* d_dets; int32_t* d_counts; vti_frame_result* d_results;
     size_t staged_batch;
     // ---- optional per-kernel event timing
@@ -87,8 +95,33 @@ void vti_set_error(const std::string& s);
         }                                                                                          \
     } while (0)
 
+// Every device allocation of a handle goes through here: the handle records it, and vti_destroy frees the record.
+template <typename T>
+int vti_alloc(vti_handle* h, T** dptr, size_t bytes) {
+    void* p = nullptr;
+    if (const cudaError_t e = cudaMalloc(&p, bytes)) {
+        cudaGetLastError();                        // not sticky: clear it, or the next launch check would report it
+        vti_set_error(std::string("cudaMalloc: ") + cudaGetErrorString(e));
+        return VTI_ENOMEM;
+    }
+    h->allocs.push_back(p);
+    *dptr = static_cast<T*>(p);
+    return VTI_OK;
+}
+template <typename T>
+int vti_upload(vti_handle* h, T** dptr, const std::vector<T>& v) {
+    if (const int rc = vti_alloc(h, dptr, sizeof(T) * (v.empty() ? 1 : v.size()))) return rc;
+    if (!v.empty()) VTI_CUDA(cudaMemcpy(*dptr, v.data(), sizeof(T) * v.size(), cudaMemcpyHostToDevice));
+    return VTI_OK;
+}
+
 // raises (never lowers) a kernel function's dynamic shared-memory limit on the current device
 int vti_raise_dyn_smem(const void* func, size_t bytes);
+// create-time preparation of the post kernels (dynamic shared-memory limits) and K3's padded candidate list length
+int vti_k3_prepare(int cap);
+int vti_k3_cap_pad(int cap);
+int vti_k4_prepare();
+int vti_k5_prepare(int max_det);
 // kernel launchers (each returns VTI_OK / VTI_ECUDA)
 int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector<int32_t>& yi,
                 const std::vector<int16_t>& xa, const std::vector<int16_t>& yb,
@@ -98,7 +131,7 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cu
 int vti_launch_k2(vti_handle* h, const float* p3, const float* p4, const float* p5, int B, cudaStream_t s);
 int vti_launch_k3(vti_handle* h, const float* coef, int B, vti_det* dets, int32_t* counts, int all_dets, cudaStream_t s);
 int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const int32_t* counts, uint32_t* masks,
-                  cudaStream_t s);
+                  int all_dets, cudaStream_t s);
 int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* res, cudaStream_t s);
 // copies, per frame, the prototype rectangle K4 will read (all 32 channels) from device-mapped host memory
 int vti_launch_fetch_proto(vti_handle* h, const float* host_proto_mapped, float* dev_proto, int B, cudaStream_t s);
