@@ -40,7 +40,6 @@ extern "C" {
 
 #define VTI_NM 32          /* mask coefficients / prototype channels */
 #define VTI_REG_MAX 16     /* DFL bins */
-#define VTI_K4_DENSE_COVER 24  /* k4_dense = 1: frames whose summed crop-window cells exceed this many plane covers */
 
 /* det.flags */
 #define VTI_F_IN_ROI 1u      /* passed measurement.py:253-260 (always set when ROI is off) */
@@ -91,10 +90,6 @@ typedef struct vti_params {
     int32_t mask_variant;         /* SURVEY 8a U6.  0 = "A" (Ultralytics <= 8.0.x, the north-star wording):
                                      sigmoid -> crop -> bilinear x4 -> > 0.5.  1 = "B" (newer releases): no sigmoid,
                                      crop, bilinear x4, > 0.0, and detections whose mask is empty are dropped */
-    int32_t k4_dense;             /* tensor-core (tcgen05) tile form of the mask contraction: 0 = never (default: the
-                                     crop makes the contraction < 1 % dense on every configured workload), 1 = per
-                                     frame, when the crop windows cover the prototype plane more than
-                                     VTI_K4_DENSE_COVER times over (measured crossover, DESIGN.md 4), 2 = always */
 } vti_params;
 
 typedef struct vti_geometry {

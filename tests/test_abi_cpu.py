@@ -27,8 +27,9 @@ def test_exports_match_header():
 
 
 def test_struct_sizes_match_header():
-    # 22 int32 + conf, iou + K, dist, R, t, iou_threshold doubles + mask_variant, k4_dense (round 2)
-    assert C.sizeof(_lib.VtiParams) == 22 * 4 + 2 * 4 + (9 + 5 + 9 + 3 + 1) * 8 + 2 * 4
+    # 22 int32 + conf, iou + K, dist, R, t, iou_threshold doubles + mask_variant; the last 4 bytes are padding (the
+    # struct is 8-byte aligned), so callers built when a second int32 followed mask_variant pass the same struct_size
+    assert C.sizeof(_lib.VtiParams) == 22 * 4 + 2 * 4 + (9 + 5 + 9 + 3 + 1) * 8 + 4 + 4
     assert _lib.DET_DTYPE.itemsize == 160
 
 

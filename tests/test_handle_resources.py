@@ -19,18 +19,17 @@ def make_engine(cfg, max_batch, device=None, **over):
 
 
 @pytest.mark.parametrize("pinned", [False, True])
-@pytest.mark.parametrize("k4_dense", [0, 2])
-def test_all_dets_env_host_path_matches_device_path(monkeypatch, k4_dense, pinned):
-    """With VTI_ALL_DETS=1, vti_process_host evaluates the masks of the detections outside the ROI exactly as
-    vti_post_measure does, unit form or tile form, with the head tensors copied or read in place (pinned: zero copy
-    plus the prototype fetch, whose rectangle must cover those detections too)."""
-    monkeypatch.setenv("VTI_ALL_DETS", "1")
+def test_host_path_matches_device_path_when_every_mask_is_evaluated(pinned):
+    """Mask variant B evaluates every kept detection's mask, routed or not; the host path exports no masks, so this is
+    the setting in which it does.  vti_process_host then evaluates the masks of the detections outside the ROI exactly
+    as vti_post_measure does, with the head tensors copied or read in place (pinned: zero copy plus the prototype
+    fetch, whose rectangle must cover those detections too)."""
     cfg = synth.CONFIGS["cfg2"]
     B = 3
     batch = synth.make_batch(cfg, B, seed0=2000)
     # the synthetic stitch rows span the frame's width: an ROI ending at 3/4 of it leaves the right quarter's outside
     on, x_min, _, y_min, y_max = cfg.roi()
-    eng = make_engine(cfg, B, k4_dense=k4_dense, roi=(on, x_min, cfg.frame_w * 3 // 4, y_min, y_max))
+    eng = make_engine(cfg, B, mask_variant=1, roi=(on, x_min, cfg.frame_w * 3 // 4, y_min, y_max))
     heads = [*batch["levels"], batch["coef"], batch["proto"]]
     host = [batch["frames"]] + heads
     if pinned:

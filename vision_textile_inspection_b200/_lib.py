@@ -26,7 +26,7 @@ class VtiParams(C.Structure):
         ("max_px_distance", C.c_int32), ("neighborhood", C.c_int32), ("max_candidates", C.c_int32),
         ("conf", C.c_float), ("iou", C.c_float),
         ("K", C.c_double * 9), ("dist", C.c_double * 5), ("R", C.c_double * 9), ("t", C.c_double * 3),
-        ("iou_threshold", C.c_double), ("mask_variant", C.c_int32), ("k4_dense", C.c_int32),
+        ("iou_threshold", C.c_double), ("mask_variant", C.c_int32),
     ]
 
 

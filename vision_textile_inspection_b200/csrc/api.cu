@@ -215,7 +215,6 @@ static int init_handle(vti_handle* h, const vti_params* p) {
     }
     const vti_geometry& g = h->g;
     const int fh = p->frame_h, fw = p->frame_w;
-    h->all_dets_env = getenv("VTI_ALL_DETS") != nullptr;
     if (p->variant == 0 && p->roi_enabled) {                // measurement.py:220-238
         const int x_min = std::clamp(p->roi_x_min, 0, fw - 1), x_max = std::clamp(p->roi_x_max, 0, fw - 1);
         const int y_min = std::clamp(p->roi_y_min, 0, fh - 1), y_max = std::clamp(p->roi_y_max, 0, fh - 1);
@@ -284,9 +283,8 @@ static int init_handle(vti_handle* h, const vti_params* p) {
     h->units_per_det = ((g.ph + 1 + VTI_K4_UR - 1) / VTI_K4_UR) * ((g.pw + 1 + VTI_K4_UC - 1) / VTI_K4_UC);
     alloc(&h->d_units, sizeof(uint4) * B * p->max_det * h->units_per_det);
     alloc(&h->d_proto_bbox, sizeof(int4) * B);
-    alloc(&h->d_dense, sizeof(int32_t) * B);
     if (rc) return rc;
-    if ((rc = vti_k3_prepare(g.max_candidates)) || (rc = vti_k4_prepare()) || (rc = vti_k5_prepare(p->max_det))) return rc;
+    if ((rc = vti_k3_prepare(g.max_candidates)) || (rc = vti_k5_prepare(p->max_det))) return rc;
     return VTI_OK;
 }
 
@@ -300,7 +298,7 @@ extern "C" int vti_create(const vti_params* p, vti_handle** out) {
     // nc: K2 packs the class into the top byte of a candidate key; max_batch: K3 packs the frame index into 15 bits
     if (p->nc < 1 || p->nc > 255 || p->max_det < 1 || p->max_det > 1024 || p->max_batch < 1 || p->max_batch > 32767 ||
         p->neighborhood < 0 || p->neighborhood > 7 || (p->variant != 0 && p->variant != 1) ||
-        (p->mask_variant != 0 && p->mask_variant != 1) || p->k4_dense < 0 || p->k4_dense > 2) {
+        (p->mask_variant != 0 && p->mask_variant != 1)) {
         vti_set_error("vti_create: parameter out of range (nc 1..255, max_det 1..1024, max_batch 1..32767, "
                       "neighborhood 0..7, variant 0/1, mask_variant 0/1)");
         return VTI_EINVAL;
@@ -392,9 +390,9 @@ static int post_chain(vti_handle* h, const float* const head[5], float* fetch_in
                       uint32_t* masks, vti_frame_result* results, bool timed, cudaStream_t s) {
     auto stage = [&](int i) { if (timed) mark(h, i, s); };
     // K3 and K4 evaluate the masks of every kept detection, not only of the routed stitch / fabric ones, when masks are
-    // exported, under VTI_ALL_DETS (the dense-overlap experiments of tools/k4_dense_bench.py) and for mask variant B: it
-    // removes every detection whose mask is empty (newer Ultralytics, construct_result), routed or not.
-    const int all_dets = masks != nullptr || h->p.mask_variant == 1 || h->all_dets_env;
+    // exported and for mask variant B: it removes every detection whose mask is empty (newer Ultralytics,
+    // construct_result), routed or not.
+    const int all_dets = masks != nullptr || h->p.mask_variant == 1;
     int rc;
     stage(2);
     if ((rc = vti_launch_k2(h, head[0], head[1], head[2], B, s))) return rc;
@@ -402,7 +400,7 @@ static int post_chain(vti_handle* h, const float* const head[5], float* fetch_in
     if ((rc = vti_launch_k3(h, head[3], B, dets, counts, all_dets, s))) return rc;
     stage(4);
     if (fetch_into && (rc = vti_launch_fetch_proto(h, head[4], fetch_into, B, s))) return rc;
-    if ((rc = vti_launch_k4(h, fetch_into ? fetch_into : head[4], B, dets, counts, masks, all_dets, s))) return rc;
+    if ((rc = vti_launch_k4(h, fetch_into ? fetch_into : head[4], B, dets, counts, masks, s))) return rc;
     stage(5);
     return results ? vti_launch_k5(h, B, dets, counts, results, s) : VTI_OK;
 }

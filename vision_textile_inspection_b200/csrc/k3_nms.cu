@@ -55,8 +55,6 @@ struct K3Args {
     int ph, pw, all_dets, units_per_det;
     int32_t* unit_count;        // one counter for the whole batch
     uint4* units;
-    int32_t* dense_flag;        // [B] K4 form of the frame: 1 = tcgen05 tiles (no work units are emitted), 0 = units
-    int dense_mode;             // vti_params.k4_dense
     int4* proto_bbox;           // [B] union of the crop windows K4 will read (x_lo, y_lo, x_hi, y_hi), empty = (1, 1, 0, 0)
 };
 
@@ -401,16 +399,7 @@ __global__ void __launch_bounds__(K3_THREADS, 1) k3_nms_kernel(const K3Args a) {
         __syncthreads();
         const int excl = incl - nu + (warp ? s_wsum[warp - 1] : 0);
         if (tid <= nk) s_upre[tid] = excl;                 // s_upre[nk] = total (nu = 0 there)
-        int total = s_wsum[31];
-        {
-            // Frame-level choice of the K4 form: the units' cells, summed over the kept detections, against the cells of
-            // the prototype plane = how many times over the crop windows cover it
-            const long long cells = (long long)total * VTI_K4_UR * VTI_K4_UC;
-            const bool dense = a.dense_mode == 2 || (a.dense_mode == 1 && total > 0 &&
-                                                      cells >= (long long)VTI_K4_DENSE_COVER * (a.ph + 1) * (a.pw + 1));
-            if (tid == 0) a.dense_flag[b] = dense ? 1 : 0;
-            if (dense) total = 0;                              // the tile form lists its detections itself
-        }
+        const int total = s_wsum[31];
         if (tid == 0) { s_ubase = total ? atomicAdd(a.unit_count, total) : 0; s_bb[0] = INT_MAX; s_bb[1] = INT_MAX; s_bb[2] = -1; s_bb[3] = -1; }
         __syncthreads();
         if (tid < nk && nu > 0) {                          // union of the windows that have work units
@@ -509,7 +498,6 @@ int vti_launch_k3(vti_handle* h, const float* coef, int B, vti_det* dets, int32_
     a.unit_count = h->d_cand_count + h->p.max_batch;
     a.units = h->d_units;
     a.proto_bbox = h->d_proto_bbox;
-    a.dense_flag = h->d_dense; a.dense_mode = h->p.k4_dense;
     k3_nms_kernel<<<B, K3_THREADS, vti_k3_smem_bytes(h->g.max_candidates), s>>>(a);
     h->launches++;
     VTI_CUDA(cudaGetLastError());

@@ -41,7 +41,6 @@ constexpr int UR = VTI_K4_UR, UC = VTI_K4_UC;
 constexpr int SCW = UC + 1;                 // corner columns per unit
 constexpr float MARGIN = 1e-5f;             // >> fp32 rounding of the lerp; cells within the margin are evaluated per pixel
 constexpr float MARGIN_B = 1e-3f;           // variant B: logits (|values| up to ~30) instead of probabilities
-constexpr int MAX_DENSE_DETS = 1024;        // = the max_det ceiling of vti_create
 
 struct K4Args {
     const float* proto;         // [B][32][ph][pw]
@@ -251,233 +250,6 @@ __global__ void __launch_bounds__(K4_THREADS, 1024 / K4_THREADS) k4_units_kernel
 }
 
 
-// ====================================================================================================================
-// Dense tile form on the 5th-generation tensor cores (tcgen05.mma kind::tf32, accumulators in TMEM).
-//
-// The north star names the N x 32 @ 32 x (ph*pw) contraction as the one tensor-core candidate.  On the configured
-// workloads the box crop makes it 0.1-0.8 % dense and the unit form above wins by a wide margin (DESIGN.md 4); this form
-// is for scenes where MANY kept boxes overlap the same prototype pixels (dispatch: vti_params.k4_dense).  Work item =
-// (frame, tile of DT_R x DT_C interpolation cells = 7 x 17 = 119 corner prototype pixels, padded to M = 128):
-//   * the tile's detections (those whose crop window touches the tile's cells) are listed,
-//   * A = the tile's prototype values [128 px][32 ch], B = the listed detections' coefficients [N][32], both K-major
-//     and split into tf32 hi + lo parts in shared memory: L = A_hi B_hi + A_lo B_hi + A_hi B_lo, three
-//     accumulating passes of 4 k-steps each (fp32 accumulate in TMEM) -- a single tf32 pass flips mask pixels on ~2 % of
-//     the instances (SURVEY 7), the three-term split is at fp32 rounding level,
-//   * tcgen05.ld brings D[128 px][DN dets] back, thread t owning TMEM lane t = corner pixel t; sigmoid (or the raw logit,
-//     variant B) + box crop go to shared memory as one corner array per detection,
-//   * the cells of every detection are then classified and reduced by exactly the code of the unit form (unit_cells).
-// The prototype tile is read ONCE per tile instead of once per (detection, unit).
-// ====================================================================================================================
-constexpr int DT_R = 6, DT_C = UC;                  // cells per tile: 6 x 16  (corner rows x cols: 7 x 17 = 119 <= 128)
-constexpr int DT_CR = DT_R + 1, DT_CC = DT_C + 1;
-constexpr int DT_M = 128;                           // MMA M (TMEM lanes); rows >= 119 are zero padding
-constexpr int DN = 64;                              // detections per MMA pass = MMA N = TMEM columns
-constexpr int DENSE_THREADS = 256;
-constexpr int DA_BYTES = DT_M * VTI_NM * 4;         // 16 KB per A part
-constexpr int DB_BYTES = DN * VTI_NM * 4;           // 8 KB per B part
-constexpr size_t K4_DENSE_SMEM = 2 * DA_BYTES + 2 * DB_BYTES + (size_t)DN * DT_M * 4 + 1024;   // + s_c, + alignment slack
-static_assert(DT_CR * DT_CC <= DT_M, "tile corners must fit the MMA M");
-
-__device__ __forceinline__ unsigned k4_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ unsigned tf32_rna(float x) {
-    unsigned r;
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(r) : "f"(x));
-    return r;
-}
-// shared-memory matrix descriptor, no swizzle: start address, leading / stride byte offsets (all >> 4), version 1 (sm_100)
-__device__ __forceinline__ unsigned long long umma_desc(unsigned saddr, unsigned lbo_bytes, unsigned sbo_bytes) {
-    return (unsigned long long)((saddr >> 4) & 0x3FFFu) | ((unsigned long long)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((unsigned long long)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
-// Both operands K-major, no swizzle: element (row, k) at (row / 8) * 1024 + (k / 4) * 128 + (row % 8) * 16 + (k % 4) * 4
-// [core matrix = 8 rows x 4 k = 128 contiguous bytes; the two core matrices of a k-step lie LBO = 128 B apart, 8-row groups
-// SBO = 1024 B apart].  (tools/probe/tcgen05_probe.cu: with this layout kind::tf32 reproduces an integer test product
-// exactly; an MN-major A -- the prototype plane's native order -- returned zeros on this toolkit, hence the transposing
-// staging pass, which the hi / lo split needs anyway.)
-__device__ __forceinline__ int da_off(int m, int k) { return (m >> 3) * 1024 + (k >> 2) * 128 + (m & 7) * 16 + (k & 3) * 4; }
-__device__ __forceinline__ int db_off(int n, int k) { return (n >> 3) * 1024 + (k >> 2) * 128 + (n & 7) * 16 + (k & 3) * 4; }
-
-template <bool EXPORT, bool VB>
-__global__ void __launch_bounds__(DENSE_THREADS, 2) k4_dense_kernel(const K4Args a, const int32_t* __restrict__ counts,
-                                                                    const int32_t* __restrict__ dense_flag, int all_dets) {
-    extern __shared__ __align__(16) unsigned char s_raw8[];
-    __shared__ __align__(8) unsigned long long s_mbar;
-    __shared__ unsigned s_tmem;
-    __shared__ short s_list[MAX_DENSE_DETS];
-    __shared__ int s_nt;
-    __shared__ int s_envw[DENSE_THREADS / 32][4 * UC];
-
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int b = blockIdx.y;
-    if (dense_flag && !dense_flag[b]) return;
-    const int ntx = (a.pw + 1 + DT_C - 1) / DT_C;
-    const int Ty = blockIdx.x / ntx, Tx = blockIdx.x - Ty * ntx;
-    const int R0 = Ty * DT_R, C0 = Tx * DT_C;                              // first cell of the tile
-    const int R1 = min(R0 + DT_R - 1, a.ph), C1 = min(C0 + DT_C - 1, a.pw); // last cell (cells exist for 0..ph / 0..pw)
-    const int nr = R1 - R0 + 2, ncw = C1 - C0 + 2;                          // corner rows / cols actually used
-    const int n = min(counts[b], MAX_DENSE_DETS);
-    vti_det* __restrict__ dets = a.dets + (size_t)b * a.max_det;
-
-    // ---- the tile's detections
-    if (tid == 0) s_nt = 0;
-    __syncthreads();
-    for (int k = tid; k < n; k += DENSE_THREADS) {
-        const unsigned f = dets[k].flags;
-        const bool wanted = all_dets || ((f & VTI_F_IN_ROI) && (f & (VTI_F_STITCH | VTI_F_FABRIC)));
-        const VtiWindow w = vti_det_window(dets[k].box_lb, a.ph, a.pw);
-        // the detection's non-zero cells are rows [cy_lo, cy_hi + 1], cols [cx_lo, cx_hi + 1]
-        if (wanted && !w.empty && w.cy_lo <= R1 && w.cy_hi + 1 >= R0 && w.cx_lo <= C1 && w.cx_hi + 1 >= C0)
-            s_list[atomicAdd(&s_nt, 1)] = (short)k;
-    }
-    __syncthreads();
-    const int nt = s_nt;
-    if (nt == 0) return;
-
-    unsigned char* sA_hi = reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(s_raw8) + 1023) & ~uintptr_t(1023));
-    unsigned char* sA_lo = sA_hi + DA_BYTES;
-    unsigned char* sB_hi = sA_lo + DA_BYTES;
-    unsigned char* sB_lo = sB_hi + DB_BYTES;
-    float* s_c = reinterpret_cast<float*>(sB_lo + DB_BYTES);               // [DN][DT_M] corner values per detection
-
-    // ---- TMEM allocation (one warp), barrier init
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;"
-                     :: "r"(k4_smem_u32(&s_tmem)), "n"(DN) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    if (tid == 32) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(k4_smem_u32(&s_mbar)) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    // ---- A: the tile's prototype corner pixels (replicate-clamped like the unit form), tf32 hi + lo
-    const float* __restrict__ proto = a.proto + (size_t)b * VTI_NM * a.ph * a.pw;
-    const size_t plane = (size_t)a.ph * a.pw;
-    for (int i = tid; i < DT_M * VTI_NM; i += DENSE_THREADS) {
-        const int q = i / DT_M, m = i - q * DT_M;                          // consecutive threads: consecutive pixels
-        const int r = m / DT_CC, c = m - r * DT_CC;
-        float v = 0.0f;
-        if (r < nr && c < ncw) {
-            const int py = min(max(R0 - 1 + r, 0), a.ph - 1), px = min(max(C0 - 1 + c, 0), a.pw - 1);
-            v = __ldg(proto + q * plane + (size_t)py * a.pw + px);
-        }
-        const unsigned hi = tf32_rna(v);
-        const unsigned lo = tf32_rna(__fsub_rn(v, __uint_as_float(hi)));
-        *reinterpret_cast<unsigned*>(sA_hi + da_off(m, q)) = hi;
-        *reinterpret_cast<unsigned*>(sA_lo + da_off(m, q)) = lo;
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const unsigned tmem = s_tmem;
-    // instruction descriptor: D = F32, A = B = TF32, both K-major, N = DN, M = 128
-    constexpr unsigned IDESC = (1u << 4) | (2u << 7) | (2u << 10) | (0u << 15) | (0u << 16) | ((unsigned)(DN >> 3) << 17) |
-                               ((unsigned)(DT_M >> 4) << 24);
-    unsigned phase = 0u;
-    const int my_m = tid & 127;                                            // TMEM lane = corner pixel of this thread
-    const int mr = my_m / DT_CC, mc = my_m - mr * DT_CC;
-    const int mpy = R0 - 1 + mr, mpx = C0 - 1 + mc;                        // un-clamped prototype coordinates (crop test)
-
-    for (int d0 = 0; d0 < nt; d0 += DN) {
-        const int nd = min(DN, nt - d0);
-        // ---- B: coefficients of this pass's detections, tf32 hi + lo (rows >= nd zero)
-        for (int i = tid; i < DN * VTI_NM; i += DENSE_THREADS) {
-            const int j = i >> 5, q = i & 31;
-            float v = 0.0f;
-            if (j < nd) v = __ldg(a.det_coef + ((size_t)b * a.max_det + s_list[d0 + j]) * VTI_NM + q);
-            const unsigned hi = tf32_rna(v);
-            const unsigned lo = tf32_rna(__fsub_rn(v, __uint_as_float(hi)));
-            *reinterpret_cast<unsigned*>(sB_hi + db_off(j, q)) = hi;
-            *reinterpret_cast<unsigned*>(sB_lo + db_off(j, q)) = lo;
-        }
-        // generic-proxy writes -> visible to the tensor core's async-proxy reads
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        if (tid == 0) {
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const unsigned aH = k4_smem_u32(sA_hi), aL = k4_smem_u32(sA_lo), bH = k4_smem_u32(sB_hi), bL = k4_smem_u32(sB_lo);
-            bool acc = false;
-#pragma unroll
-            for (int term = 0; term < 3; ++term) {
-                const unsigned aa = term == 1 ? aL : aH, bb = term == 2 ? bL : bH;
-#pragma unroll
-                for (int ks = 0; ks < VTI_NM / 8; ++ks) {
-                    // a k-step = two 4-channel core matrices, 128 B apart (LBO); 8-row groups 1024 B apart (SBO)
-                    const unsigned long long da = umma_desc(aa + ks * 256, 128, 1024);
-                    const unsigned long long db = umma_desc(bb + ks * 256, 128, 1024);
-                    const unsigned en = acc ? 1u : 0u;
-                    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-                                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-                                 :: "r"(tmem), "l"(da), "l"(db), "r"(IDESC), "r"(en) : "memory");
-                    acc = true;
-                }
-            }
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
-                         :: "r"(k4_smem_u32(&s_mbar)) : "memory");
-        }
-        // ---- wait for the accumulator
-        {
-            const unsigned bar = k4_smem_u32(&s_mbar);
-            asm volatile(
-                "{\n\t.reg .pred p;\n\t"
-                "W_%=:\n\t"
-                "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-                "@p bra D_%=;\n\t"
-                "bra W_%=;\n\t"
-                "D_%=:\n\t}"
-                :: "r"(bar), "r"(phase) : "memory");
-            phase ^= 1u;
-        }
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        // ---- epilogue 1: D[lane = pixel][column = detection] -> sigmoid + crop -> s_c[det][pixel]
-        {
-            const int col0 = (warp >> 2) * (DN / 2);                       // warps 0-3: columns 0..31, warps 4-7: 32..63
-            const unsigned taddr = tmem + ((unsigned)((warp & 3) * 32) << 16) + (unsigned)col0;
-#pragma unroll
-            for (int cc = 0; cc < DN / 2; cc += 16) {
-                unsigned v[16];
-                asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                             : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-                               "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                             : "r"(taddr + (unsigned)cc));
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-                for (int j = 0; j < 16; ++j) {
-                    const int dj = col0 + cc + j;
-                    float val = 0.0f;
-                    if (dj < nd && mr < nr && mc < ncw) {
-                        const VtiWindow w = vti_det_window(dets[s_list[d0 + dj]].box_lb, a.ph, a.pw);
-                        const int py = min(max(mpy, 0), a.ph - 1), px = min(max(mpx, 0), a.pw - 1);
-                        if (py >= w.cy_lo && py <= w.cy_hi && px >= w.cx_lo && px <= w.cx_hi) {
-                            const float acc = __uint_as_float(v[j]);
-                            val = VB ? acc : 1.0f / (1.0f + expf(-acc));
-                        }
-                    }
-                    s_c[dj * DT_M + my_m] = val;
-                }
-            }
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        // ---- epilogue 2: cells of every detection of this pass, one warp per detection (the unit form's code)
-        for (int j = warp; j < nd; j += DENSE_THREADS / 32) {
-            const int k = s_list[d0 + j];
-            vti_det* __restrict__ det = dets + k;
-            const unsigned f = det->flags;
-            const bool fabric = (f & VTI_F_FABRIC) && (f & VTI_F_IN_ROI);
-            if (fabric) { s_envw[warp][lane] = a.upper ? INT_MAX : -1; s_envw[warp][lane + 32] = a.upper ? INT_MAX : -1; }
-            __syncwarp();
-            unit_cells<EXPORT, VB>(a, b, k, det, fabric, R0, C0, nr, ncw, s_c + j * DT_M, s_envw[warp], lane);
-            __syncwarp();
-        }
-        __syncthreads();                                                   // s_c, sB are rewritten by the next pass
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" :: "r"(tmem), "n"(DN) : "memory");
-    }
-}
-
-
 // Host-buffer path: copy, per frame and channel, the union rectangle of the crop windows (the only prototype values the
 // unit kernel reads) from device-mapped pinned host memory into the device prototype buffer.  Rows are widened to
 // 16-byte boundaries for float4 accesses; blockIdx = (channel, frame), warps take rows.
@@ -499,17 +271,8 @@ __global__ void __launch_bounds__(256) k4_fetch_proto_kernel(const float* __rest
 
 }  // namespace
 
-int vti_k4_prepare() {
-    int rc;
-    if ((rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<true, true>, K4_DENSE_SMEM)) ||
-        (rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<true, false>, K4_DENSE_SMEM)) ||
-        (rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<false, true>, K4_DENSE_SMEM)) ||
-        (rc = vti_raise_dyn_smem((const void*)k4_dense_kernel<false, false>, K4_DENSE_SMEM))) return rc;
-    return VTI_OK;
-}
-
 int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const int32_t* counts, uint32_t* masks,
-                  int all_dets, cudaStream_t s) {
+                  cudaStream_t s) {
     K4Args a;
     a.proto = proto;
     a.dets = dets;
@@ -533,21 +296,11 @@ int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const
     const bool vb = h->p.mask_variant == 1;
     const bool k1_heavy = h->p.undistort || h->p.frame_w != h->g.new_w || h->p.frame_h != h->g.new_h;
     const int grid = (k1_heavy ? 2 : 4) * h->num_sms;
-    if (h->p.k4_dense == 2) { /* every frame goes through the tile form below: K3 emitted no units */ }
-    else if (masks && vb) k4_units_kernel<true, true><<<grid, K4_THREADS, 0, s>>>(a);
+    if (masks && vb) k4_units_kernel<true, true><<<grid, K4_THREADS, 0, s>>>(a);
     else if (masks) k4_units_kernel<true, false><<<grid, K4_THREADS, 0, s>>>(a);
     else if (vb) k4_units_kernel<false, true><<<grid, K4_THREADS, 0, s>>>(a);
     else k4_units_kernel<false, false><<<grid, K4_THREADS, 0, s>>>(a);
-    if (h->p.k4_dense != 2) h->launches++;
-    if (h->p.k4_dense) {
-        // tcgen05 tile form for the frames K3 flagged: one CTA per (tile, frame); CTAs of other frames / empty tiles exit
-        const dim3 dgrid(((a.pw + 1 + DT_C - 1) / DT_C) * ((a.ph + 1 + DT_R - 1) / DT_R), B);
-        if (masks && vb) k4_dense_kernel<true, true><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);
-        else if (masks) k4_dense_kernel<true, false><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);
-        else if (vb) k4_dense_kernel<false, true><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);
-        else k4_dense_kernel<false, false><<<dgrid, DENSE_THREADS, K4_DENSE_SMEM, s>>>(a, counts, h->d_dense, all_dets);
-        h->launches++;
-    }
+    h->launches++;
     VTI_CUDA(cudaGetLastError());
     return VTI_OK;
 }

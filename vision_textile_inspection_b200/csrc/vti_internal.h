@@ -9,6 +9,7 @@
 #include "../../include/vti.h"
 
 static_assert(sizeof(vti_det) == 160, "vti_det must stay 160 bytes");
+static_assert(sizeof(vti_params) == 320, "vti_params must stay 320 bytes (struct_size of existing callers)");
 
 #define VTI_CAND_CAP_MAX 32768      /* hard ceiling of the per-frame candidate list */
 #define VTI_CAND_CAP_DEFAULT 30000  /* Ultralytics' max_nms: with A <= 30000 anchors the list can never overflow */
@@ -40,7 +41,6 @@ struct vti_handle {
     int device;
     int num_sms;
     int64_t launches;
-    bool all_dets_env;                             // VTI_ALL_DETS, read at create
     VtiRoi roi;
     std::vector<void*> allocs;                     // every device allocation of the handle (vti_alloc)
 
@@ -69,7 +69,6 @@ struct vti_handle {
     uint4* d_units;                                // K4 work units: (frame | fabric << 15 | det << 16, block row | block col << 16,
                                                    //                 cx_lo | cy_lo << 16, cx_hi | cy_hi << 16)
     int units_per_det;                             // capacity per detection slot
-    int32_t* d_dense;                              // [B] 1 = this frame's masks go through the tcgen05 tile form of K4
     int4* d_proto_bbox;                            // [B] union of the crop windows of a frame (prototype pixels K4 reads)
     // ---- host-buffer path
     cudaStream_t own_stream, copy_stream;
@@ -120,7 +119,6 @@ int vti_raise_dyn_smem(const void* func, size_t bytes);
 // create-time preparation of the post kernels (dynamic shared-memory limits) and K3's padded candidate list length
 int vti_k3_prepare(int cap);
 int vti_k3_cap_pad(int cap);
-int vti_k4_prepare();
 int vti_k5_prepare(int max_det);
 // kernel launchers (each returns VTI_OK / VTI_ECUDA)
 int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector<int32_t>& yi,
@@ -131,7 +129,7 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cu
 int vti_launch_k2(vti_handle* h, const float* p3, const float* p4, const float* p5, int B, cudaStream_t s);
 int vti_launch_k3(vti_handle* h, const float* coef, int B, vti_det* dets, int32_t* counts, int all_dets, cudaStream_t s);
 int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const int32_t* counts, uint32_t* masks,
-                  int all_dets, cudaStream_t s);
+                  cudaStream_t s);
 int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* res, cudaStream_t s);
 // copies, per frame, the prototype rectangle K4 will read (all 32 channels) from device-mapped host memory
 int vti_launch_fetch_proto(vti_handle* h, const float* host_proto_mapped, float* dev_proto, int B, cudaStream_t s);

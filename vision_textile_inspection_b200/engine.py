@@ -62,7 +62,6 @@ class EngineConfig:
     max_px_distance: int = 250
     neighborhood: int = 3
     max_candidates: int = 0
-    k4_dense: int = 0             # tcgen05 tile form of the mask contraction: 0 never, 1 per frame by coverage, 2 always
     mask_variant: int = 0         # 0 = "A" (sigmoid, > 0.5), 1 = "B" (newer Ultralytics: logits, > 0.0, empty masks dropped)
 
     @staticmethod
@@ -93,7 +92,6 @@ class EngineConfig:
         p.min_stitches, p.max_px_distance, p.neighborhood = self.min_stitches, self.max_px_distance, self.neighborhood
         p.max_candidates = self.max_candidates
         p.mask_variant = int(self.mask_variant)
-        p.k4_dense = int(self.k4_dense)
         p.conf, p.iou = self.conf, self.iou
         p.iou_threshold = float(self.iou)          # the Python float torchvision.ops.nms receives (a C++ double)
         p.K[:] = np.asarray(self.K, np.float64).reshape(9).tolist()
