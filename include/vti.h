@@ -59,6 +59,9 @@ extern "C" {
 #define VTI_ST_NO_FABRIC 2   /* 'Fabric not detected'   measurement.py:281-287 */
 #define VTI_ST_NO_STITCH 3   /* 'No stitches detected'  measurement.py:332-337 */
 #define VTI_ST_OVERFLOW 0x100 /* OR-ed in: more NMS candidates than max_candidates (results truncated) */
+#define VTI_ST_BAD_CAMERA 0x200 /* OR-ed in: the frame's camera id was outside [0, n_cameras) (nothing routed or measured) */
+
+#define VTI_MAX_CAMERAS 256   /* cameras of one handle (vti_create_multi) */
 
 typedef struct vti_handle vti_handle;
 
@@ -91,6 +94,13 @@ typedef struct vti_params {
                                      sigmoid -> crop -> bilinear x4 -> > 0.5.  1 = "B" (newer releases): no sigmoid,
                                      crop, bilinear x4, > 0.0, and detections whose mask is empty are dropped */
 } vti_params;
+
+/* One camera's calibration on a multi-camera handle (vti_create_multi).  216 bytes. */
+typedef struct vti_camera {
+    int32_t struct_size;          /* = sizeof(vti_camera), ABI check */
+    int32_t reserved;             /* 0 */
+    double K[9], dist[5], R[9], t[3];   /* same meaning as in vti_params */
+} vti_camera;
 
 typedef struct vti_geometry {
     int32_t new_h, new_w;         /* resized (unpadded) size */
@@ -222,6 +232,36 @@ int vti_decode_jpeg(vti_handle* h, const uint8_t* jpeg, long long nbytes, uint8_
 int vti_decode_jpeg_batch(vti_handle* h, const uint8_t* const* jpegs, const long long* nbytes, int n, uint8_t* frames,
                           void* stream);
 const char* vti_jpeg_backend(void);
+
+/* ---- Several cameras of one frame size behind one handle.
+ * vti_create_multi: like vti_create, with the calibration of camera c taken from cameras[c] (p->K / dist / R / t are
+ * ignored).  n_cameras is 1..VTI_MAX_CAMERAS and every struct_size must match; both are checked before the device, so a
+ * machine without a GPU still reports VTI_EINVAL for bad arguments.  cameras[0] becomes the handle's own calibration:
+ * every entry point without a camera argument (vti_preprocess, vti_measure, vti_post_measure, vti_process_host[_yuyv],
+ * vti_annotate) treats each frame as camera 0.  vti_create(p) is vti_create_multi(p, 1, {p's calibration}).  Every
+ * per-camera table is built at create; steady state still allocates nothing.  Only K1 (the undistort remap) and K5
+ * (the pixel -> world projection) depend on the camera; vti_postprocess and vti_annotate take no camera ids.
+ *
+ * `camera`: one int32 camera id per frame -- a DEVICE array for the stream entry points, read by the kernels when they
+ * run (a captured CUDA graph follows the buffer's current contents), a HOST array for the two host-buffer entry points.
+ * NULL means camera 0 for every frame.  A device id outside [0, n_cameras) is never used as an index: K1 undistorts
+ * that frame with camera 0's tables (its net_in is unspecified), and K5 ORs VTI_ST_BAD_CAMERA into its status, leaves
+ * its records as K4 left them and routes and measures nothing (n_stitch = n_fabric = n_dist = n_width = env_valid = 0,
+ * NaN averages).  The host entry points check their ids before any work and return VTI_EINVAL. */
+int vti_create_multi(const vti_params* p, int n_cameras, const vti_camera* cameras, vti_handle** out);
+int vti_camera_count(const vti_handle* h);
+int vti_preprocess_multi(vti_handle* h, const uint8_t* frames, const int32_t* camera, int B, float* net_in, void* stream);
+int vti_measure_multi(vti_handle* h, int B, const int32_t* camera, vti_det* dets, const int32_t* counts,
+                      vti_frame_result* results, void* stream);
+int vti_post_measure_multi(vti_handle* h, const float* p3, const float* p4, const float* p5, const float* coef,
+                           const float* proto, int B, const int32_t* camera, vti_det* dets, int32_t* counts,
+                           uint32_t* masks, vti_frame_result* results, void* stream);
+int vti_process_host_multi(vti_handle* h, const uint8_t* frames, const float* p3, const float* p4, const float* p5,
+                           const float* coef, const float* proto, int B, const int32_t* camera, float* net_in,
+                           vti_det* dets, int32_t* counts, vti_frame_result* results);
+int vti_process_host_yuyv_multi(vti_handle* h, const uint8_t* yuyv, const float* p3, const float* p4, const float* p5,
+                                const float* coef, const float* proto, int B, const int32_t* camera, float* net_in,
+                                vti_det* dets, int32_t* counts, vti_frame_result* results);
 
 /* Number of kernel launches issued by this handle since creation (bench.py's gpu_launches). */
 int64_t vti_launch_count(const vti_handle* h);

@@ -14,6 +14,8 @@ VTI_NM = 32
 F_IN_ROI, F_STITCH, F_FABRIC, F_HAS_MASK, F_SELECTED, F_FINAL, F_HAS_WIDTH, F_HAS_DIST = 1, 2, 4, 8, 16, 32, 64, 128
 F_LB_MASK, F_DROPPED = 256, 512
 ST_OK, ST_NO_FABRIC, ST_NO_STITCH, ST_OVERFLOW = 0, 2, 3, 0x100
+ST_BAD_CAMERA = 0x200
+MAX_CAMERAS = 256
 
 
 class VtiParams(C.Structure):
@@ -27,6 +29,13 @@ class VtiParams(C.Structure):
         ("conf", C.c_float), ("iou", C.c_float),
         ("K", C.c_double * 9), ("dist", C.c_double * 5), ("R", C.c_double * 9), ("t", C.c_double * 3),
         ("iou_threshold", C.c_double), ("mask_variant", C.c_int32),
+    ]
+
+
+class VtiCamera(C.Structure):
+    _fields_ = [
+        ("struct_size", C.c_int32), ("reserved", C.c_int32),
+        ("K", C.c_double * 9), ("dist", C.c_double * 5), ("R", C.c_double * 9), ("t", C.c_double * 3),
     ]
 
 
@@ -59,6 +68,8 @@ EXPORTS = [
     "vti_preprocess", "vti_postprocess", "vti_measure", "vti_post_measure", "vti_process_host", "vti_launch_count",
     "vti_set_profiling", "vti_get_stage_ms", "vti_annotate", "vti_draw_text", "vti_encode_jpeg", "vti_decode_jpeg",
     "vti_decode_jpeg_batch", "vti_jpeg_backend", "vti_ingest_yuyv", "vti_process_host_yuyv",
+    "vti_create_multi", "vti_camera_count", "vti_preprocess_multi", "vti_measure_multi", "vti_post_measure_multi",
+    "vti_process_host_multi", "vti_process_host_yuyv_multi",
 ]
 
 _lib = None
@@ -104,6 +115,13 @@ def load():
     lib.vti_decode_jpeg_batch.argtypes = [vp, C.POINTER(C.c_char_p), C.POINTER(i64), i32, vp, vp]
     lib.vti_jpeg_backend.argtypes = []
     lib.vti_jpeg_backend.restype = C.c_char_p
+    lib.vti_create_multi.argtypes = [C.POINTER(VtiParams), i32, C.POINTER(VtiCamera), C.POINTER(vp)]
+    lib.vti_camera_count.argtypes = [vp]
+    lib.vti_preprocess_multi.argtypes = [vp, vp, vp, i32, vp, vp]
+    lib.vti_measure_multi.argtypes = [vp, i32, vp, vp, vp, vp, vp]
+    lib.vti_post_measure_multi.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp, vp]
+    lib.vti_process_host_multi.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
+    lib.vti_process_host_yuyv_multi.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp, vp, vp]
     for name in EXPORTS:
         getattr(lib, name)
     _lib = lib

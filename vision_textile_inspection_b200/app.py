@@ -49,6 +49,59 @@ def load_json(path):
         return json.load(f)
 
 
+def load_camera(calib_path, extr_path):
+    """(K, dist, R, t) of one camera from the reference's two JSON files, with its errors (measurement.py:127-146)."""
+    if not os.path.exists(calib_path):
+        raise FileNotFoundError(f"Calibration file missing: {calib_path}")
+    calib = load_json(calib_path)
+    K = np.array(calib["camera_matrix"], dtype=np.float64)
+    dist = np.array(calib["dist_coeffs"], dtype=np.float64).ravel()
+    if not os.path.exists(extr_path):
+        raise FileNotFoundError(f"Extrinsics file missing: {extr_path}")
+    extr = load_json(extr_path)
+    rvec = np.array(extr["rvec"], dtype=np.float64).reshape(3, 1)
+    t = np.array(extr["tvec"], dtype=np.float64).reshape(3,)
+    from .engine import rodrigues
+    try:
+        import cv2
+        R = cv2.Rodrigues(rvec)[0]
+    except Exception:  # pragma: no cover
+        R = rodrigues(rvec)
+    return K, dist, R, t
+
+
+def smooth(buf_dist: deque, buf_width: deque, avg_dist, avg_width):
+    """measurement.py:474-484 -- frame-ordered state, hence on the host."""
+    sd = sw = None
+    if avg_dist is not None:
+        buf_dist.append(avg_dist)
+        sd = float(np.median(buf_dist))
+    if avg_width is not None:
+        buf_width.append(avg_width)
+        sw = float(np.median(buf_width))
+    return sd, sw
+
+
+def measurement_dict(r, buf_dist: deque, buf_width: deque) -> dict:
+    """process_frame's dict (measurement.py:281-287, 332-337, 474-511) for one vti_frame_result, smoothing with the
+    camera's two deques."""
+    if int(r["status"]) & _lib.ST_OVERFLOW:
+        # more confidence-passing anchors than the handle's candidate capacity: the kept subset is not the
+        # top-scoring one (Ultralytics keeps the best max_nms) -- never silent
+        import warnings
+        warnings.warn(f"vti: candidate list overflow ({int(r['n_cand'])} candidates): raise max_candidates or conf",
+                      RuntimeWarning, stacklevel=3)
+    status = int(r["status"]) & 0xFF
+    if status in _ERRORS:
+        return {"edge_distance_mm": None, "stitch_width_mm": None, "stitch_count": 0,
+                "timestamp": datetime.now(), "error": _ERRORS[status]}
+    ad = None if np.isnan(r["avg_dist"]) else float(r["avg_dist"])
+    aw = None if np.isnan(r["avg_width"]) else float(r["avg_width"])
+    sd, sw = smooth(buf_dist, buf_width, ad, aw)
+    return {"edge_distance_mm": sd, "stitch_width_mm": sw, "stitch_count": int(r["n_dist"]),
+            "timestamp": datetime.now()}
+
+
 def force_camera_resolution(cap, w, h):
     """Same contract as measurement.py:23-42: set the capture size, report what the camera gave."""
     import cv2
@@ -199,22 +252,7 @@ class StitchMeasurementApp:
                  roi=ROI_DEFAULT, conf=CONF_THRESH, iou=IOU_THRESH, max_det=MAX_DETECTIONS, imgsz=960, undistort=0,
                  max_px_distance=MAX_PX_DISTANCE, neighborhood=ENVELOPE_NEIGHBORHOOD, annotate=True, device=None,
                  mask_variant=0, jpeg_quality=0):
-        if not os.path.exists(calib_path):
-            raise FileNotFoundError(f"Calibration file missing: {calib_path}")
-        calib = load_json(calib_path)
-        self.K = np.array(calib["camera_matrix"], dtype=np.float64)
-        self.dist = np.array(calib["dist_coeffs"], dtype=np.float64).ravel()
-        if not os.path.exists(extr_path):
-            raise FileNotFoundError(f"Extrinsics file missing: {extr_path}")
-        extr = load_json(extr_path)
-        rvec = np.array(extr["rvec"], dtype=np.float64).reshape(3, 1)
-        self.t = np.array(extr["tvec"], dtype=np.float64).reshape(3,)
-        from .engine import rodrigues
-        try:
-            import cv2
-            self.R = cv2.Rodrigues(rvec)[0]
-        except Exception:  # pragma: no cover
-            self.R = rodrigues(rvec)
+        self.K, self.dist, self.R, self.t = load_camera(calib_path, extr_path)
         self.n_c = self.R[:, 2].astype(np.float64)                  # measurement.py:44-48
         self.d_c = -float(self.n_c.dot(self.t))
 
@@ -245,32 +283,10 @@ class StitchMeasurementApp:
 
     # ------------------------------------------------------------------------------------------------------------
     def _smooth(self, avg_dist, avg_width):
-        """measurement.py:474-484 -- frame-ordered state, hence on the host."""
-        sd = sw = None
-        if avg_dist is not None:
-            self.frame_buf_dist.append(avg_dist)
-            sd = float(np.median(self.frame_buf_dist))
-        if avg_width is not None:
-            self.frame_buf_width.append(avg_width)
-            sw = float(np.median(self.frame_buf_width))
-        return sd, sw
+        return smooth(self.frame_buf_dist, self.frame_buf_width, avg_dist, avg_width)
 
     def _finish(self, r) -> dict:
-        if int(r["status"]) & _lib.ST_OVERFLOW:
-            # more confidence-passing anchors than the handle's candidate capacity: the kept subset is not the
-            # top-scoring one (Ultralytics keeps the best max_nms) -- never silent
-            import warnings
-            warnings.warn(f"vti: candidate list overflow ({int(r['n_cand'])} candidates): raise max_candidates or conf",
-                          RuntimeWarning, stacklevel=2)
-        status = int(r["status"]) & 0xFF
-        if status in _ERRORS:
-            return {"edge_distance_mm": None, "stitch_width_mm": None, "stitch_count": 0,
-                    "timestamp": datetime.now(), "error": _ERRORS[status]}
-        ad = None if np.isnan(r["avg_dist"]) else float(r["avg_dist"])
-        aw = None if np.isnan(r["avg_width"]) else float(r["avg_width"])
-        sd, sw = self._smooth(ad, aw)
-        return {"edge_distance_mm": sd, "stitch_width_mm": sw, "stitch_count": int(r["n_dist"]),
-                "timestamp": datetime.now()}
+        return measurement_dict(r, self.frame_buf_dist, self.frame_buf_width)
 
     def process_frames(self, frames: np.ndarray):
         """Batched form of process_frame: (B,h,w,3) uint8 -> list of measurement dicts, smoothing in frame order."""
@@ -425,3 +441,68 @@ class CheckStitchDistanceApp(StitchMeasurementApp):
             except Exception:  # pragma: no cover
                 pass
         return annotated, text
+
+
+class MultiCameraApp:
+    """Several cameras of one frame size behind ONE libvti handle: the reference's per-frame measurement
+    (StitchMeasurementApp.process_frame's dict, measurement.py semantics) for batches that mix cameras.
+
+    `cameras` = [(calib_path, extr_path), ...], one pair per camera as the reference reads them (FileNotFoundError
+    like StitchMeasurementApp).  Keywords as StitchMeasurementApp's (`backbone`, `roi`, `conf`, `iou`, `max_det`,
+    `imgsz`, `undistort`, `frame_buffer`, `min_stitches`, ...).  Each frame is undistorted (undistort=1) and measured
+    with its own camera's calibration; each camera keeps its own two median deques, fed in batch order.  The ROI,
+    thresholds and classes are shared by all cameras.  Opens no capture device and draws no overlay.
+    """
+
+    def __init__(self, cameras, model_path, frame_buffer=8, min_stitches=MIN_STITCHES, stitch_id=STITCH_CLASS_ID,
+                 fabric_id=FABRIC_CLASS_ID, *, backbone=None, roi=ROI_DEFAULT, conf=CONF_THRESH, iou=IOU_THRESH,
+                 max_det=MAX_DETECTIONS, imgsz=960, undistort=0, max_px_distance=MAX_PX_DISTANCE,
+                 neighborhood=ENVELOPE_NEIGHBORHOOD, device=None, mask_variant=0):
+        if not cameras or len(cameras) > _lib.MAX_CAMERAS:
+            raise ValueError(f"MultiCameraApp: 1..{_lib.MAX_CAMERAS} cameras, got {len(cameras or [])}")
+        self.cameras = [dict(zip(("K", "dist", "R", "t"), load_camera(cp, ep))) for cp, ep in cameras]
+        if not torch.cuda.is_available():
+            raise _lib.VtiError("MultiCameraApp needs a CUDA device: the hot path has no CPU fallback")
+        self.backbone = backbone if backbone is not None else backbone_from_ultralytics(model_path)
+        self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
+        self.config = dict(imgsz=imgsz, conf=conf, iou=iou, max_det=max_det, undistort=undistort,
+                           roi=tuple(int(v) for v in roi), min_stitches=min_stitches, stitch_id=stitch_id,
+                           fabric_id=fabric_id, max_px_distance=max_px_distance, neighborhood=neighborhood,
+                           mask_variant=mask_variant)
+        self.min_stitches = min_stitches
+        self.buffers = [(deque(maxlen=frame_buffer), deque(maxlen=frame_buffer)) for _ in self.cameras]
+        self._engines = {}
+        self.last_records = None
+
+    def engine_for(self, h, w, batch) -> InspectionEngine:
+        """The handle for (frame size, batch): every camera's tables, built once and kept."""
+        key = (h, w, batch)
+        eng = self._engines.get(key)
+        if eng is None:
+            c0 = self.cameras[0]
+            ec = EngineConfig(frame_h=h, frame_w=w, K=c0["K"], dist=c0["dist"], R=c0["R"], t=c0["t"], nc=2,
+                              max_batch=batch, channel_flip=0, cameras=self.cameras, **self.config)
+            eng = self._engines[key] = InspectionEngine(ec, self.device)
+        return eng
+
+    @torch.no_grad()
+    def process_frames(self, frames: np.ndarray, camera_ids) -> list:
+        """frames (B,h,w,3) uint8 BGR (or (B,h,w,2) packed YUYV) and camera_ids (B ints) -> B measurement dicts."""
+        frames = np.ascontiguousarray(frames)
+        B, h, w = frames.shape[:3]
+        ids = np.asarray(camera_ids).reshape(-1)
+        if ids.shape != (B,) or not np.issubdtype(ids.dtype, np.integer):
+            raise ValueError(f"process_frames: {B} integer camera ids expected, got {ids.dtype} {ids.shape}")
+        if B and (ids.min() < 0 or ids.max() >= len(self.cameras)):
+            raise ValueError(f"process_frames: camera ids must be in [0, {len(self.cameras)}), got {ids.tolist()}")
+        eng = self.engine_for(h, w, B)
+        cam = torch.from_numpy(ids.astype(np.int32)).to(self.device)
+        d_frames = torch.from_numpy(frames).to(self.device, non_blocking=True)
+        if frames.shape[3] == 2:
+            d_frames = eng.ingest_yuyv(d_frames)                            # K0
+        net_in = eng.preprocess(d_frames, camera=cam)                       # K1, each frame with its camera's remap
+        p3, p4, p5, coef, proto = self.backbone(net_in)
+        dets, counts, results, _ = eng.post_measure(p3, p4, p5, coef, proto, camera=cam)    # K2..K5
+        dets, counts, results = eng.dets_to_numpy(dets), counts.cpu().numpy(), eng.results_to_numpy(results)
+        self.last_records = [dets[b, :int(counts[b])] for b in range(B)]
+        return [measurement_dict(results[b], *self.buffers[int(ids[b])]) for b in range(B)]

@@ -197,11 +197,17 @@ extern "C" void vti_destroy(vti_handle* h) {
     delete h;
 }
 
-// vti_create after the argument checks; on failure vti_create destroys the partial handle
-static int init_handle(vti_handle* h, const vti_params* p) {
+// vti_create_multi after the argument checks; on failure the caller destroys the partial handle
+static int init_handle(vti_handle* h, const vti_params* params, int n_cameras, const vti_camera* cams) {
     VTI_CUDA(cudaGetDevice(&h->device));
     VTI_CUDA(cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device));
-    h->p = *p;
+    h->p = *params;
+    std::copy(cams[0].K, cams[0].K + 9, h->p.K);               // camera 0 is the handle's own calibration
+    std::copy(cams[0].dist, cams[0].dist + 5, h->p.dist);
+    std::copy(cams[0].R, cams[0].R + 9, h->p.R);
+    std::copy(cams[0].t, cams[0].t + 3, h->p.t);
+    h->n_cameras = n_cameras;
+    const vti_params* p = &h->p;
     int rc = vti_plan_geometry(p->frame_h, p->frame_w, p->imgsz, p->stride, p->max_det, p->max_candidates, &h->g);
     if (rc) return rc;
     {
@@ -245,25 +251,34 @@ static int init_handle(vti_handle* h, const vti_params* p) {
     if ((rc = vti_upload(h, &h->d_tap_x_idx, xi)) || (rc = vti_upload(h, &h->d_tap_x_a, xa)) ||
         (rc = vti_upload(h, &h->d_tap_y_i, yi)) || (rc = vti_upload(h, &h->d_tap_y_b, yb))) return rc;
     {
-        std::vector<int32_t> ix, iy;
+        // every camera's cv2.undistort source map, [camera][fh * fw] (1/32 px), and its packed displacements
+        std::vector<int32_t> ix, iy, packed;
         if (p->undistort) {
-            ix.resize((size_t)fh * fw); iy.resize((size_t)fh * fw);
-            std::vector<int32_t> packed((size_t)fh * fw);
-            vti_plan_undistort_map(p->K, p->dist, fh, fw, ix.data(), iy.data());
-            for (int v = 0; v < fh; ++v)
-                for (int u = 0; u < fw; ++u) {
-                    const size_t i = (size_t)v * fw + u;
-                    const int dx = ix[i] - 32 * u, dy = iy[i] - 32 * v;
-                    if (dx < -32768 || dx > 32767 || dy < -32768 || dy > 32767) {
-                        vti_set_error("vti_create: lens displacement exceeds +-1024 px, unsupported");
-                        return VTI_EINVAL;
+            const size_t npx = (size_t)fh * fw;
+            ix.resize(n_cameras * npx); iy.resize(n_cameras * npx); packed.resize(n_cameras * npx);
+            for (int c = 0; c < n_cameras; ++c) {
+                int32_t* cx = ix.data() + c * npx;
+                int32_t* cy = iy.data() + c * npx;
+                vti_plan_undistort_map(cams[c].K, cams[c].dist, fh, fw, cx, cy);
+                for (int v = 0; v < fh; ++v)
+                    for (int u = 0; u < fw; ++u) {
+                        const size_t i = (size_t)v * fw + u;
+                        const int dx = cx[i] - 32 * u, dy = cy[i] - 32 * v;
+                        if (dx < -32768 || dx > 32767 || dy < -32768 || dy > 32767) {
+                            vti_set_error(n_cameras == 1 ? std::string("vti_create: lens displacement exceeds +-1024 px, unsupported")
+                                                         : "vti_create_multi: lens displacement of camera " + std::to_string(c) +
+                                                               " exceeds +-1024 px, unsupported");
+                            return VTI_EINVAL;
+                        }
+                        packed[c * npx + i] = (int32_t)(((uint32_t)(uint16_t)(int16_t)dy << 16) | (uint32_t)(uint16_t)(int16_t)dx);
                     }
-                    packed[i] = (int32_t)(((uint32_t)(uint16_t)(int16_t)dy << 16) | (uint32_t)(uint16_t)(int16_t)dx);
-                }
-            if ((rc = vti_upload(h, &h->d_und_lut, packed))) return rc;
+            }
         }
-        if ((rc = vti_k1_plan(h, xi, yi, xa, yb, p->undistort ? &ix : nullptr, p->undistort ? &iy : nullptr))) return rc;
+        if ((rc = vti_k1_plan(h, xi, yi, xa, yb, p->undistort ? &ix : nullptr, p->undistort ? &iy : nullptr,
+                              p->undistort ? &packed : nullptr)))
+            return rc;
     }
+    if ((rc = vti_k5_cameras(h, cams, n_cameras))) return rc;
     // ---- measurement tables
     if ((rc = build_axis_lut(h, fh, g.LH, &h->lutY, nullptr)) || (rc = build_axis_lut(h, fw, g.LW, &h->lutX, &h->d_xmap)))
         return rc;
@@ -288,9 +303,8 @@ static int init_handle(vti_handle* h, const vti_params* p) {
     return VTI_OK;
 }
 
-extern "C" int vti_create(const vti_params* p, vti_handle** out) {
-    if (!p || !out) { vti_set_error("vti_create: null argument"); return VTI_EINVAL; }
-    *out = nullptr;
+// the checks of vti_params that need no device
+static int check_params(const vti_params* p) {
     if (p->struct_size != (int32_t)sizeof(vti_params)) {
         vti_set_error("vti_create: vti_params.struct_size mismatch (ABI)");
         return VTI_EINVAL;
@@ -303,6 +317,11 @@ extern "C" int vti_create(const vti_params* p, vti_handle** out) {
                       "neighborhood 0..7, variant 0/1, mask_variant 0/1)");
         return VTI_EINVAL;
     }
+    return VTI_OK;
+}
+
+// after the argument checks of both create calls
+static int create_checked(const vti_params* p, int n_cameras, const vti_camera* cams, vti_handle** out) {
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
         cudaGetLastError();
@@ -310,11 +329,44 @@ extern "C" int vti_create(const vti_params* p, vti_handle** out) {
         return VTI_ENODEV;
     }
     vti_handle* h = new vti_handle();
-    const int rc = init_handle(h, p);
+    const int rc = init_handle(h, p, n_cameras, cams);
     if (rc) { vti_destroy(h); return rc; }
     *out = h;
     return VTI_OK;
 }
+
+extern "C" int vti_create(const vti_params* p, vti_handle** out) {
+    if (!p || !out) { vti_set_error("vti_create: null argument"); return VTI_EINVAL; }
+    *out = nullptr;
+    int rc = check_params(p);
+    if (rc) return rc;
+    vti_camera cam{};                                          // the one camera: p's own calibration
+    cam.struct_size = (int32_t)sizeof(vti_camera);
+    std::copy(p->K, p->K + 9, cam.K);
+    std::copy(p->dist, p->dist + 5, cam.dist);
+    std::copy(p->R, p->R + 9, cam.R);
+    std::copy(p->t, p->t + 3, cam.t);
+    return create_checked(p, 1, &cam, out);
+}
+
+extern "C" int vti_create_multi(const vti_params* p, int n_cameras, const vti_camera* cameras, vti_handle** out) {
+    if (!p || !cameras || !out) { vti_set_error("vti_create_multi: null argument"); return VTI_EINVAL; }
+    *out = nullptr;
+    int rc = check_params(p);
+    if (rc) return rc;
+    if (n_cameras < 1 || n_cameras > VTI_MAX_CAMERAS) {
+        vti_set_error("vti_create_multi: n_cameras must be 1.." + std::to_string(VTI_MAX_CAMERAS));
+        return VTI_EINVAL;
+    }
+    for (int c = 0; c < n_cameras; ++c)
+        if (cameras[c].struct_size != (int32_t)sizeof(vti_camera)) {
+            vti_set_error("vti_create_multi: cameras[" + std::to_string(c) + "].struct_size mismatch (ABI)");
+            return VTI_EINVAL;
+        }
+    return create_checked(p, n_cameras, cameras, out);
+}
+
+extern "C" int vti_camera_count(const vti_handle* h) { return h ? h->n_cameras : VTI_EINVAL; }
 
 extern "C" int vti_get_geometry(const vti_handle* h, vti_geometry* out) {
     if (!h || !out) return VTI_EINVAL;
@@ -373,21 +425,28 @@ static int check_aligned(const char* fn, std::initializer_list<Aligned> bufs) {
     return VTI_OK;
 }
 
-extern "C" int vti_preprocess(vti_handle* h, const uint8_t* frames, int B, float* net_in, void* stream) {
+extern "C" int vti_preprocess_multi(vti_handle* h, const uint8_t* frames, const int32_t* camera, int B, float* net_in,
+                                    void* stream) {
     int rc = check_batch(h, B);
     if (rc) return rc;
     if (!frames || !net_in) { vti_set_error("vti_preprocess: null buffer"); return VTI_EINVAL; }
+    if ((rc = check_aligned("vti_preprocess_multi", {{"camera", camera, 4}}))) return rc;
     mark(h, 0, (cudaStream_t)stream);
-    rc = vti_launch_k1(h, frames, B, net_in, (cudaStream_t)stream);
+    rc = vti_launch_k1(h, frames, B, net_in, camera, (cudaStream_t)stream);
     mark(h, 1, (cudaStream_t)stream);
     return rc;
 }
 
+extern "C" int vti_preprocess(vti_handle* h, const uint8_t* frames, int B, float* net_in, void* stream) {
+    return vti_preprocess_multi(h, frames, nullptr, B, net_in, stream);
+}
+
 // K2 -> K3 -> K4 [-> K5], the one post chain of vti_postprocess (so of vti_post_measure) and of every chunk of
 // vti_process_host.  head: p3, p4, p5, coef, proto.  fetch_into: the prototypes are device-mapped host memory, fetched
-// after K3 (which sizes the rectangle K4 reads) into fetch_into.  results: K5 too.  timed: record the stage events.
+// after K3 (which sizes the rectangle K4 reads) into fetch_into.  results: K5 too, with the frames' camera ids (device,
+// or null).  timed: record the stage events.
 static int post_chain(vti_handle* h, const float* const head[5], float* fetch_into, int B, vti_det* dets, int32_t* counts,
-                      uint32_t* masks, vti_frame_result* results, bool timed, cudaStream_t s) {
+                      uint32_t* masks, vti_frame_result* results, const int32_t* camera, bool timed, cudaStream_t s) {
     auto stage = [&](int i) { if (timed) mark(h, i, s); };
     // K3 and K4 evaluate the masks of every kept detection, not only of the routed stitch / fabric ones, when masks are
     // exported and for mask variant B: it removes every detection whose mask is empty (newer Ultralytics,
@@ -402,7 +461,7 @@ static int post_chain(vti_handle* h, const float* const head[5], float* fetch_in
     if (fetch_into && (rc = vti_launch_fetch_proto(h, head[4], fetch_into, B, s))) return rc;
     if ((rc = vti_launch_k4(h, fetch_into ? fetch_into : head[4], B, dets, counts, masks, s))) return rc;
     stage(5);
-    return results ? vti_launch_k5(h, B, dets, counts, results, s) : VTI_OK;
+    return results ? vti_launch_k5(h, B, dets, counts, results, camera, s) : VTI_OK;
 }
 
 extern "C" int vti_postprocess(vti_handle* h, const float* p3, const float* p4, const float* p5, const float* coef,
@@ -414,27 +473,39 @@ extern "C" int vti_postprocess(vti_handle* h, const float* p3, const float* p4, 
     if ((rc = check_aligned("vti_postprocess", {{"dets", dets, 8}, {"counts", counts, 4}, {"p3", p3, 4}, {"p4", p4, 4}, {"p5", p5, 4},
                                                 {"coef", coef, 4}, {"proto", proto, 4}, {"masks", masks, 16}}))) return rc;
     const float* head[5] = {p3, p4, p5, coef, proto};
-    return post_chain(h, head, nullptr, B, dets, counts, masks, nullptr, true, (cudaStream_t)stream);
+    return post_chain(h, head, nullptr, B, dets, counts, masks, nullptr, nullptr, true, (cudaStream_t)stream);
+}
+
+extern "C" int vti_measure_multi(vti_handle* h, int B, const int32_t* camera, vti_det* dets, const int32_t* counts,
+                                 vti_frame_result* results, void* stream) {
+    int rc = check_batch(h, B);
+    if (rc) return rc;
+    if (!dets || !counts || !results) { vti_set_error("vti_measure: null buffer"); return VTI_EINVAL; }
+    if ((rc = check_aligned("vti_measure", {{"dets", dets, 8}, {"results", results, 8}, {"counts", counts, 4},
+                                            {"camera", camera, 4}}))) return rc;
+    mark(h, 6, (cudaStream_t)stream);
+    rc = vti_launch_k5(h, B, dets, counts, results, camera, (cudaStream_t)stream);
+    mark(h, 7, (cudaStream_t)stream);
+    return rc;
 }
 
 extern "C" int vti_measure(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* results,
                            void* stream) {
-    int rc = check_batch(h, B);
+    return vti_measure_multi(h, B, nullptr, dets, counts, results, stream);
+}
+
+extern "C" int vti_post_measure_multi(vti_handle* h, const float* p3, const float* p4, const float* p5, const float* coef,
+                                      const float* proto, int B, const int32_t* camera, vti_det* dets, int32_t* counts,
+                                      uint32_t* masks, vti_frame_result* results, void* stream) {
+    int rc = vti_postprocess(h, p3, p4, p5, coef, proto, B, dets, counts, masks, stream);
     if (rc) return rc;
-    if (!dets || !counts || !results) { vti_set_error("vti_measure: null buffer"); return VTI_EINVAL; }
-    if ((rc = check_aligned("vti_measure", {{"dets", dets, 8}, {"results", results, 8}, {"counts", counts, 4}}))) return rc;
-    mark(h, 6, (cudaStream_t)stream);
-    rc = vti_launch_k5(h, B, dets, counts, results, (cudaStream_t)stream);
-    mark(h, 7, (cudaStream_t)stream);
-    return rc;
+    return vti_measure_multi(h, B, camera, dets, counts, results, stream);
 }
 
 extern "C" int vti_post_measure(vti_handle* h, const float* p3, const float* p4, const float* p5, const float* coef,
                                 const float* proto, int B, vti_det* dets, int32_t* counts, uint32_t* masks,
                                 vti_frame_result* results, void* stream) {
-    int rc = vti_postprocess(h, p3, p4, p5, coef, proto, B, dets, counts, masks, stream);
-    if (rc) return rc;
-    return vti_measure(h, B, dets, counts, results, stream);
+    return vti_post_measure_multi(h, p3, p4, p5, coef, proto, B, nullptr, dets, counts, masks, results, stream);
 }
 
 // The host-buffer path's streams, events and buffers, made by its first call
@@ -450,6 +521,7 @@ static int create_staging(vti_handle* h) {
     alloc(&h->d_dets, sizeof(vti_det) * B * h->p.max_det);
     alloc(&h->d_counts, sizeof(int32_t) * B);
     alloc(&h->d_results, sizeof(vti_frame_result) * B);
+    alloc(&h->d_camera, sizeof(int32_t) * B);
     if (!rc) h->staged_batch = B;
     return rc;
 }
@@ -472,16 +544,23 @@ static const float* mapped_alias(const float* host) {
     return at.type == cudaMemoryTypeHost ? static_cast<const float*>(at.devicePointer) : nullptr;
 }
 
-// fmt 0: BGR frames (3 bytes per pixel); 1: camera-native YUYV (2 bytes per pixel, converted by K0 on the device)
+// fmt 0: BGR frames (3 bytes per pixel); 1: camera-native YUYV (2 bytes per pixel, converted by K0 on the device).
+// camera: HOST camera ids, or null (camera 0 throughout)
 static int process_host_impl(vti_handle* h, const uint8_t* frames, int fmt, const float* p3, const float* p4, const float* p5,
-                             const float* coef, const float* proto, int B, float* net_in, vti_det* dets,
-                             int32_t* counts, vti_frame_result* results) {
+                             const float* coef, const float* proto, int B, const int32_t* camera, float* net_in,
+                             vti_det* dets, int32_t* counts, vti_frame_result* results) {
     int rc = check_batch(h, B);
     if (rc) return rc;
     if (!frames || !p3 || !p4 || !p5 || !coef || !proto || !dets || !counts || !results) {
         vti_set_error("vti_process_host: null buffer");
         return VTI_EINVAL;
     }
+    for (int b = 0; camera && b < B; ++b)
+        if (camera[b] < 0 || camera[b] >= h->n_cameras) {
+            vti_set_error("vti_process_host_multi: camera id " + std::to_string(camera[b]) + " of frame " + std::to_string(b) +
+                          " is outside [0, " + std::to_string(h->n_cameras) + ")");
+            return VTI_EINVAL;
+        }
     if (fmt == 1 && (h->p.frame_w & 1)) { vti_set_error("vti_process_host_yuyv: packed 4:2:2 needs an even frame width"); return VTI_EINVAL; }
     const size_t keep = h->allocs.size();                  // all or nothing: a call after a failure starts clean
     if (!h->staged_batch && (rc = create_staging(h))) { release_from(h, keep); return rc; }
@@ -508,6 +587,8 @@ static int process_host_impl(vti_handle* h, const uint8_t* frames, int fmt, cons
         if (nb <= 0) continue;
         if (fmt == 1) VTI_CUDA(cudaMemcpyAsync(h->d_yuyv + b0 * ysz, frames + b0 * ysz, nb * ysz, cudaMemcpyHostToDevice, cs));
         else VTI_CUDA(cudaMemcpyAsync(h->d_frames + b0 * fsz, frames + b0 * fsz, nb * fsz, cudaMemcpyHostToDevice, cs));
+        const int32_t* cam = camera ? h->d_camera + b0 : nullptr;
+        if (camera) VTI_CUDA(cudaMemcpyAsync(h->d_camera + b0, camera + b0, sizeof(int32_t) * nb, cudaMemcpyHostToDevice, cs));
         const float* head[5];
         for (int t = 0; t < 5; ++t) {
             head[t] = (mapped[t] ? mapped[t] : h->d_head[t]) + b0 * hsz[t];
@@ -519,9 +600,9 @@ static int process_host_impl(vti_handle* h, const uint8_t* frames, int fmt, cons
         VTI_CUDA(cudaStreamWaitEvent(s, h->chunk_ev[c], 0));
         vti_det* cd = h->d_dets + (size_t)b0 * h->p.max_det;
         if (fmt == 1 && (rc = vti_launch_k0_yuyv(h, h->d_yuyv + b0 * ysz, nb, h->d_frames + b0 * fsz, s))) return rc;
-        if ((rc = vti_launch_k1(h, h->d_frames + b0 * fsz, nb, h->d_net_in + b0 * nsz, s))) return rc;
+        if ((rc = vti_launch_k1(h, h->d_frames + b0 * fsz, nb, h->d_net_in + b0 * nsz, cam, s))) return rc;
         if ((rc = post_chain(h, head, mapped[4] ? h->d_head[4] + b0 * hsz[4] : nullptr, nb, cd, h->d_counts + b0, nullptr,
-                             h->d_results + b0, false, s)))
+                             h->d_results + b0, cam, false, s)))
             return rc;
         if (net_in)
             VTI_CUDA(cudaMemcpyAsync(net_in + b0 * nsz, h->d_net_in + b0 * nsz, sizeof(float) * nb * nsz, cudaMemcpyDeviceToHost, s));
@@ -536,11 +617,24 @@ static int process_host_impl(vti_handle* h, const uint8_t* frames, int fmt, cons
 extern "C" int vti_process_host(vti_handle* h, const uint8_t* frames, const float* p3, const float* p4, const float* p5,
                                 const float* coef, const float* proto, int B, float* net_in, vti_det* dets,
                                 int32_t* counts, vti_frame_result* results) {
-    return process_host_impl(h, frames, 0, p3, p4, p5, coef, proto, B, net_in, dets, counts, results);
+    return process_host_impl(h, frames, 0, p3, p4, p5, coef, proto, B, nullptr, net_in, dets, counts, results);
+}
+
+extern "C" int vti_process_host_multi(vti_handle* h, const uint8_t* frames, const float* p3, const float* p4, const float* p5,
+                                      const float* coef, const float* proto, int B, const int32_t* camera, float* net_in,
+                                      vti_det* dets, int32_t* counts, vti_frame_result* results) {
+    return process_host_impl(h, frames, 0, p3, p4, p5, coef, proto, B, camera, net_in, dets, counts, results);
 }
 
 extern "C" int vti_process_host_yuyv(vti_handle* h, const uint8_t* yuyv, const float* p3, const float* p4, const float* p5,
                                      const float* coef, const float* proto, int B, float* net_in, vti_det* dets,
                                      int32_t* counts, vti_frame_result* results) {
-    return process_host_impl(h, yuyv, 1, p3, p4, p5, coef, proto, B, net_in, dets, counts, results);
+    return process_host_impl(h, yuyv, 1, p3, p4, p5, coef, proto, B, nullptr, net_in, dets, counts, results);
+}
+
+extern "C" int vti_process_host_yuyv_multi(vti_handle* h, const uint8_t* yuyv, const float* p3, const float* p4,
+                                           const float* p5, const float* coef, const float* proto, int B,
+                                           const int32_t* camera, float* net_in, vti_det* dets, int32_t* counts,
+                                           vti_frame_result* results) {
+    return process_host_impl(h, yuyv, 1, p3, p4, p5, coef, proto, B, camera, net_in, dets, counts, results);
 }

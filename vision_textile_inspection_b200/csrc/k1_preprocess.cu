@@ -19,6 +19,7 @@
 // HBM traffic: frame read once (tile halos hit L2) + 12*LH*LW written once; the 4 B/px remap table is L2-resident
 // across the batch.
 #include <algorithm>
+#include <type_traits>
 #include <vector>
 
 #include "vti_internal.h"
@@ -39,14 +40,19 @@ struct K1Args {
     const int16_t* tap_x_a;     // [new_w][2]
     const int32_t* tap_y_i;     // [new_h][2]
     const int16_t* tap_y_b;     // [new_h][2]
-    const int32_t* und_lut;     // [h*w] (dy16 << 16) | (dx16 & 0xffff)
-    const int4* tile_box;       // MODE_RAW: per tile (bx0, by0, bw, bh | interior << 30)
+    const int32_t* und_lut;     // [camera][h*w] (dy16 << 16) | (dx16 & 0xffff)
+    const int4* tile_box;       // MODE_RAW: [camera] per tile (bx0, by0, bw, bh | interior << 30)
     int h, w, new_h, new_w, top, left, LH, LW;
     int area2x;                 // exact-2x shrink: OpenCV's INTER_AREA switch
     int flip;
     int pitch_u;                // words per row of the footprint buffer
     int rows_u;                 // rows of the footprint buffer
     int undistort;
+};
+// The per-frame camera forms take the ids in a derived struct: the one-camera kernels keep their parameter block
+struct K1CamArgs : K1Args {
+    const int32_t* camera;      // [B] camera id per frame
+    int n_cameras;
 };
 
 __device__ __forceinline__ unsigned pack_px(unsigned b0, unsigned b1, unsigned b2, int flip) {
@@ -94,8 +100,9 @@ __device__ __forceinline__ unsigned remap_packed(unsigned t00, unsigned t01, uns
     return b | (g << 8) | (r << 16);
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a) {
+// Frame b takes camera b's remap tables (MULTI: a.camera[b]; an id out of range: camera 0's), else camera 0's.
+template <int MODE, bool MULTI>
+__global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const std::conditional_t<MULTI, K1CamArgs, K1Args> a) {
     extern __shared__ __align__(128) unsigned s_dyn[];     // [footprint rows][pitch_u] then the raw box (MODE_RAW)
     __shared__ float s_div[256];
     __shared__ int s_rowsrc[MAXROWS];
@@ -108,6 +115,15 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a
     const uint8_t* __restrict__ frame = a.frames + (size_t)b * a.h * a.w * 3;
     float* __restrict__ out = a.out + (size_t)b * 3 * a.LH * a.LW;
     unsigned* s_und = s_dyn;
+    const int32_t* und_lut = a.und_lut;
+    const int4* tile_box = a.tile_box;
+    if constexpr (MULTI) {
+        const int cam = __ldg(a.camera + b);
+        if ((unsigned)cam < (unsigned)a.n_cameras) {
+            und_lut += (size_t)cam * a.h * a.w;
+            tile_box += (size_t)cam * gridDim.x * gridDim.y;
+        }
+    }
 
     s_div[tid] = __fdiv_rn((float)tid, 255.0f);
 
@@ -165,7 +181,7 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a
             }
         } else if (MODE == MODE_RAW) {
             unsigned* s_raw = s_dyn + a.rows_u * a.pitch_u;
-            const int4 box = a.tile_box[blockIdx.y * gridDim.x + blockIdx.x];
+            const int4 box = tile_box[blockIdx.y * gridDim.x + blockIdx.x];
             const int bx0 = box.x, by0 = box.y, bw = box.z, bh = box.w & 0xFFFF;
             const bool interior = (box.w >> 30) & 1;
             for (int r = warp; r < bh; r += K1_THREADS / 32)
@@ -173,7 +189,7 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a
             __syncthreads();
             for (int r = warp; r < nrows; r += K1_THREADS / 32) {
                 const int sy = s_rowsrc[r];
-                const int32_t* __restrict__ lrow = a.und_lut + (size_t)sy * a.w;
+                const int32_t* __restrict__ lrow = und_lut + (size_t)sy * a.w;
                 for (int c = lane; c < ncols; c += 32) {
                     const int sx = c_lo + c;
                     const int lut = __ldg(lrow + sx);
@@ -199,7 +215,7 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a
                 const int sy = s_rowsrc[r];
                 for (int c = lane; c < ncols; c += 32) {
                     const int sx = s_colsrc[c];
-                    const int lut = __ldg(a.und_lut + (size_t)sy * a.w + sx);
+                    const int lut = __ldg(und_lut + (size_t)sy * a.w + sx);
                     const int ix = sx * 32 + (int)(short)(lut & 0xffff), iy = sy * 32 + (lut >> 16);
                     const int x = ix >> 5, y = iy >> 5;
                     const bool x0 = (unsigned)x < (unsigned)a.w, x1 = (unsigned)(x + 1) < (unsigned)a.w;
@@ -299,8 +315,8 @@ constexpr int K1_RAWP = 112;                 // raw-box row pitch (words) baked 
 struct K1FastArgs {
     const uint8_t* frames;
     float* out;
-    const int4* tile_hdr;       // [tiles][2]: (bx0, by0, bw, bh), (r_lo, c_lo, nrows, ncols)
-    const unsigned* lut;        // [tiles][lut_stride] 4-byte entries   (REMAP only)
+    const int4* tile_hdr;       // [camera][tiles][2]: (bx0, by0, bw, bh), (r_lo, c_lo, nrows, ncols)
+    const unsigned* lut;        // [camera][tiles][lut_stride] 4-byte entries, + one spare chunk   (REMAP only)
     const int32_t* tap_x_idx;   // [new_w]
     const int16_t* tap_x_a;     // [new_w][2]
     const int32_t* tap_y_i;     // [new_h][2]
@@ -310,7 +326,11 @@ struct K1FastArgs {
     int pitch_u, rows_u;
     int und_words;              // words reserved for the footprint buffer (multiple of FT_CHUNK, > rows_u * pitch_u)
     int lut_stride;             // entries per tile (multiple of FT_CHUNK)
-    int raw_pitch;              // words per row of the raw box in shared memory (the same for every tile)
+    int raw_pitch;              // words per row of the raw box in shared memory (the same for every tile and camera)
+};
+struct K1FastCamArgs : K1FastArgs {
+    const int32_t* camera;      // [B] camera id per frame
+    int n_cameras;
 };
 
 // Stage rows [y0, y0+nr) x 8-pixel groups [x0, x0 + 8*ng) of the frame as packed words (B | G<<8 | R<<16, byte 3 = 0);
@@ -516,8 +536,9 @@ __device__ __forceinline__ void resize_phase(const K1FastArgs& a, float* __restr
     }
 }
 
-template <bool REMAP, bool AREA, int LW_T, int RAWP_T>
-__global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const K1FastArgs a) {
+// MULTI (REMAP only): frame b takes the headers and remap table of camera a.camera[b] (an id out of range: camera 0's).
+template <bool REMAP, bool AREA, int LW_T, int RAWP_T, bool MULTI>
+__global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const std::conditional_t<MULTI, K1FastCamArgs, K1FastArgs> a) {
     extern __shared__ __align__(128) unsigned s_dyn[];     // s_und [und_words], then the raw box (REMAP)
     __shared__ int4 s_rowtap[FTY];                          // (byte offset row0, byte offset row1, b0, b1)
 
@@ -529,8 +550,18 @@ __global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const K1Fa
     const uint8_t* __restrict__ frame = a.frames + (size_t)b * a.h * a.w * 3;
     float* __restrict__ out = a.out + (size_t)b * 3 * a.LH * LW;
     unsigned* s_und = s_dyn;
+    const int4* tile_hdr = a.tile_hdr;
+    const unsigned* lut_base = a.lut;
+    if constexpr (MULTI) {
+        const int cam = __ldg(a.camera + b);
+        if ((unsigned)cam < (unsigned)a.n_cameras) {
+            const size_t ntiles = (size_t)gridDim.x * gridDim.y;
+            tile_hdr += 2 * ntiles * cam;
+            lut_base += ntiles * a.lut_stride * cam;
+        }
+    }
 
-    const int4 h0 = __ldg(a.tile_hdr + 2 * tile), h1 = __ldg(a.tile_hdr + 2 * tile + 1);
+    const int4 h0 = __ldg(tile_hdr + 2 * tile), h1 = __ldg(tile_hdr + 2 * tile + 1);
     const int r_lo = h1.x, c_lo = h1.y, nrows = h1.z;
     if (tid < FTY) {
         const int ry = Y0 + tid - a.top;
@@ -559,7 +590,7 @@ __global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const K1Fa
             const int rem = total - n_it * FT_CHUNK;
             const unsigned raw8 = smem_addr(s_raw);
             const unsigned bw4 = (unsigned)a.raw_pitch * 4u;
-            const unsigned* __restrict__ lut = a.lut + (size_t)tile * a.lut_stride + tid;
+            const unsigned* __restrict__ lut = lut_base + (size_t)tile * a.lut_stride + tid;
             unsigned e0 = __ldg(lut), e1 = __ldg(lut + FT_THREADS);
             for (int it = 0; it < n_it; ++it, dst += FT_CHUNK) {
                 lut += FT_CHUNK;                               // next entries in flight while these are computed
@@ -588,8 +619,10 @@ __global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const K1Fa
 // ---------------------------------------------------------------------------------------------------- host plan
 // Mirrors the kernel's per-tile footprint logic to size the shared buffers and, with undistort on, to find the
 // raw-frame bounding box of every tile's remap taps.
-// Fast-path plan: per-tile headers and (undistort) the per-tile pre-resolved remap table.  Returns false when the
-// geometry is not eligible (the generic kernel below takes over).
+// Fast-path plan: per-tile headers and (undistort) the per-tile pre-resolved remap table, per camera.  The footprints
+// come from the resize taps alone and are the same for every camera; the raw boxes and the remap entries are per camera,
+// at one raw-box pitch common to all cameras.  Returns false when the geometry is not eligible for every camera (the
+// generic kernel below takes over).
 static bool k1_fast_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector<int32_t>& yi,
                          const std::vector<int16_t>& xa, const std::vector<int16_t>& yb,
                          const std::vector<int32_t>* und_ix, const std::vector<int32_t>* und_iy,
@@ -637,52 +670,65 @@ static bool k1_fast_plan(vti_handle* h, const std::vector<int32_t>& xi, const st
     lut_stride = (rows_u * pitch_u + FT_CHUNK - 1) / FT_CHUNK * FT_CHUNK;
     raw_pitch = 0;
     if (!und_ix) return true;
-    // pass 2: raw boxes, then remap entries (entry 0 = offset 0, weights 0: a valid cell for the padded tail)
-    const size_t ntiles = (size_t)ntx * nty;
+    // pass 2: (1) every camera's raw boxes, (2) one raw-box pitch and height for all of them, (3) every camera's remap
+    // entries at that pitch (entry 0 = offset 0, weights 0: a valid cell for the padded tail)
+    const size_t ntiles = (size_t)ntx * nty, npx = (size_t)fh * fw;
+    const int ncam = h->n_cameras;
     auto clampx = [&](int x) { return x < -1 ? -2 : (x > fw - 1 ? fw : x); };
     auto clampy = [&](int y) { return y < -1 ? -2 : (y > fh - 1 ? fh : y); };
     int bh_max = 0;
-    for (size_t t = 0; t < ntiles; ++t) {
-        const int4 f = hdr[2 * t + 1];
-        const int r_lo = f.x, c_lo = f.y, nrows = f.z;
-        if (nrows == 0) continue;
-        const int c_end = std::min(c_lo + pitch_u, fw);            // remap every staged column that exists
-        int minx = INT32_MAX, miny = INT32_MAX, maxx = INT32_MIN, maxy = INT32_MIN;
-        for (int sy = r_lo; sy < r_lo + nrows; ++sy)
-            for (int sx = c_lo; sx < c_end; ++sx) {
-                const size_t i = (size_t)sy * fw + sx;
-                const int x = clampx((*und_ix)[i] >> 5), y = clampy((*und_iy)[i] >> 5);
-                minx = std::min(minx, x); maxx = std::max(maxx, x);
-                miny = std::min(miny, y); maxy = std::max(maxy, y);
-            }
-        const int bx0 = (minx >= 0) ? (minx & ~7) : -8;
-        const int bx1 = (maxx + 2 + 7) & ~7;                        // exclusive, covers x + 1
-        const int bw = bx1 - bx0, by0 = miny, bh = maxy + 2 - miny;
-        if ((size_t)bw * bh > 16384) return false;                  // 16-bit byte offsets
-        raw_words = std::max(raw_words, (size_t)bw * bh);
-        raw_pitch = std::max(raw_pitch, bw);
-        bh_max = std::max(bh_max, bh);
-        hdr[2 * t] = make_int4(bx0, by0, bw, bh);
+    std::vector<int4> boxes((size_t)ncam * ntiles, make_int4(0, 0, 0, 0));
+    for (int cam = 0; cam < ncam; ++cam) {
+        const int32_t* ux = und_ix->data() + cam * npx;
+        const int32_t* uy = und_iy->data() + cam * npx;
+        for (size_t t = 0; t < ntiles; ++t) {
+            const int4 f = hdr[2 * t + 1];
+            const int r_lo = f.x, c_lo = f.y, nrows = f.z;
+            if (nrows == 0) continue;
+            const int c_end = std::min(c_lo + pitch_u, fw);        // remap every staged column that exists
+            int minx = INT32_MAX, miny = INT32_MAX, maxx = INT32_MIN, maxy = INT32_MIN;
+            for (int sy = r_lo; sy < r_lo + nrows; ++sy)
+                for (int sx = c_lo; sx < c_end; ++sx) {
+                    const size_t i = (size_t)sy * fw + sx;
+                    const int x = clampx(ux[i] >> 5), y = clampy(uy[i] >> 5);
+                    minx = std::min(minx, x); maxx = std::max(maxx, x);
+                    miny = std::min(miny, y); maxy = std::max(maxy, y);
+                }
+            const int bx0 = (minx >= 0) ? (minx & ~7) : -8;
+            const int bx1 = (maxx + 2 + 7) & ~7;                    // exclusive, covers x + 1
+            const int bw = bx1 - bx0, by0 = miny, bh = maxy + 2 - miny;
+            if ((size_t)bw * bh > 16384) return false;              // 16-bit byte offsets
+            raw_pitch = std::max(raw_pitch, bw);
+            bh_max = std::max(bh_max, bh);
+            boxes[cam * ntiles + t] = make_int4(bx0, by0, bw, bh);
+        }
     }
     {                                                               // every tile's raw box at ONE pitch
         if (raw_pitch <= K1_RAWP) raw_pitch = K1_RAWP;              // the pitch the kernel has as an immediate
         if ((size_t)raw_pitch * bh_max > 16384) return false;
         raw_words = (size_t)raw_pitch * bh_max;                     // every tile's box at the one pitch
     }
-    lut.assign(ntiles * lut_stride + FT_CHUNK, 0u);         // + one spare chunk: the loop prefetches
+    const std::vector<int4> foot(hdr);
+    hdr.assign((size_t)ncam * ntiles * 2, make_int4(0, 0, 0, 0));
+    lut.assign((size_t)ncam * ntiles * lut_stride + FT_CHUNK, 0u);  // + one spare chunk: the loop prefetches
+    for (int cam = 0; cam < ncam; ++cam)
     for (size_t t = 0; t < ntiles; ++t) {
-        const int4 f = hdr[2 * t + 1], bx = hdr[2 * t];
+        const int4 f = foot[2 * t + 1], bx = boxes[cam * ntiles + t];
+        hdr[2 * (cam * ntiles + t)] = bx;
+        hdr[2 * (cam * ntiles + t) + 1] = f;
         const int r_lo = f.x, c_lo = f.y, nrows = f.z;
         if (nrows == 0) continue;
         const int bx0 = bx.x, by0 = bx.y, bw = raw_pitch;
-        unsigned* L = lut.data() + t * lut_stride;
+        const int32_t* ux = und_ix->data() + cam * npx;
+        const int32_t* uy = und_iy->data() + cam * npx;
+        unsigned* L = lut.data() + (cam * ntiles + t) * lut_stride;
         for (int r = 0; r < nrows; ++r)
             for (int c = 0; c < pitch_u; ++c) {
                 const int sy = r_lo + r, sx = c_lo + c;
                 unsigned off = 0u, fx = 0u, fy = 0u;                // columns past the frame: any valid cell
                 if (sx < fw) {
                     const size_t i = (size_t)sy * fw + sx;
-                    const int ix = (*und_ix)[i], iy = (*und_iy)[i];
+                    const int ix = ux[i], iy = uy[i];
                     const int x = clampx(ix >> 5), y = clampy(iy >> 5);
                     off = (unsigned)(((y - by0) * bw + (x - bx0)) * 4);
                     fx = (unsigned)(ix & 31); fy = (unsigned)(iy & 31);
@@ -696,44 +742,56 @@ static bool k1_fast_plan(vti_handle* h, const std::vector<int32_t>& xi, const st
 
 // The one place that names every instantiation of the fast kernel: launch == 0 raises each one's dynamic
 // shared-memory limit (plan time), launch == 1 launches the one that matches the handle.
-template <bool REMAP, bool AREA, int LW_T, int RAWP_T>
-static int k1_fast_one(const K1FastArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
-    if (!launch) return vti_raise_dyn_smem((const void*)k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T>, smem);
-    k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T><<<*grid, FT_THREADS, smem, s>>>(*f);
+template <bool REMAP, bool AREA, int LW_T, int RAWP_T, bool MULTI>
+static int k1_fast_one(const K1FastCamArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
+    if (!launch) return vti_raise_dyn_smem((const void*)k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI>, smem);
+    if constexpr (MULTI) k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI><<<*grid, FT_THREADS, smem, s>>>(*f);
+    else k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI><<<*grid, FT_THREADS, smem, s>>>(static_cast<const K1FastArgs&>(*f));
     return VTI_OK;
 }
-template <int LW_T>
-static int k1_fast_lw(bool remap, bool area, int rawp, const K1FastArgs* f, int launch, const dim3* grid, size_t smem,
-                      cudaStream_t s) {
+template <bool AREA, int LW_T, int RAWP_T>
+static int k1_fast_remap(bool multi, const K1FastCamArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
     int rc = VTI_OK;
-    const bool fixed = rawp == K1_RAWP;
-    if (!launch || (remap && area && fixed)) if ((rc = k1_fast_one<true, true, LW_T, K1_RAWP>(f, launch, grid, smem, s))) return rc;
-    if (!launch || (remap && !area && fixed)) if ((rc = k1_fast_one<true, false, LW_T, K1_RAWP>(f, launch, grid, smem, s))) return rc;
-    if (!launch || (remap && area && !fixed)) if ((rc = k1_fast_one<true, true, LW_T, 0>(f, launch, grid, smem, s))) return rc;
-    if (!launch || (remap && !area && !fixed)) if ((rc = k1_fast_one<true, false, LW_T, 0>(f, launch, grid, smem, s))) return rc;
-    if (!launch || (!remap && area)) if ((rc = k1_fast_one<false, true, LW_T, 0>(f, launch, grid, smem, s))) return rc;
-    if (!launch || (!remap && !area)) if ((rc = k1_fast_one<false, false, LW_T, 0>(f, launch, grid, smem, s))) return rc;
+    if (!launch || !multi) if ((rc = k1_fast_one<true, AREA, LW_T, RAWP_T, false>(f, launch, grid, smem, s))) return rc;
+    if (!launch || multi) rc = k1_fast_one<true, AREA, LW_T, RAWP_T, true>(f, launch, grid, smem, s);
     return rc;
 }
-static int k1_fast_dispatch(vti_handle* h, const K1FastArgs* f, int launch, const dim3* grid, size_t smem,
-                            cudaStream_t s = nullptr) {
+template <int LW_T>
+static int k1_fast_lw(bool remap, bool area, int rawp, bool multi, const K1FastCamArgs* f, int launch, const dim3* grid,
+                      size_t smem, cudaStream_t s) {
+    int rc = VTI_OK;
+    const bool fixed = rawp == K1_RAWP;
+    if (!launch || (remap && area && fixed)) if ((rc = k1_fast_remap<true, LW_T, K1_RAWP>(multi, f, launch, grid, smem, s))) return rc;
+    if (!launch || (remap && !area && fixed)) if ((rc = k1_fast_remap<false, LW_T, K1_RAWP>(multi, f, launch, grid, smem, s))) return rc;
+    if (!launch || (remap && area && !fixed)) if ((rc = k1_fast_remap<true, LW_T, 0>(multi, f, launch, grid, smem, s))) return rc;
+    if (!launch || (remap && !area && !fixed)) if ((rc = k1_fast_remap<false, LW_T, 0>(multi, f, launch, grid, smem, s))) return rc;
+    if (!launch || (!remap && area)) if ((rc = k1_fast_one<false, true, LW_T, 0, false>(f, launch, grid, smem, s))) return rc;
+    if (!launch || (!remap && !area)) if ((rc = k1_fast_one<false, false, LW_T, 0, false>(f, launch, grid, smem, s))) return rc;
+    return rc;
+}
+// multi: the per-frame camera form (remap only; without undistort K1 does not depend on the camera)
+static int k1_fast_dispatch(vti_handle* h, const K1FastCamArgs* f, int launch, const dim3* grid, size_t smem,
+                            cudaStream_t s = nullptr, bool multi = false) {
     const bool remap = h->k1_mode == MODE_FAST_REMAP, area = h->resize_mode == 2;
     const int LW = h->g.LW, rawp = h->k1_raw_pitch;
     int rc = VTI_OK;
     // imgsz 960 and 640 letterboxes (every BASELINE config) get the output row pitch as a compile-time constant: the
     // plane stores take immediate offsets
-    if (!launch || LW == 960) if ((rc = k1_fast_lw<960>(remap, area, rawp, f, launch, grid, smem, s))) return rc;
-    if (!launch || LW == 640) if ((rc = k1_fast_lw<640>(remap, area, rawp, f, launch, grid, smem, s))) return rc;
-    if (!launch || (LW != 960 && LW != 640)) rc = k1_fast_lw<0>(remap, area, rawp, f, launch, grid, smem, s);
+    if (!launch || LW == 960) if ((rc = k1_fast_lw<960>(remap, area, rawp, multi, f, launch, grid, smem, s))) return rc;
+    if (!launch || LW == 640) if ((rc = k1_fast_lw<640>(remap, area, rawp, multi, f, launch, grid, smem, s))) return rc;
+    if (!launch || (LW != 960 && LW != 640)) rc = k1_fast_lw<0>(remap, area, rawp, multi, f, launch, grid, smem, s);
     return rc;
 }
 
 int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector<int32_t>& yi,
                 const std::vector<int16_t>& xa, const std::vector<int16_t>& yb,
-                const std::vector<int32_t>* und_ix, const std::vector<int32_t>* und_iy) {
+                const std::vector<int32_t>* und_ix, const std::vector<int32_t>* und_iy,
+                const std::vector<int32_t>* und_packed) {
     const vti_geometry& g = h->g;
     const int fw = h->p.frame_w, fh = h->p.frame_h;
     const int ntx = (g.LW + TX - 1) / TX, nty = (g.LH + TY - 1) / TY;
+    const int ncam = h->n_cameras;
+    const size_t npx = (size_t)fh * fw, ntiles = (size_t)ntx * nty;
     {
         std::vector<int4> hdr;
         std::vector<unsigned> lut;
@@ -761,7 +819,7 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
     }
     int ncols_max = 4, nrows_max = 1;
     bool all_contig = true;
-    std::vector<int4> boxes((size_t)ntx * nty, make_int4(0, 0, 0, 0));
+    std::vector<int4> boxes(ncam * ntiles, make_int4(0, 0, 0, 0));
     size_t raw_max = 0;
     for (int ty = 0; ty < nty; ++ty)
         for (int tx = 0; tx < ntx; ++tx) {
@@ -779,31 +837,35 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
             ncols_max = std::max(ncols_max, ncols);
             all_contig = all_contig && rc && cc;
             if (und_ix && rc && cc) {
-                int minx = INT32_MAX, miny = INT32_MAX, maxx = -1, maxy = -1;
-                bool interior = true;
-                for (int sy = r_lo; sy <= r_hi; ++sy)
-                    for (int sx = c_lo; sx <= c_hi; ++sx) {
-                        const size_t i = (size_t)sy * fw + sx;
-                        const int x = (*und_ix)[i] >> 5, y = (*und_iy)[i] >> 5;
-                        for (int dy = 0; dy < 2; ++dy)
-                            for (int dx = 0; dx < 2; ++dx) {
-                                const int xx = x + dx, yy = y + dy;
-                                if (xx < 0 || xx >= fw || yy < 0 || yy >= fh) { interior = false; continue; }
-                                minx = std::min(minx, xx); maxx = std::max(maxx, xx);
-                                miny = std::min(miny, yy); maxy = std::max(maxy, yy);
-                            }
+                for (int cam = 0; cam < ncam; ++cam) {
+                    const int32_t* ux = und_ix->data() + cam * npx;
+                    const int32_t* uy = und_iy->data() + cam * npx;
+                    int minx = INT32_MAX, miny = INT32_MAX, maxx = -1, maxy = -1;
+                    bool interior = true;
+                    for (int sy = r_lo; sy <= r_hi; ++sy)
+                        for (int sx = c_lo; sx <= c_hi; ++sx) {
+                            const size_t i = (size_t)sy * fw + sx;
+                            const int x = ux[i] >> 5, y = uy[i] >> 5;
+                            for (int dy = 0; dy < 2; ++dy)
+                                for (int dx = 0; dx < 2; ++dx) {
+                                    const int xx = x + dx, yy = y + dy;
+                                    if (xx < 0 || xx >= fw || yy < 0 || yy >= fh) { interior = false; continue; }
+                                    minx = std::min(minx, xx); maxx = std::max(maxx, xx);
+                                    miny = std::min(miny, yy); maxy = std::max(maxy, yy);
+                                }
+                        }
+                    int4 bx = make_int4(0, 0, 4, 0);
+                    if (maxx >= 0) {
+                        bx.x = minx & ~3;
+                        bx.z = std::min(((maxx + 1 + 3) & ~3), (fw + 3) & ~3) - bx.x;
+                        bx.y = miny;
+                        bx.w = maxy - miny + 1;
                     }
-                int4 bx = make_int4(0, 0, 4, 0);
-                if (maxx >= 0) {
-                    bx.x = minx & ~3;
-                    bx.z = std::min(((maxx + 1 + 3) & ~3), (fw + 3) & ~3) - bx.x;
-                    bx.y = miny;
-                    bx.w = maxy - miny + 1;
+                    raw_max = std::max(raw_max, (size_t)bx.z * (bx.w & 0xFFFF));
+                    if (bx.w > 0xFFFF) all_contig = false;
+                    bx.w |= interior ? (1 << 30) : 0;
+                    boxes[cam * ntiles + (size_t)ty * ntx + tx] = bx;
                 }
-                raw_max = std::max(raw_max, (size_t)bx.z * (bx.w & 0xFFFF));
-                if (bx.w > 0xFFFF) all_contig = false;
-                bx.w |= interior ? (1 << 30) : 0;
-                boxes[(size_t)ty * ntx + tx] = bx;
             }
         }
     h->k1_pitch_u = (ncols_max + 3) & ~3;
@@ -812,6 +874,7 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
     h->k1_mode = MODE_PLAIN;
     h->k1_smem = und_bytes;
     if (h->p.undistort) {
+        if (const int rc = vti_upload(h, &h->d_und_lut, *und_packed)) return rc;
         const size_t tot = und_bytes + raw_max * 4;
         if (all_contig && (fw & 3) == 0 && tot <= 160 * 1024) {
             h->k1_mode = MODE_RAW;
@@ -821,18 +884,28 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
             h->k1_mode = MODE_GATHER;
         }
     }
-    if (h->k1_mode == MODE_RAW) return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_RAW>, h->k1_smem);
-    if (h->k1_mode == MODE_GATHER) return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_GATHER>, h->k1_smem);
-    return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_PLAIN>, h->k1_smem);
+    int rc;
+    if (h->k1_mode == MODE_RAW) {
+        if ((rc = vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_RAW, false>, h->k1_smem))) return rc;
+        return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_RAW, true>, h->k1_smem);
+    }
+    if (h->k1_mode == MODE_GATHER) {
+        if ((rc = vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_GATHER, false>, h->k1_smem))) return rc;
+        return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_GATHER, true>, h->k1_smem);
+    }
+    return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_PLAIN, false>, h->k1_smem);
 }
 
-int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cudaStream_t s) {
+// camera: per-frame ids (device) or null.  Only the remap depends on the camera, and a one-camera handle has one set of
+// tables for every id, so the per-frame form runs only for undistort with more than one camera.
+int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, const int32_t* camera, cudaStream_t s) {
+    const bool multi = camera && h->p.undistort && h->n_cameras > 1;
     if (h->k1_mode == MODE_FAST_PLAIN || h->k1_mode == MODE_FAST_REMAP) {
         if ((reinterpret_cast<uintptr_t>(frames) & 7) || (reinterpret_cast<uintptr_t>(net_in) & 3)) {
             vti_set_error("vti_preprocess: frames must be 8-byte aligned and net_in 4-byte aligned (64-bit staging loads)");
             return VTI_EINVAL;
         }
-        K1FastArgs f;
+        K1FastCamArgs f;
         f.frames = frames; f.out = net_in;
         f.tile_hdr = h->d_k1_tiles; f.lut = h->d_k1_lut;
         f.tap_x_idx = h->d_tap_x_idx; f.tap_x_a = h->d_tap_x_a; f.tap_y_i = h->d_tap_y_i; f.tap_y_b = h->d_tap_y_b;
@@ -842,14 +915,15 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cu
         f.pitch_u = h->k1_pitch_u; f.rows_u = h->k1_rows_u;
         f.und_words = h->k1_und_words; f.lut_stride = h->k1_lut_stride;
         f.raw_pitch = h->k1_raw_pitch;
+        f.camera = camera; f.n_cameras = h->n_cameras;
         dim3 grid((f.LW + FTX - 1) / FTX, (f.LH + FTY - 1) / FTY, B);
-        int rc = k1_fast_dispatch(h, &f, 1, &grid, h->k1_smem, s);
+        int rc = k1_fast_dispatch(h, &f, 1, &grid, h->k1_smem, s, multi);
         if (rc) return rc;
         h->launches++;
         VTI_CUDA(cudaGetLastError());
         return VTI_OK;
     }
-    K1Args a;
+    K1CamArgs a;
     a.frames = frames;
     a.out = net_in;
     a.tap_x_idx = h->d_tap_x_idx;
@@ -867,13 +941,19 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cu
     a.pitch_u = h->k1_pitch_u;
     a.rows_u = h->k1_rows_u;
     a.undistort = h->p.undistort;
+    a.camera = camera; a.n_cameras = h->n_cameras;
     dim3 grid((a.LW + TX - 1) / TX, (a.LH + TY - 1) / TY, B);
-    if (h->k1_mode == MODE_RAW)
-        k1_letterbox_kernel<MODE_RAW><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
+    const K1Args& one = a;
+    if (h->k1_mode == MODE_RAW && multi)
+        k1_letterbox_kernel<MODE_RAW, true><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
+    else if (h->k1_mode == MODE_RAW)
+        k1_letterbox_kernel<MODE_RAW, false><<<grid, K1_THREADS, h->k1_smem, s>>>(one);
+    else if (h->k1_mode == MODE_GATHER && multi)
+        k1_letterbox_kernel<MODE_GATHER, true><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
     else if (h->k1_mode == MODE_GATHER)
-        k1_letterbox_kernel<MODE_GATHER><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
+        k1_letterbox_kernel<MODE_GATHER, false><<<grid, K1_THREADS, h->k1_smem, s>>>(one);
     else
-        k1_letterbox_kernel<MODE_PLAIN><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
+        k1_letterbox_kernel<MODE_PLAIN, false><<<grid, K1_THREADS, h->k1_smem, s>>>(one);
     h->launches++;
     VTI_CUDA(cudaGetLastError());
     return VTI_OK;

@@ -19,6 +19,7 @@
 // Compiled with --fmad=false: numpy / OpenCV do not fuse multiply-adds.
 // The 8-frame temporal median (measurement.py:474-484) is frame-ordered state and stays on the host.
 #include <climits>
+#include <vector>
 
 #include "vti_internal.h"
 
@@ -45,7 +46,27 @@ struct K5Args {
     int variant, min_stitches, max_px, nb;
     int mask_variant;
     int cap;                   // entries per shared array: max_det rounded up to 8
+    const Camera* cams;        // [n_cameras] (multi-camera kernel)
+    const int32_t* camera;     // [B] camera id per frame (multi-camera kernel)
+    int n_cameras;
 };
+
+// measurement.py:44-48 for one calibration.  undistort: the image was already undistorted by K1, so points are
+// measured with dist = 0.  One function for the handle's own camera and for every camera of the device array, so that
+// camera 0 of a multi-camera handle projects bit for bit like a one-camera handle.
+Camera camera_of(const double K[9], const double dist[5], const double R[9], const double t[3], int undistort) {
+    Camera c;
+    c.fx = K[0]; c.fy = K[4]; c.cx = K[2]; c.cy = K[5];
+    c.ifx = 1.0 / c.fx; c.ify = 1.0 / c.fy;
+    const bool lens = !undistort;
+    c.k1 = lens ? dist[0] : 0.0; c.k2 = lens ? dist[1] : 0.0;
+    c.p1 = lens ? dist[2] : 0.0; c.p2 = lens ? dist[3] : 0.0; c.k3 = lens ? dist[4] : 0.0;
+    for (int i = 0; i < 9; ++i) c.R[i] = R[i];
+    for (int i = 0; i < 3; ++i) c.t[i] = t[i];
+    c.n[0] = R[2]; c.n[1] = R[5]; c.n[2] = R[8];                 // n_c = R[:, 2]   (measurement.py:46)
+    c.d_c = -(c.n[0] * t[0] + c.n[1] * t[1] + c.n[2] * t[2]);     // measurement.py:47
+    return c;
+}
 
 __device__ __forceinline__ bool pixel_to_world(const Camera& c, double u, double v, double out[3]) {
     const double x0 = (u - c.cx) * c.ifx, y0 = (v - c.cy) * c.ify;
@@ -217,8 +238,7 @@ __device__ __forceinline__ bool env_median(const int32_t* envf, int w, int cx_in
 // Area of every bitmap on the fabric plane (north-star "area"; spec: oracle/measure_port.py defect_area_mm2): m00 pixels x
 // the plane area of one pixel at the centroid, |dP/du x dP/dv| by central differences.  The four projections of a
 // detection run on four neighbouring lanes.  Called by whole warps: thread t of nt (both multiples of 32 apart).
-__device__ void areas(const K5Args& a, vti_det* __restrict__ dets, int n, int t, int nt, int lane) {
-    const Camera& cam = a.cam;
+__device__ void areas(const Camera& cam, vti_det* __restrict__ dets, int n, int t, int nt, int lane) {
     for (int base = 0; base < 4 * n; base += nt) {                   // warp-uniform trip count (shuffles below)
         const int q4 = base + t, k = q4 >> 2, j = q4 & 3;
         double p[3] = {0.0, 0.0, 0.0};
@@ -247,6 +267,8 @@ __device__ void areas(const K5Args& a, vti_det* __restrict__ dets, int n, int t,
     }
 }
 
+// MULTI: frame b is measured with camera a.camera[b] of a.cams (an id out of range: VTI_ST_BAD_CAMERA, nothing measured)
+template <bool MULTI>
 __global__ void __launch_bounds__(K5_THREADS, 4) k5_measure_kernel(const K5Args a) {
     // everything warp 0 walks sequentially lives in shared memory (global round trips were 70 % of v1's time); the
     // arrays hold a.cap = max_det (rounded up to 8) entries each
@@ -275,8 +297,25 @@ __global__ void __launch_bounds__(K5_THREADS, 4) k5_measure_kernel(const K5Args 
     const int n = a.counts[b];
     vti_det* __restrict__ dets = a.dets + (size_t)b * a.max_det;
     int32_t* __restrict__ envf = a.env_frame + (size_t)b * a.w;
-    const Camera& cam = a.cam;
     const double qnan = __longlong_as_double(0x7ff8000000000000LL);
+    int cam_id = 0;
+    if (MULTI) {
+        cam_id = a.camera[b];
+        if ((unsigned)cam_id >= (unsigned)a.n_cameras) {
+            for (int x = tid; x < a.w; x += K5_THREADS) envf[x] = -1;    // no envelope for the overlay to draw
+            if (tid == 0) {
+                vti_frame_result r;
+                r.status = VTI_ST_BAD_CAMERA | ((a.flags[b] & 1) ? VTI_ST_OVERFLOW : 0);
+                r.n_det = n;
+                r.n_cand = a.flags[b] >> 8;
+                r.n_stitch = 0; r.n_fabric = 0; r.n_dist = 0; r.n_width = 0; r.env_valid = 0;
+                r.avg_dist = qnan; r.avg_width = qnan; r.env_mean = qnan;
+                a.res[b] = r;
+            }
+            return;
+        }
+    }
+    const Camera& cam = MULTI ? a.cams[cam_id] : a.cam;
 
     if (tid == 0) { s_envsum = 0; s_envcnt = 0; s_nfab = 0; s_ns = 0; s_ndrop = 0; }
     __syncthreads();
@@ -384,7 +423,7 @@ __global__ void __launch_bounds__(K5_THREADS, 4) k5_measure_kernel(const K5Args 
             r.status = (s_envcnt == 0 ? VTI_ST_NO_FABRIC : VTI_ST_NO_STITCH) | ovf;
             a.res[b] = r;
         }
-        areas(a, dets, n, tid, K5_THREADS, lane);
+        areas(cam, dets, n, tid, K5_THREADS, lane);
         return;
     }
 
@@ -517,7 +556,7 @@ __global__ void __launch_bounds__(K5_THREADS, 4) k5_measure_kernel(const K5Args 
                 s_wsp[i] = wv;
             }
         }
-        areas(a, dets, n, t0, NT, lane);
+        areas(cam, dets, n, t0, NT, lane);
     }
     __syncthreads();
     const int nsel = s_nsel;
@@ -602,9 +641,23 @@ __global__ void __launch_bounds__(K5_THREADS, 4) k5_measure_kernel(const K5Args 
 // 7 double, 1 unsigned, 3 short and 4 byte arrays of max_det (rounded up to 8) entries
 size_t vti_k5_smem_bytes(int max_det) { return (size_t)((max_det + 7) & ~7) * (7 * 8 + 4 + 3 * 2 + 4); }
 
-int vti_k5_prepare(int max_det) { return vti_raise_dyn_smem((const void*)k5_measure_kernel, vti_k5_smem_bytes(max_det)); }
+int vti_k5_prepare(int max_det) {
+    int rc = vti_raise_dyn_smem((const void*)k5_measure_kernel<false>, vti_k5_smem_bytes(max_det));
+    if (!rc) rc = vti_raise_dyn_smem((const void*)k5_measure_kernel<true>, vti_k5_smem_bytes(max_det));
+    return rc;
+}
 
-int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* res, cudaStream_t s) {
+int vti_k5_cameras(vti_handle* h, const vti_camera* cams, int n) {
+    std::vector<Camera> c(n);
+    for (int i = 0; i < n; ++i) c[i] = camera_of(cams[i].K, cams[i].dist, cams[i].R, cams[i].t, h->p.undistort);
+    Camera* d = nullptr;
+    const int rc = vti_upload(h, &d, c);
+    h->d_k5_cams = d;
+    return rc;
+}
+
+int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* res, const int32_t* camera,
+                  cudaStream_t s) {
     K5Args a;
     a.dets = dets;
     a.counts = counts;
@@ -614,21 +667,18 @@ int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vt
     a.flags = h->d_flags;
     a.res = res;
     const vti_params& p = h->p;
-    Camera& c = a.cam;
-    c.fx = p.K[0]; c.fy = p.K[4]; c.cx = p.K[2]; c.cy = p.K[5];
-    c.ifx = 1.0 / c.fx; c.ify = 1.0 / c.fy;
-    const bool lens = !p.undistort;     // image already undistorted by K1 -> points are measured with dist = 0
-    c.k1 = lens ? p.dist[0] : 0.0; c.k2 = lens ? p.dist[1] : 0.0;
-    c.p1 = lens ? p.dist[2] : 0.0; c.p2 = lens ? p.dist[3] : 0.0; c.k3 = lens ? p.dist[4] : 0.0;
-    for (int i = 0; i < 9; ++i) c.R[i] = p.R[i];
-    for (int i = 0; i < 3; ++i) c.t[i] = p.t[i];
-    c.n[0] = p.R[2]; c.n[1] = p.R[5]; c.n[2] = p.R[8];                 // n_c = R[:, 2]   (measurement.py:46)
-    c.d_c = -(c.n[0] * p.t[0] + c.n[1] * p.t[1] + c.n[2] * p.t[2]);     // measurement.py:47
+    a.cam = camera_of(p.K, p.dist, p.R, p.t, p.undistort);
     a.max_det = p.max_det; a.LW = h->g.LW; a.w = p.frame_w; a.h = p.frame_h;
     a.variant = p.variant; a.min_stitches = p.min_stitches; a.max_px = p.max_px_distance; a.nb = p.neighborhood;
     a.mask_variant = p.mask_variant;
     a.cap = (p.max_det + 7) & ~7;
-    k5_measure_kernel<<<B, K5_THREADS, vti_k5_smem_bytes(p.max_det), s>>>(a);
+    a.cams = static_cast<const Camera*>(h->d_k5_cams);
+    a.camera = camera;
+    a.n_cameras = h->n_cameras;
+    if (camera)
+        k5_measure_kernel<true><<<B, K5_THREADS, vti_k5_smem_bytes(p.max_det), s>>>(a);
+    else
+        k5_measure_kernel<false><<<B, K5_THREADS, vti_k5_smem_bytes(p.max_det), s>>>(a);
     h->launches++;
     VTI_CUDA(cudaGetLastError());
     return VTI_OK;

@@ -10,6 +10,7 @@
 
 static_assert(sizeof(vti_det) == 160, "vti_det must stay 160 bytes");
 static_assert(sizeof(vti_params) == 320, "vti_params must stay 320 bytes (struct_size of existing callers)");
+static_assert(sizeof(vti_camera) == 216, "vti_camera is 216 bytes");
 
 #define VTI_CAND_CAP_MAX 32768      /* hard ceiling of the per-frame candidate list */
 #define VTI_CAND_CAP_DEFAULT 30000  /* Ultralytics' max_nms: with A <= 30000 anchors the list can never overflow */
@@ -42,19 +43,20 @@ struct vti_handle {
     int num_sms;
     int64_t launches;
     VtiRoi roi;
+    int n_cameras;                                 // calibrations of the handle (camera 0 is also in p)
     std::vector<void*> allocs;                     // every device allocation of the handle (vti_alloc)
 
     // ---- K1 tables (device)
     int32_t* d_tap_x_idx;  int16_t* d_tap_x_a;    // [new_w], [new_w*2]
     int32_t* d_tap_y_i;    int16_t* d_tap_y_b;    // [new_h*2], [new_h*2]
-    int32_t* d_und_lut;                            // [frame_h*frame_w] packed (dy16<<16 | dx16), undistort only
+    int32_t* d_und_lut;                            // [camera][frame_h*frame_w] packed (dy16<<16 | dx16), generic remap only
     int resize_mode;                               // 1 bilinear (incl. identity taps), 2 exact-2x area
     int k1_mode, k1_pitch_u, k1_rows_u;            // staging mode + shared footprint buffer shape (k1 plan)
     size_t k1_smem;
     int k1_und_words, k1_lut_stride;               // fast path: footprint buffer words, table entries per tile
     int k1_raw_pitch;                              // fast remap path: words per row of the staged raw box
-    int4* d_k1_tiles;                              // per-tile headers (fast path) / raw bounding boxes (MODE_RAW)
-    unsigned* d_k1_lut;                            // per-tile pre-resolved remap entries (fast path, undistort)
+    int4* d_k1_tiles;                              // [camera] per-tile headers (fast path) / raw bounding boxes (MODE_RAW)
+    unsigned* d_k1_lut;                            // [camera] per-tile pre-resolved remap entries (fast path, undistort)
     // ---- measurement tables (device)
     AxisLut lutY, lutX;                            // [LH], [LW]
     int32_t* d_xmap;                               // [frame_w] frame col -> letterbox col
@@ -70,6 +72,7 @@ struct vti_handle {
                                                    //                 cx_lo | cy_lo << 16, cx_hi | cy_hi << 16)
     int units_per_det;                             // capacity per detection slot
     int4* d_proto_bbox;                            // [B] union of the crop windows of a frame (prototype pixels K4 reads)
+    void* d_k5_cams;                               // [n_cameras] K5's per-camera projection constants
     // ---- host-buffer path
     cudaStream_t own_stream, copy_stream;
     cudaEvent_t chunk_ev[4];
@@ -77,6 +80,7 @@ struct vti_handle {
     uint8_t* d_frames; float* d_net_in; float* d_head[5];     // head: p3, p4, p5, coef, proto
     size_t head_floats[5];                         // floats per frame of each head tensor
     vti_det* d_dets; int32_t* d_counts; vti_frame_result* d_results;
+    int32_t* d_camera;                             // [max_batch] the camera ids of vti_process_host[_yuyv]_multi
     size_t staged_batch;
     // ---- optional per-kernel event timing
     int profiling;
@@ -120,17 +124,23 @@ int vti_raise_dyn_smem(const void* func, size_t bytes);
 int vti_k3_prepare(int cap);
 int vti_k3_cap_pad(int cap);
 int vti_k5_prepare(int max_det);
-// kernel launchers (each returns VTI_OK / VTI_ECUDA)
+// uploads K5's projection constants of every camera of the handle (h->d_k5_cams)
+int vti_k5_cameras(vti_handle* h, const vti_camera* cams, int n);
+// K1 plan.  With undistort on, und_ix / und_iy hold the cv2.undistort source maps of every camera ([camera][h*w], 1/32
+// px) and und_packed their packed displacements ([camera][h*w], uploaded only if the generic kernel runs).
 int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector<int32_t>& yi,
                 const std::vector<int16_t>& xa, const std::vector<int16_t>& yb,
-                const std::vector<int32_t>* und_ix, const std::vector<int32_t>* und_iy);
+                const std::vector<int32_t>* und_ix, const std::vector<int32_t>* und_iy,
+                const std::vector<int32_t>* und_packed);
+// kernel launchers (each returns VTI_OK / VTI_ECUDA).  camera: device ids per frame, or null (camera 0 throughout)
 int vti_launch_k0_yuyv(vti_handle* h, const uint8_t* yuyv, int B, uint8_t* frames, cudaStream_t s);
-int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, cudaStream_t s);
+int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, const int32_t* camera, cudaStream_t s);
 int vti_launch_k2(vti_handle* h, const float* p3, const float* p4, const float* p5, int B, cudaStream_t s);
 int vti_launch_k3(vti_handle* h, const float* coef, int B, vti_det* dets, int32_t* counts, int all_dets, cudaStream_t s);
 int vti_launch_k4(vti_handle* h, const float* proto, int B, vti_det* dets, const int32_t* counts, uint32_t* masks,
                   cudaStream_t s);
-int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* res, cudaStream_t s);
+int vti_launch_k5(vti_handle* h, int B, vti_det* dets, const int32_t* counts, vti_frame_result* res, const int32_t* camera,
+                  cudaStream_t s);
 // copies, per frame, the prototype rectangle K4 will read (all 32 channels) from device-mapped host memory
 int vti_launch_fetch_proto(vti_handle* h, const float* host_proto_mapped, float* dev_proto, int B, cudaStream_t s);
 

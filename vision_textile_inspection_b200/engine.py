@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import DET_DTYPE, RESULT_DTYPE, VtiGeometry, VtiParams, check
+from ._lib import DET_DTYPE, RESULT_DTYPE, VtiCamera, VtiGeometry, VtiParams, check
 
 DATA = os.path.join(os.path.dirname(os.path.abspath(__file__)), "data")
 
@@ -35,6 +35,15 @@ def rodrigues(rvec) -> np.ndarray:
     k = r / th
     Kx = np.array([[0, -k[2], k[1]], [k[2], 0, -k[0]], [-k[1], k[0], 0]])
     return np.cos(th) * np.eye(3) + (1 - np.cos(th)) * np.outer(k, k) + np.sin(th) * Kx
+
+
+def _dist5(dist, what: str) -> list:
+    """Distortion coefficients as the 5 of the implemented model (k1, k2, p1, p2, k3), zero-padded."""
+    d = np.asarray(dist, np.float64).reshape(-1)
+    if d.size > 5 and np.any(d[5:] != 0.0):
+        raise ValueError(f"{what}: only the 5-coefficient model (k1, k2, p1, p2, k3) is implemented; "
+                         f"got {d.size} coefficients with non-zero higher terms")
+    return np.concatenate([d[:5], np.zeros(max(0, 5 - d.size))]).tolist()
 
 
 @dataclass
@@ -63,6 +72,7 @@ class EngineConfig:
     neighborhood: int = 3
     max_candidates: int = 0
     mask_variant: int = 0         # 0 = "A" (sigmoid, > 0.5), 1 = "B" (newer Ultralytics: logits, > 0.0, empty masks dropped)
+    cameras: list | None = None   # several cameras of this frame size: [{K, dist, R, t}, ...]; K / dist / R / t are then unused
 
     @staticmethod
     def for_workload(cfg, calib: dict | None = None, max_batch: int | None = None) -> "EngineConfig":
@@ -95,15 +105,22 @@ class EngineConfig:
         p.conf, p.iou = self.conf, self.iou
         p.iou_threshold = float(self.iou)          # the Python float torchvision.ops.nms receives (a C++ double)
         p.K[:] = np.asarray(self.K, np.float64).reshape(9).tolist()
-        d = np.asarray(self.dist, np.float64).reshape(-1)
-        if d.size > 5 and np.any(d[5:] != 0.0):
-            raise ValueError("EngineConfig.dist: only the 5-coefficient model (k1, k2, p1, p2, k3) is implemented; "
-                             f"got {d.size} coefficients with non-zero higher terms")
-        d = np.concatenate([d[:5], np.zeros(max(0, 5 - d.size))])
-        p.dist[:] = d.tolist()
+        p.dist[:] = _dist5(self.dist, "EngineConfig.dist")
         p.R[:] = np.asarray(self.R, np.float64).reshape(9).tolist()
         p.t[:] = np.asarray(self.t, np.float64).reshape(3).tolist()
         return p
+
+    def to_cameras(self):
+        """`cameras` as a ctypes array of VtiCamera (vti_create_multi)."""
+        arr = (VtiCamera * len(self.cameras))()
+        for i, cam in enumerate(self.cameras):
+            c = arr[i]
+            c.struct_size = C.sizeof(VtiCamera)
+            c.K[:] = np.asarray(cam["K"], np.float64).reshape(9).tolist()
+            c.dist[:] = _dist5(cam["dist"], f"EngineConfig.cameras[{i}].dist")
+            c.R[:] = np.asarray(cam["R"], np.float64).reshape(9).tolist()
+            c.t[:] = np.asarray(cam["t"], np.float64).reshape(3).tolist()
+        return arr
 
 
 class InspectionEngine:
@@ -119,7 +136,12 @@ class InspectionEngine:
             raise _lib.VtiError("InspectionEngine device must be CUDA")
         self._h = C.c_void_p()
         with torch.cuda.device(self.device):
-            check(self.lib.vti_create(C.byref(cfg.to_params()), C.byref(self._h)), "vti_create")
+            if cfg.cameras:
+                check(self.lib.vti_create_multi(C.byref(cfg.to_params()), len(cfg.cameras), cfg.to_cameras(),
+                                                C.byref(self._h)), "vti_create_multi")
+            else:
+                check(self.lib.vti_create(C.byref(cfg.to_params()), C.byref(self._h)), "vti_create")
+        self.n_cameras = int(self.lib.vti_camera_count(self._h))
         g = VtiGeometry()
         check(self.lib.vti_get_geometry(self._h, C.byref(g)), "vti_get_geometry")
         self.g = g
@@ -146,6 +168,13 @@ class InspectionEngine:
             raise ValueError(f"{name}: expected contiguous {dtype} {tuple(shape)} on {self.device}, got "
                              f"{t.dtype} {tuple(t.shape)} on {t.device}")
 
+    def _chk_camera(self, camera, B):
+        """Device pointer of a per-frame camera id tensor (int32 (B,) on the engine's device), or None."""
+        if camera is None:
+            return None
+        self._chk(camera, torch.int32, (B,), "camera")
+        return camera.data_ptr()
+
     def alloc_outputs(self, B: int, masks: bool = False):
         dets = torch.empty((B, self.cfg.max_det, DET_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         counts = torch.empty((B,), dtype=torch.int32, device=self.device)
@@ -156,15 +185,21 @@ class InspectionEngine:
         return dets, counts, results, m
 
     # ------------------------------------------------------------------------------------------------- stages
-    def preprocess(self, frames: torch.Tensor, out: torch.Tensor | None = None) -> torch.Tensor:
-        """K1.  frames (B,h,w,3) uint8 -> (B,3,LH,LW) float32."""
+    def preprocess(self, frames: torch.Tensor, out: torch.Tensor | None = None, camera=None) -> torch.Tensor:
+        """K1.  frames (B,h,w,3) uint8 -> (B,3,LH,LW) float32.  camera: int32 (B,) device tensor of camera ids (None:
+        camera 0 for every frame)."""
         B = frames.shape[0]
         self._chk(frames, torch.uint8, (B, self.cfg.frame_h, self.cfg.frame_w, 3), "frames")
+        cam = self._chk_camera(camera, B)
         if out is None:
             out = torch.empty((B, 3, self.LH, self.LW), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            check(self.lib.vti_preprocess(self._h, frames.data_ptr(), B, out.data_ptr(), self._stream()),
-                  "vti_preprocess")
+            if cam is None:
+                check(self.lib.vti_preprocess(self._h, frames.data_ptr(), B, out.data_ptr(), self._stream()),
+                      "vti_preprocess")
+            else:
+                check(self.lib.vti_preprocess_multi(self._h, frames.data_ptr(), cam, B, out.data_ptr(), self._stream()),
+                      "vti_preprocess_multi")
         return out
 
     def _check_head(self, p3, p4, p5, coef, proto):
@@ -186,31 +221,42 @@ class InspectionEngine:
                   "vti_postprocess")
         return dets, counts, masks
 
-    def measure(self, dets, counts, results=None):
-        """K5.  Completes the records in place; returns the per-frame result tensor."""
+    def measure(self, dets, counts, results=None, camera=None):
+        """K5.  Completes the records in place; returns the per-frame result tensor.  camera: as in preprocess."""
         B = dets.shape[0]
+        cam = self._chk_camera(camera, B)
         if results is None:
             results = torch.empty((B, RESULT_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         with torch.cuda.device(self.device):
-            check(self.lib.vti_measure(self._h, B, dets.data_ptr(), counts.data_ptr(), results.data_ptr(),
-                                       self._stream()), "vti_measure")
+            if cam is None:
+                check(self.lib.vti_measure(self._h, B, dets.data_ptr(), counts.data_ptr(), results.data_ptr(),
+                                           self._stream()), "vti_measure")
+            else:
+                check(self.lib.vti_measure_multi(self._h, B, cam, dets.data_ptr(), counts.data_ptr(), results.data_ptr(),
+                                                 self._stream()), "vti_measure_multi")
         return results
 
-    def post_measure(self, p3, p4, p5, coef, proto, outputs=None, export_masks: bool = False):
+    def post_measure(self, p3, p4, p5, coef, proto, outputs=None, export_masks: bool = False, camera=None):
         B = self._check_head(p3, p4, p5, coef, proto)
+        cam = self._chk_camera(camera, B)
         dets, counts, results, masks = outputs if outputs is not None else self.alloc_outputs(B, export_masks)
+        head = [p3.data_ptr(), p4.data_ptr(), p5.data_ptr(), coef.data_ptr(), proto.data_ptr()]
+        mptr = masks.data_ptr() if masks is not None else None
         with torch.cuda.device(self.device):
-            check(self.lib.vti_post_measure(self._h, p3.data_ptr(), p4.data_ptr(), p5.data_ptr(), coef.data_ptr(),
-                                            proto.data_ptr(), B, dets.data_ptr(), counts.data_ptr(),
-                                            masks.data_ptr() if masks is not None else None, results.data_ptr(),
-                                            self._stream()), "vti_post_measure")
+            if cam is None:
+                check(self.lib.vti_post_measure(self._h, *head, B, dets.data_ptr(), counts.data_ptr(), mptr,
+                                                results.data_ptr(), self._stream()), "vti_post_measure")
+            else:
+                check(self.lib.vti_post_measure_multi(self._h, *head, B, cam, dets.data_ptr(), counts.data_ptr(), mptr,
+                                                      results.data_ptr(), self._stream()), "vti_post_measure_multi")
         return dets, counts, results, masks
 
-    def capture_step(self, frames, p3, p4, p5, coef, proto, net_in=None, outputs=None, export_masks: bool = False):
+    def capture_step(self, frames, p3, p4, p5, coef, proto, net_in=None, outputs=None, export_masks: bool = False,
+                     camera=None):
         """One pass of the hot path as ONE CUDA graph: K1 on a forked branch beside K2 -> K3 -> K4 -> K5, joined at the
         end.  The stage entry points only launch kernels on the stream they are handed (no allocation, no
         synchronisation), so they are capturable as they are.  Returns (graph, net_in, (dets, counts, results, masks));
-        `graph.replay()` re-runs the step on the CURRENT contents of the captured buffers."""
+        `graph.replay()` re-runs the step on the CURRENT contents of the captured buffers, the camera ids included."""
         B = self._check_head(p3, p4, p5, coef, proto)
         self._chk(frames, torch.uint8, (B, self.cfg.frame_h, self.cfg.frame_w, 3), "frames")
         if net_in is None:
@@ -218,8 +264,8 @@ class InspectionEngine:
         if outputs is None:
             outputs = self.alloc_outputs(B, export_masks)
         with torch.cuda.device(self.device):
-            self.preprocess(frames, out=net_in)              # warm-up outside the capture (lazy module loading)
-            self.post_measure(p3, p4, p5, coef, proto, outputs=outputs)
+            self.preprocess(frames, out=net_in, camera=camera)     # warm-up outside the capture (lazy module loading)
+            self.post_measure(p3, p4, p5, coef, proto, outputs=outputs, camera=camera)
             torch.cuda.synchronize(self.device)
             graph = torch.cuda.CUDAGraph()
             side = torch.cuda.Stream(self.device, priority=-1)   # kernel nodes keep the priority of their stream:
@@ -227,8 +273,8 @@ class InspectionEngine:
                 cur = torch.cuda.current_stream(self.device)
                 side.wait_stream(cur)                        # fork: K1 does not depend on the post stage
                 with torch.cuda.stream(side):
-                    self.post_measure(p3, p4, p5, coef, proto, outputs=outputs)
-                self.preprocess(frames, out=net_in)
+                    self.post_measure(p3, p4, p5, coef, proto, outputs=outputs, camera=camera)
+                self.preprocess(frames, out=net_in, camera=camera)
                 cur.wait_stream(side)                        # join
         return graph, net_in, outputs
 
@@ -300,13 +346,23 @@ class InspectionEngine:
             check(self.lib.vti_ingest_yuyv(self._h, yuyv.data_ptr(), B, out.data_ptr(), self._stream()), "vti_ingest_yuyv")
         return out
 
-    def process_host(self, frames: np.ndarray, p3, p4, p5, coef, proto, want_net_in: bool = False, out=None):
+    def process_host(self, frames: np.ndarray, p3, p4, p5, coef, proto, want_net_in: bool = False, out=None, camera=None):
         """End-to-end with HOST numpy buffers (ideally pinned): H2D, K1..K5, D2H.  Returns (dets, counts, results[, net_in]).
-        `frames` is (B,h,w,3) BGR, or (B,h,w,2) camera-native YUYV (converted on the device by K0)."""
+        `frames` is (B,h,w,3) BGR, or (B,h,w,2) camera-native YUYV (converted on the device by K0).  camera: host array of
+        B camera ids (None: camera 0 for every frame); an id out of range raises VtiError before any work."""
         B = frames.shape[0]
         if frames.dtype != np.uint8 or frames.ndim != 4 or frames.shape[1:3] != (self.cfg.frame_h, self.cfg.frame_w) or frames.shape[3] not in (2, 3):
             raise ValueError(f"process_host: frames must be uint8 (B,{self.cfg.frame_h},{self.cfg.frame_w},3) BGR or (..,2) YUYV, got {frames.dtype} {frames.shape}")
-        entry = self.lib.vti_process_host if frames.shape[3] == 3 else self.lib.vti_process_host_yuyv
+        if camera is None:
+            entry = self.lib.vti_process_host if frames.shape[3] == 3 else self.lib.vti_process_host_yuyv
+        else:
+            cam = np.ascontiguousarray(camera, dtype=np.int32)
+            if cam.shape != (B,):
+                raise ValueError(f"process_host: camera must hold {B} ids, got shape {cam.shape}")
+            multi = self.lib.vti_process_host_multi if frames.shape[3] == 3 else self.lib.vti_process_host_yuyv_multi
+
+            def entry(h, fr, a3, a4, a5, co, pr, nb, *rest):
+                return multi(h, fr, a3, a4, a5, co, pr, nb, cam.ctypes.data, *rest)
         if out is None:
             out = (np.empty((B, self.cfg.max_det), DET_DTYPE), np.empty((B,), np.int32), np.empty((B,), RESULT_DTYPE))
         dets, counts, results = out
