@@ -19,7 +19,6 @@
 // HBM traffic: frame read once (tile halos hit L2) + 12*LH*LW written once; the 4 B/px remap table is L2-resident
 // across the batch.
 #include <algorithm>
-#include <type_traits>
 #include <vector>
 
 #include "vti_internal.h"
@@ -48,12 +47,12 @@ struct K1Args {
     int pitch_u;                // words per row of the footprint buffer
     int rows_u;                 // rows of the footprint buffer
     int undistort;
-};
-// The per-frame camera forms take the ids in a derived struct: the one-camera kernels keep their parameter block
-struct K1CamArgs : K1Args {
-    const int32_t* camera;      // [B] camera id per frame
     int n_cameras;
+    const int32_t* camera;      // [B] camera id per frame, or null: camera 0 for every frame
 };
+// K1Args and K1FastArgs stay within 128 bytes: past that, nvcc compiles every K1 kernel differently, also those that
+// read no camera.
+static_assert(sizeof(K1Args) <= 128, "K1Args: parameter block over 128 bytes");
 
 __device__ __forceinline__ unsigned pack_px(unsigned b0, unsigned b1, unsigned b2, int flip) {
     return flip ? (b2 | (b1 << 8) | (b0 << 16)) : (b0 | (b1 << 8) | (b2 << 16));
@@ -100,9 +99,9 @@ __device__ __forceinline__ unsigned remap_packed(unsigned t00, unsigned t01, uns
     return b | (g << 8) | (r << 16);
 }
 
-// Frame b takes camera b's remap tables (MULTI: a.camera[b]; an id out of range: camera 0's), else camera 0's.
-template <int MODE, bool MULTI>
-__global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const std::conditional_t<MULTI, K1CamArgs, K1Args> a) {
+// Frame b takes the remap tables of camera a.camera[b] (null ids, or an id out of range: camera 0's).
+template <int MODE>
+__global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const K1Args a) {
     extern __shared__ __align__(128) unsigned s_dyn[];     // [footprint rows][pitch_u] then the raw box (MODE_RAW)
     __shared__ float s_div[256];
     __shared__ int s_rowsrc[MAXROWS];
@@ -115,12 +114,13 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const std::con
     const uint8_t* __restrict__ frame = a.frames + (size_t)b * a.h * a.w * 3;
     float* __restrict__ out = a.out + (size_t)b * 3 * a.LH * a.LW;
     unsigned* s_und = s_dyn;
-    const int32_t* und_lut = a.und_lut;
+    // the camera's first row in und_lut [camera][h][w]; an offset pointer instead takes MODE_RAW from 32 to 40 registers
+    int cam_row = 0;
     const int4* tile_box = a.tile_box;
-    if constexpr (MULTI) {
+    if (MODE != MODE_PLAIN && a.camera) {
         const int cam = __ldg(a.camera + b);
         if ((unsigned)cam < (unsigned)a.n_cameras) {
-            und_lut += (size_t)cam * a.h * a.w;
+            cam_row = cam * a.h;
             tile_box += (size_t)cam * gridDim.x * gridDim.y;
         }
     }
@@ -189,7 +189,7 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const std::con
             __syncthreads();
             for (int r = warp; r < nrows; r += K1_THREADS / 32) {
                 const int sy = s_rowsrc[r];
-                const int32_t* __restrict__ lrow = und_lut + (size_t)sy * a.w;
+                const int32_t* __restrict__ lrow = a.und_lut + (size_t)(cam_row + sy) * a.w;
                 for (int c = lane; c < ncols; c += 32) {
                     const int sx = c_lo + c;
                     const int lut = __ldg(lrow + sx);
@@ -215,7 +215,7 @@ __global__ void __launch_bounds__(K1_THREADS) k1_letterbox_kernel(const std::con
                 const int sy = s_rowsrc[r];
                 for (int c = lane; c < ncols; c += 32) {
                     const int sx = s_colsrc[c];
-                    const int lut = __ldg(und_lut + (size_t)sy * a.w + sx);
+                    const int lut = __ldg(a.und_lut + (size_t)(cam_row + sy) * a.w + sx);
                     const int ix = sx * 32 + (int)(short)(lut & 0xffff), iy = sy * 32 + (lut >> 16);
                     const int x = ix >> 5, y = iy >> 5;
                     const bool x0 = (unsigned)x < (unsigned)a.w, x1 = (unsigned)(x + 1) < (unsigned)a.w;
@@ -323,15 +323,14 @@ struct K1FastArgs {
     const int16_t* tap_y_b;     // [new_h][2]
     int h, w, new_h, new_w, top, left, LH, LW;
     int flip;
-    int pitch_u, rows_u;
-    int und_words;              // words reserved for the footprint buffer (multiple of FT_CHUNK, > rows_u * pitch_u)
+    int pitch_u;
+    int n_cameras;              // (in a dropped field's slot: the fields keep their offsets, the one-camera kernels their code)
+    int und_words;              // words reserved for the footprint buffer (multiple of FT_CHUNK, > its rows * pitch_u)
     int lut_stride;             // entries per tile (multiple of FT_CHUNK)
     int raw_pitch;              // words per row of the raw box in shared memory (the same for every tile and camera)
+    const int32_t* camera;      // [B] camera id per frame   (MULTI only)
 };
-struct K1FastCamArgs : K1FastArgs {
-    const int32_t* camera;      // [B] camera id per frame
-    int n_cameras;
-};
+static_assert(sizeof(K1FastArgs) <= 128, "K1FastArgs: parameter block over 128 bytes (see K1Args)");
 
 // Stage rows [y0, y0+nr) x 8-pixel groups [x0, x0 + 8*ng) of the frame as packed words (B | G<<8 | R<<16, byte 3 = 0);
 // anything outside the image becomes 0 (the zero margin of cv2.remap's BORDER_CONSTANT).  x0 % 8 == 0, w % 8 == 0, so a
@@ -537,8 +536,9 @@ __device__ __forceinline__ void resize_phase(const K1FastArgs& a, float* __restr
 }
 
 // MULTI (REMAP only): frame b takes the headers and remap table of camera a.camera[b] (an id out of range: camera 0's).
+// A test of a.camera at run time instead makes the one-camera remap kernel 0.3 % slower on cfg2 (DESIGN.md 3).
 template <bool REMAP, bool AREA, int LW_T, int RAWP_T, bool MULTI>
-__global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const std::conditional_t<MULTI, K1FastCamArgs, K1FastArgs> a) {
+__global__ void __launch_bounds__(FT_THREADS, FT_MINB) k1_fast_kernel(const K1FastArgs a) {
     extern __shared__ __align__(128) unsigned s_dyn[];     // s_und [und_words], then the raw box (REMAP)
     __shared__ int4 s_rowtap[FTY];                          // (byte offset row0, byte offset row1, b0, b1)
 
@@ -743,21 +743,20 @@ static bool k1_fast_plan(vti_handle* h, const std::vector<int32_t>& xi, const st
 // The one place that names every instantiation of the fast kernel: launch == 0 raises each one's dynamic
 // shared-memory limit (plan time), launch == 1 launches the one that matches the handle.
 template <bool REMAP, bool AREA, int LW_T, int RAWP_T, bool MULTI>
-static int k1_fast_one(const K1FastCamArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
+static int k1_fast_one(const K1FastArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
     if (!launch) return vti_raise_dyn_smem((const void*)k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI>, smem);
-    if constexpr (MULTI) k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI><<<*grid, FT_THREADS, smem, s>>>(*f);
-    else k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI><<<*grid, FT_THREADS, smem, s>>>(static_cast<const K1FastArgs&>(*f));
+    k1_fast_kernel<REMAP, AREA, LW_T, RAWP_T, MULTI><<<*grid, FT_THREADS, smem, s>>>(*f);
     return VTI_OK;
 }
 template <bool AREA, int LW_T, int RAWP_T>
-static int k1_fast_remap(bool multi, const K1FastCamArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
+static int k1_fast_remap(bool multi, const K1FastArgs* f, int launch, const dim3* grid, size_t smem, cudaStream_t s) {
     int rc = VTI_OK;
     if (!launch || !multi) if ((rc = k1_fast_one<true, AREA, LW_T, RAWP_T, false>(f, launch, grid, smem, s))) return rc;
     if (!launch || multi) rc = k1_fast_one<true, AREA, LW_T, RAWP_T, true>(f, launch, grid, smem, s);
     return rc;
 }
 template <int LW_T>
-static int k1_fast_lw(bool remap, bool area, int rawp, bool multi, const K1FastCamArgs* f, int launch, const dim3* grid,
+static int k1_fast_lw(bool remap, bool area, int rawp, bool multi, const K1FastArgs* f, int launch, const dim3* grid,
                       size_t smem, cudaStream_t s) {
     int rc = VTI_OK;
     const bool fixed = rawp == K1_RAWP;
@@ -770,7 +769,7 @@ static int k1_fast_lw(bool remap, bool area, int rawp, bool multi, const K1FastC
     return rc;
 }
 // multi: the per-frame camera form (remap only; without undistort K1 does not depend on the camera)
-static int k1_fast_dispatch(vti_handle* h, const K1FastCamArgs* f, int launch, const dim3* grid, size_t smem,
+static int k1_fast_dispatch(vti_handle* h, const K1FastArgs* f, int launch, const dim3* grid, size_t smem,
                             cudaStream_t s = nullptr, bool multi = false) {
     const bool remap = h->k1_mode == MODE_FAST_REMAP, area = h->resize_mode == 2;
     const int LW = h->g.LW, rawp = h->k1_raw_pitch;
@@ -809,7 +808,7 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
             if (und_ix) smem = std::max(smem, (size_t)(46 * 1024 + 512));     // (measured with the remap path)
             if (smem <= 110 * 1024) {
                 h->k1_mode = und_ix ? MODE_FAST_REMAP : MODE_FAST_PLAIN;
-                h->k1_pitch_u = pitch_u; h->k1_rows_u = rows_u; h->k1_smem = smem;
+                h->k1_pitch_u = pitch_u; h->k1_smem = smem;
                 h->k1_und_words = und_words; h->k1_lut_stride = lut_stride; h->k1_raw_pitch = raw_pitch;
                 int rc;
                 if ((rc = vti_upload(h, &h->d_k1_tiles, hdr)) || (und_ix && (rc = vti_upload(h, &h->d_k1_lut, lut)))) return rc;
@@ -884,20 +883,14 @@ int vti_k1_plan(vti_handle* h, const std::vector<int32_t>& xi, const std::vector
             h->k1_mode = MODE_GATHER;
         }
     }
-    int rc;
-    if (h->k1_mode == MODE_RAW) {
-        if ((rc = vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_RAW, false>, h->k1_smem))) return rc;
-        return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_RAW, true>, h->k1_smem);
-    }
-    if (h->k1_mode == MODE_GATHER) {
-        if ((rc = vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_GATHER, false>, h->k1_smem))) return rc;
-        return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_GATHER, true>, h->k1_smem);
-    }
-    return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_PLAIN, false>, h->k1_smem);
+    if (h->k1_mode == MODE_RAW) return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_RAW>, h->k1_smem);
+    if (h->k1_mode == MODE_GATHER) return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_GATHER>, h->k1_smem);
+    return vti_raise_dyn_smem((const void*)k1_letterbox_kernel<MODE_PLAIN>, h->k1_smem);
 }
 
 // camera: per-frame ids (device) or null.  Only the remap depends on the camera, and a one-camera handle has one set of
-// tables for every id, so the per-frame form runs only for undistort with more than one camera.
+// tables for every id, so ids reach the kernels only for undistort with more than one camera: the fast path then runs
+// its per-frame camera form, and the generic kernel reads ids only when they are not null.
 int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, const int32_t* camera, cudaStream_t s) {
     const bool multi = camera && h->p.undistort && h->n_cameras > 1;
     if (h->k1_mode == MODE_FAST_PLAIN || h->k1_mode == MODE_FAST_REMAP) {
@@ -905,14 +898,14 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, co
             vti_set_error("vti_preprocess: frames must be 8-byte aligned and net_in 4-byte aligned (64-bit staging loads)");
             return VTI_EINVAL;
         }
-        K1FastCamArgs f;
+        K1FastArgs f;
         f.frames = frames; f.out = net_in;
         f.tile_hdr = h->d_k1_tiles; f.lut = h->d_k1_lut;
         f.tap_x_idx = h->d_tap_x_idx; f.tap_x_a = h->d_tap_x_a; f.tap_y_i = h->d_tap_y_i; f.tap_y_b = h->d_tap_y_b;
         f.h = h->p.frame_h; f.w = h->p.frame_w; f.new_h = h->g.new_h; f.new_w = h->g.new_w;
         f.top = h->g.top; f.left = h->g.left; f.LH = h->g.LH; f.LW = h->g.LW;
         f.flip = h->p.channel_flip;
-        f.pitch_u = h->k1_pitch_u; f.rows_u = h->k1_rows_u;
+        f.pitch_u = h->k1_pitch_u;
         f.und_words = h->k1_und_words; f.lut_stride = h->k1_lut_stride;
         f.raw_pitch = h->k1_raw_pitch;
         f.camera = camera; f.n_cameras = h->n_cameras;
@@ -923,7 +916,7 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, co
         VTI_CUDA(cudaGetLastError());
         return VTI_OK;
     }
-    K1CamArgs a;
+    K1Args a;
     a.frames = frames;
     a.out = net_in;
     a.tap_x_idx = h->d_tap_x_idx;
@@ -941,19 +934,14 @@ int vti_launch_k1(vti_handle* h, const uint8_t* frames, int B, float* net_in, co
     a.pitch_u = h->k1_pitch_u;
     a.rows_u = h->k1_rows_u;
     a.undistort = h->p.undistort;
-    a.camera = camera; a.n_cameras = h->n_cameras;
+    a.camera = multi ? camera : nullptr; a.n_cameras = h->n_cameras;
     dim3 grid((a.LW + TX - 1) / TX, (a.LH + TY - 1) / TY, B);
-    const K1Args& one = a;
-    if (h->k1_mode == MODE_RAW && multi)
-        k1_letterbox_kernel<MODE_RAW, true><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
-    else if (h->k1_mode == MODE_RAW)
-        k1_letterbox_kernel<MODE_RAW, false><<<grid, K1_THREADS, h->k1_smem, s>>>(one);
-    else if (h->k1_mode == MODE_GATHER && multi)
-        k1_letterbox_kernel<MODE_GATHER, true><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
+    if (h->k1_mode == MODE_RAW)
+        k1_letterbox_kernel<MODE_RAW><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
     else if (h->k1_mode == MODE_GATHER)
-        k1_letterbox_kernel<MODE_GATHER, false><<<grid, K1_THREADS, h->k1_smem, s>>>(one);
+        k1_letterbox_kernel<MODE_GATHER><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
     else
-        k1_letterbox_kernel<MODE_PLAIN, false><<<grid, K1_THREADS, h->k1_smem, s>>>(one);
+        k1_letterbox_kernel<MODE_PLAIN><<<grid, K1_THREADS, h->k1_smem, s>>>(a);
     h->launches++;
     VTI_CUDA(cudaGetLastError());
     return VTI_OK;

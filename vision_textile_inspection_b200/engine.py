@@ -194,12 +194,8 @@ class InspectionEngine:
         if out is None:
             out = torch.empty((B, 3, self.LH, self.LW), dtype=torch.float32, device=self.device)
         with torch.cuda.device(self.device):
-            if cam is None:
-                check(self.lib.vti_preprocess(self._h, frames.data_ptr(), B, out.data_ptr(), self._stream()),
-                      "vti_preprocess")
-            else:
-                check(self.lib.vti_preprocess_multi(self._h, frames.data_ptr(), cam, B, out.data_ptr(), self._stream()),
-                      "vti_preprocess_multi")
+            check(self.lib.vti_preprocess_multi(self._h, frames.data_ptr(), cam, B, out.data_ptr(), self._stream()),
+                  "vti_preprocess_multi")
         return out
 
     def _check_head(self, p3, p4, p5, coef, proto):
@@ -228,12 +224,8 @@ class InspectionEngine:
         if results is None:
             results = torch.empty((B, RESULT_DTYPE.itemsize), dtype=torch.uint8, device=self.device)
         with torch.cuda.device(self.device):
-            if cam is None:
-                check(self.lib.vti_measure(self._h, B, dets.data_ptr(), counts.data_ptr(), results.data_ptr(),
-                                           self._stream()), "vti_measure")
-            else:
-                check(self.lib.vti_measure_multi(self._h, B, cam, dets.data_ptr(), counts.data_ptr(), results.data_ptr(),
-                                                 self._stream()), "vti_measure_multi")
+            check(self.lib.vti_measure_multi(self._h, B, cam, dets.data_ptr(), counts.data_ptr(), results.data_ptr(),
+                                             self._stream()), "vti_measure_multi")
         return results
 
     def post_measure(self, p3, p4, p5, coef, proto, outputs=None, export_masks: bool = False, camera=None):
@@ -243,12 +235,8 @@ class InspectionEngine:
         head = [p3.data_ptr(), p4.data_ptr(), p5.data_ptr(), coef.data_ptr(), proto.data_ptr()]
         mptr = masks.data_ptr() if masks is not None else None
         with torch.cuda.device(self.device):
-            if cam is None:
-                check(self.lib.vti_post_measure(self._h, *head, B, dets.data_ptr(), counts.data_ptr(), mptr,
-                                                results.data_ptr(), self._stream()), "vti_post_measure")
-            else:
-                check(self.lib.vti_post_measure_multi(self._h, *head, B, cam, dets.data_ptr(), counts.data_ptr(), mptr,
-                                                      results.data_ptr(), self._stream()), "vti_post_measure_multi")
+            check(self.lib.vti_post_measure_multi(self._h, *head, B, cam, dets.data_ptr(), counts.data_ptr(), mptr,
+                                                  results.data_ptr(), self._stream()), "vti_post_measure_multi")
         return dets, counts, results, masks
 
     def capture_step(self, frames, p3, p4, p5, coef, proto, net_in=None, outputs=None, export_masks: bool = False,
@@ -353,16 +341,12 @@ class InspectionEngine:
         B = frames.shape[0]
         if frames.dtype != np.uint8 or frames.ndim != 4 or frames.shape[1:3] != (self.cfg.frame_h, self.cfg.frame_w) or frames.shape[3] not in (2, 3):
             raise ValueError(f"process_host: frames must be uint8 (B,{self.cfg.frame_h},{self.cfg.frame_w},3) BGR or (..,2) YUYV, got {frames.dtype} {frames.shape}")
-        if camera is None:
-            entry = self.lib.vti_process_host if frames.shape[3] == 3 else self.lib.vti_process_host_yuyv
-        else:
+        cam = None
+        if camera is not None:
             cam = np.ascontiguousarray(camera, dtype=np.int32)
             if cam.shape != (B,):
                 raise ValueError(f"process_host: camera must hold {B} ids, got shape {cam.shape}")
-            multi = self.lib.vti_process_host_multi if frames.shape[3] == 3 else self.lib.vti_process_host_yuyv_multi
-
-            def entry(h, fr, a3, a4, a5, co, pr, nb, *rest):
-                return multi(h, fr, a3, a4, a5, co, pr, nb, cam.ctypes.data, *rest)
+        entry = self.lib.vti_process_host_multi if frames.shape[3] == 3 else self.lib.vti_process_host_yuyv_multi
         if out is None:
             out = (np.empty((B, self.cfg.max_det), DET_DTYPE), np.empty((B,), np.int32), np.empty((B,), RESULT_DTYPE))
         dets, counts, results = out
@@ -372,7 +356,7 @@ class InspectionEngine:
             if not a_.flags["C_CONTIGUOUS"]:
                 raise ValueError("process_host needs C-contiguous host arrays")
         with torch.cuda.device(self.device):
-            check(entry(self._h, *[a_.ctypes.data for a_ in arrs], B,
+            check(entry(self._h, *[a_.ctypes.data for a_ in arrs], B, cam.ctypes.data if cam is not None else None,
                         net_in.ctypes.data if net_in is not None else None, dets.ctypes.data,
                         counts.ctypes.data, results.ctypes.data), "vti_process_host")
         return (dets, counts, results, net_in) if want_net_in else (dets, counts, results)
